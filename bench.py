@@ -2,7 +2,7 @@
 """bench.py -- headline benchmark of the sparsepoly B200 backend (contract in the task prompt).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
-                    [--workload auto|psgd|pcd|pbcd|allsub|c1] [--scale S]
+                    [--workload auto|psgd|pcd|pbcd|allsub|c1] [--scale S] [--dump-outputs DIR]
 
 Workloads (BASELINE.json configs / SURVEY.md 8d):
   psgd   C5  FM-Clf degree=2 psgd squaredl12 logistic, Criteo-shaped d=1M 39 nnz/row k=32,
@@ -18,6 +18,13 @@ peer-memory exchange); pcd / pbcd are sequential in the coordinate order and sta
 With --workload auto (default) the headline line is psgd; at N=1 the "also" list carries C2, C3, C4 and C1,
 each with its own roofline / e2e / cpu_baseline; at N>1 it carries the strong-scaling psgd run (global
 minibatch = auto, split over the ranks).
+`--steps K` is the number of timed epochs of the headline workload (and of its e2e fit).  The "also" entries keep
+their own fixed counts (3 epochs, 10 for C1, min(K, 10) for the strong-scaling run) so that the secondary lines
+stay comparable whatever K is; each entry reports its own `steps`.
+
+`--dump-outputs DIR` writes the model the headline workload's timed epochs computed (P_ and w_, as a caller of fit()
+receives them) to DIR/<name>.npy in float64, at most 64 MB in all.  The inputs are seeded, so two builds of the
+project can be compared output for output.
 
 `--impl reference` times the reference algorithm on the host CPU (the pinned C oracle port of the numba
 path, 1 core -- the reference is single threaded; the numba package itself cannot travel to the GPU box) on
@@ -167,6 +174,22 @@ def make_problem(name, scale=1.0, rank=0):
     s = s + 0.5 * (s ** 2 - np.mean(s ** 2)) + 0.1 * np.std(s) * rng.randn(n)
     y = np.where(s > np.median(s), 1.0, -1.0) if wl["clf"] else (s / np.std(s))
     return X, y
+
+
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, arrays):
+    """Write every array as out_dir/<name>.npy in float64.  An array larger than its share of DUMP_BYTES is replaced
+    by a fixed, seeded sample of its last (feature) axis: the same columns in every run with the same arguments."""
+    os.makedirs(out_dir, exist_ok=True)
+    share = DUMP_BYTES // len(arrays)
+    for name, a in arrays.items():
+        a = np.ascontiguousarray(a, dtype=np.float64)
+        if a.nbytes > share:
+            keep = share // (a.nbytes // a.shape[-1])
+            a = a[..., np.sort(np.random.RandomState(0).choice(a.shape[-1], keep, replace=False))]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def sweep_bytes(name, nnz, n, k, degree, fit_linear):
@@ -335,7 +358,7 @@ def sweep_config(name, args, X, world):
 
 
 # --------------------------------------------------------------------------------- GPU arm
-def run_sweep_workload(name, args, rank, world, local):
+def run_sweep_workload(name, args, rank, world, local, dump_dir=None):
     import torch
     import sparsepoly_b200 as S
     from sparsepoly_b200 import _lib
@@ -407,6 +430,8 @@ def run_sweep_workload(name, args, rank, world, local):
     wspec = (C.c_ulonglong * 2)()
     lib.sp_wspec_read(wspec)
     sync()
+    if dump_dir is not None and rank == 0:
+        dump_outputs(dump_dir, {"P_": est.P_, **({"w_": est.w_} if hasattr(est, "w_") else {})})
     nz_frac = float(np.mean(est.P_ != 0))
     nz_by_order = ([float(np.mean(est.P_[o] != 0)) for o in range(est.P_.shape[0])]
                    if est.P_.ndim == 3 else [nz_frac])
@@ -497,7 +522,7 @@ def psgd_config(args, world, batch_mode):
                             f"pull / push / owner-update per minibatch (no NCCL on the data path)")}
 
 
-def run_psgd_workload(args, rank, world, local, batch_mode="weak"):
+def run_psgd_workload(args, rank, world, local, batch_mode="weak", dump_dir=None):
     """C5: step = one epoch over the rank's shard.  Device-timed value through the estimator's own epoch
     function with X / y / plan resident; e2e = fit(X_host, y_host) wall clock (H2D of X, plan, epochs, D2H)."""
     import ctypes as C
@@ -559,6 +584,13 @@ def run_psgd_workload(args, rank, world, local, batch_mode="weak"):
     torch.cuda.synchronize()
     clocks = sampler.stop() if rank == 0 else None
     ms_total = ev0.elapsed_time(ev1)
+    if dump_dir is not None:
+        # the model after the last timed epoch, as a fit() callback would see it.  On the planned path sync() folds
+        # the lazy scales into the stored model, so the epochs after this point (profiled pass, final read-back) can
+        # differ in the last bits from a run without --dump-outputs; the timed value above is not affected.
+        sync()
+        if rank == 0:
+            dump_outputs(dump_dir, {"P_": est.P_, "w_": est.w_})
     # profiled pass: the same K epochs again with a CUDA-event pair around every kernel class (sp_profile_*, on the
     # launching streams): the kernel durations of the roofline and the per-class figures
     if group is not None:
@@ -775,7 +807,7 @@ def metric_name(name):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=10)
+    ap.add_argument("--steps", type=int, default=10, help="timed epochs of the headline workload")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--workload", default="auto", choices=["auto", "pcd", "pbcd", "allsub", "c1", "psgd"])
@@ -787,6 +819,8 @@ def main():
                     help="psgd global minibatch: 'weak' (auto x n_gpus: per-GPU work fixed) or 'strong' (auto, split over the ranks)")
     ap.add_argument("--no-also", action="store_true", help="skip the secondary workloads")
     ap.add_argument("--gamma", type=float, default=None, help="override the workload's gamma (debug: other sparsity regimes)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write P_ / w_ as the headline workload's timed epochs left them to DIR/<name>.npy (float64, <= 64 MB)")
     args = ap.parse_args()
     rank, world, local = dist_env()
     global ROWS_OVERRIDE
@@ -811,9 +845,9 @@ def main():
         dist.init_process_group("nccl", device_id=torch.device("cuda", local))
     name = args.workload
     if name == "psgd":
-        res = run_psgd_workload(args, rank, world, local, args.psgd_batch)
+        res = run_psgd_workload(args, rank, world, local, args.psgd_batch, args.dump_outputs)
     else:
-        res = run_sweep_workload(name, args, rank, world, local)
+        res = run_sweep_workload(name, args, rank, world, local, args.dump_outputs)
     also = []
     if auto and not args.no_also:
         import copy

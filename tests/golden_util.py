@@ -58,7 +58,6 @@ def same_support(a, b, noise=1e-12):
 # ------------------------------------------------------------------ larger reference fits (oracle/gen_golden_large.py)
 with open(os.path.join(GOLD, "reference_large.json")) as _f:
     LARGE_INDEX = json.load(_f)
-_LARGE = None
 
 
 def large_case_names():
@@ -74,11 +73,9 @@ def large_inputs(prob):
 
 
 def load_large_case(name):
-    global _LARGE
-    if _LARGE is None:
-        _LARGE = np.load(os.path.join(GOLD, "reference_large.npz"))
     rec = next(c for c in LARGE_INDEX if c["name"] == name)
-    arr = {k.split("/", 1)[1]: _LARGE[k] for k in _LARGE.files if k.startswith(name + "/")}
+    with np.load(os.path.join(GOLD, "reference_large", name + ".npz")) as z:
+        arr = {k: z[k] for k in z.files}
     X = large_inputs(rec["prob"])
     nnz, dsum, isum = rec["x_checksum"]
     assert X.nnz == nnz and float(X.data.sum()) == dsum and int(X.indices.astype(np.int64).sum()) == isum, \

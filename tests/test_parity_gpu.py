@@ -490,7 +490,7 @@ def test_device_csc_transpose_matches_scipy():
 @pytest.mark.parametrize("name", large_case_names())
 def test_matches_reference_beyond_toy_sizes(name):
     """CUDA backend against the UNMODIFIED reference at C1 full size (5 and 25 epochs), C2/50, C3/50, C4/10, two
-    Criteo-shaped psgd problems and the omegacs negative-dcache fixture (tests/golden/reference_large.*)."""
+    Criteo-shaped psgd problems and the omegacs negative-dcache fixture (tests/golden/reference_large/)."""
     rec, X, arr = load_large_case(name)
     est = _fit(_estimator(rec), X, arr["y"])
     assert rel_err(est.P_, arr["P_"]) <= TOL
