@@ -189,6 +189,36 @@ int sp_pcd_epoch(const sp_dataset *ds, const sp_plan *plan, double *P_kd, int k,
                  int rec_stride, double *regstate, double *viol, const int32_t *idx_comp_host,
                  sp_stream stream);
 
+/* Many pcd models on one design matrix (fit_many; DESIGN.md 3.2).  One descriptor per model, passed as a
+ * host array.  Every launch of a call covers all models, and each model's sweep is the code the single-model
+ * call runs on that model's P, records and scratch, so its result is bit-identical to sp_pcd_epoch /
+ * sp_cd_linear_epoch with a cluster plan of the same n_cta / threads.  Models may share a plan (the same
+ * coordinate order), never P, rec, regstate or viol.  At most 65535 models per call. */
+typedef struct sp_pcd_model {
+    const int32_t *pos_ptr, *flag_idx, *idx_feat, *pos_conf;  /* the model's cluster plan (sp_plan fields,
+                                                                 built for the call's n_cta) */
+    double *P;                /* P_kd [k,d] of the order (sp_pcd_epoch_multi) or w [d] (sp_cd_linear_epoch_multi) */
+    const double *lams;       /* [k] (unused by the linear sweep) */
+    double ab;                /* beta (pcd) or alpha (linear) */
+    double gamma, eta;        /* unused by the linear sweep */
+    int32_t reg;              /* reg id: l1, squaredl12 or omegati (unused by the linear sweep) */
+    double *rec;              /* [n*rec_stride] the model's sample records */
+    double *regstate;         /* >= 8 doubles of scratch (unused by the linear sweep) */
+    double *viol;             /* the model's running sum of |updates| */
+    const int32_t *idx_comp_host; /* [k] the model's indices_component (unused by the linear sweep) */
+} sp_pcd_model;
+
+/* cd_linear._cd_linear_epoch (cd_linear.py:8-33) of every model: one launch. */
+int sp_cd_linear_epoch_multi(const sp_dataset *ds, int n_cta, int threads, const double *col_norm_sq,
+                             const sp_pcd_model *models, int n_models, int loss, int rec_stride, sp_stream stream);
+
+/* pcd.pcd_epoch (pcd.py:71-137; degree=-1: pcd_all.pcd_epoch, pcd_all.py:44-102) of one order of every model.
+ * Position ss of the component orders is one row-DP launch, one regularizer-cache launch (models other than
+ * l1) and one sweep launch over all models; a model's dead components (the rule of sp_pcd_epoch) get no entry,
+ * and a launch without entries is not issued.  One stream synchronisation per call (the dead-component scan). */
+int sp_pcd_epoch_multi(const sp_dataset *ds, int n_cta, int threads, const sp_pcd_model *models, int n_models,
+                       int k, int degree, int loss, int rec_stride, sp_stream stream);
+
 /* ----------------------------------------------------------------------------------- pbcd */
 /* One pbcd epoch (pbcd.pbcd_epoch, pbcd.py:82-148; degree=-1: pbcd_all.pbcd_epoch,
  * pbcd_all.py:68-132).  P_dk feature-major [d,k]; yrec [n,2] = {y_pred, y};

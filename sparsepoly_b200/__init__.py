@@ -6,9 +6,11 @@ from .estimators import (
     SparseFactorizationMachineClassifier,
     SparseFactorizationMachineRegressor,
 )
+from .multi import fit_many
 from .objective import objective
 
 __all__ = [
+    "fit_many",
     "objective",
     "SparseAllSubsetsClassifier",
     "SparseAllSubsetsRegressor",

@@ -76,6 +76,13 @@ class SpPsgdCtx(C.Structure):
                 ("seq_pull", C.c_uint64), ("aux_stream", _vp), ("aux_event", _vp * 2)]
 
 
+class SpPcdModel(C.Structure):
+    """struct sp_pcd_model (include/sparsepoly_b200.h): one model of sp_pcd_epoch_multi / sp_cd_linear_epoch_multi."""
+    _fields_ = [("pos_ptr", _vp), ("flag_idx", _vp), ("idx_feat", _vp), ("pos_conf", _vp), ("P", _vp),
+                ("lams", _vp), ("ab", C.c_double), ("gamma", C.c_double), ("eta", C.c_double), ("reg", C.c_int32),
+                ("rec", _vp), ("regstate", _vp), ("viol", _vp), ("idx_comp_host", C.POINTER(C.c_int32))]
+
+
 _DSP = C.POINTER(SpDataset)
 _PPP = C.POINTER(SpPsgdPlan)
 _PCP = C.POINTER(SpPsgdCtx)
@@ -107,6 +114,8 @@ SIGNATURES = {
     "sp_cd_linear_epoch": (_i, [_DSP, _PLP, _vp, _vp, _d, _i, _vp, _i, _vp, _vp]),
     "sp_pcd_epoch": (_i, [_DSP, _PLP, _vp, _i, _vp, _i, _d, _d, _d, _i, _i, _vp, _i, _vp, _vp,
                           C.POINTER(C.c_int32), _vp]),
+    "sp_cd_linear_epoch_multi": (_i, [_DSP, _i, _i, _vp, C.POINTER(SpPcdModel), _i, _i, _i, _vp]),
+    "sp_pcd_epoch_multi": (_i, [_DSP, _i, _i, C.POINTER(SpPcdModel), _i, _i, _i, _i, _i, _vp]),
     "sp_pbcd_epoch": (_i, [_DSP, _PLP, _vp, _i, _vp, _i, _d, _d, _d, _i, _i, _vp, _vp, _vp, _vp, _vp,
                            _vp]),
     "sp_get_eta": (_i, [_i, _d, _d, _d, _d, C.c_int64, C.POINTER(_d), C.POINTER(_d)]),

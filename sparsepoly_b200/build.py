@@ -34,7 +34,7 @@ def _stale():
     if not os.path.exists(OUT):
         return True
     t = os.path.getmtime(OUT)
-    deps = [os.path.join(CSRC, f) for f in os.listdir(CSRC) if f.endswith((".cu", ".cuh"))]
+    deps = [os.path.join(CSRC, f) for f in os.listdir(CSRC) if f.endswith((".cu", ".cuh", ".inc"))]
     deps.append(os.path.join(INC, "sparsepoly_b200.h"))
     return any(os.path.getmtime(p) > t for p in deps)
 

@@ -24,6 +24,11 @@ enum { SP_PROF_ROWS = 0, SP_PROF_REGCACHE = 1, SP_PROF_SWEEP_PCD = 2, SP_PROF_SW
 void sp_prof_begin(int cls, cudaStream_t st);
 void sp_prof_end(cudaStream_t st);
 
+// table entries of the many-model launches (sp_pcd_epoch_multi): one component row of one model with its
+// sample records (rows.cu) or regularizer scratch and cache mode (regcache.cu)
+struct SpRowsEntry { const double *p; double *rec; };
+struct SpRegEntry { const double *p; double *regstate; int mode; };
+
 void sp_set_error(const char *fmt, ...);
 int sp_check_cuda(cudaError_t e, const char *what);
 

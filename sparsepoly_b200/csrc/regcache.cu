@@ -11,9 +11,8 @@ namespace {
 //                        in a fixed tree -- all terms are >= 0, so this is well conditioned)
 //   mode 2 (omegati all-subsets): regstate[0] = prod_j (1 + |p_j|)
 constexpr int RC_THREADS = 1024;
-__global__ void __launch_bounds__(RC_THREADS) reg_cache_kernel(int mode, int degree, int d,
-                                                               const double *__restrict__ p,
-                                                               double *regstate) {
+__device__ __forceinline__ void reg_cache_body(int mode, int degree, int d, const double *__restrict__ p,
+                                               double *regstate) {
     __shared__ double sh[RC_THREADS][SP_MAXDEG + 1];
     const int tid = threadIdx.x;
     const int m = mode == 1 ? degree : 0;
@@ -51,6 +50,19 @@ __global__ void __launch_bounds__(RC_THREADS) reg_cache_kernel(int mode, int deg
         for (int t = 0; t <= SP_MAXDEG; t++) regstate[t] = (t <= m) ? sh[0][t] : 0.0;
 }
 
+__global__ void __launch_bounds__(RC_THREADS) reg_cache_kernel(int mode, int degree, int d,
+                                                               const double *__restrict__ p,
+                                                               double *regstate) {
+    reg_cache_body(mode, degree, d, p, regstate);
+}
+
+// many models (sp_pcd_epoch_multi): block b computes the cache of table[b] in that entry's mode
+__global__ void __launch_bounds__(RC_THREADS) reg_cache_multi_kernel(const SpRegEntry *__restrict__ table,
+                                                                     int degree, int d) {
+    const SpRegEntry e = table[blockIdx.x];
+    reg_cache_body(e.mode, degree, d, e.p, e.regstate);
+}
+
 }  // namespace
 
 int sp_launch_reg_cache(int mode, int degree, int d, const double *v, double *regstate, cudaStream_t st) {
@@ -62,5 +74,18 @@ int sp_launch_reg_cache(int mode, int degree, int d, const double *v, double *re
     reg_cache_kernel<<<1, RC_THREADS, 0, st>>>(mode, degree, d, v, regstate);
     sp_prof_end(st);
     SP_LAUNCH_CHECK("reg_cache_kernel");
+    return SP_OK;
+}
+
+int sp_launch_reg_cache_multi(const SpRegEntry *table, int n_tab, int degree, int d, cudaStream_t st) {
+    if (degree != -1 && (degree < 1 || degree > SP_MAXDEG)) {
+        sp_set_error("regularizer cache: degree %d unsupported", degree);
+        return SP_ERR_UNSUPPORTED;
+    }
+    if (n_tab == 0) return SP_OK;
+    sp_prof_begin(SP_PROF_REGCACHE, st);
+    reg_cache_multi_kernel<<<n_tab, RC_THREADS, 0, st>>>(table, degree, d);
+    sp_prof_end(st);
+    SP_LAUNCH_CHECK("reg_cache_multi_kernel");
     return SP_OK;
 }

@@ -115,10 +115,9 @@ rows_all_kernel(int n, int k, const int32_t *__restrict__ indptr, const int32_t 
 // load + parallel gather of p_s[j]); the recurrence itself is run redundantly by all lanes.
 // Writes rec[i*stride + 2 + (t-1)] = A^t(i), t=1..DEG-1 (ANOVA) or rec[i*stride+2] = A(i).
 template <int DEG>
-__global__ void __launch_bounds__(ROWS_THREADS)
-rows_one_kernel(int n, const int32_t *__restrict__ indptr, const int32_t *__restrict__ indices,
-                const double *__restrict__ data, const double *__restrict__ p_s, double *rec,
-                int rec_stride) {
+__device__ __forceinline__ void rows_one_body(int n, const int32_t *__restrict__ indptr,
+                                              const int32_t *__restrict__ indices, const double *__restrict__ data,
+                                              const double *__restrict__ p_s, double *rec, int rec_stride) {
     constexpr int G = 8;
     constexpr int ND = DEG > 0 ? DEG : 1;
     const int lane = threadIdx.x & (G - 1);
@@ -161,6 +160,23 @@ rows_one_kernel(int n, const int32_t *__restrict__ indptr, const int32_t *__rest
             }
         }
     }
+}
+
+template <int DEG>
+__global__ void __launch_bounds__(ROWS_THREADS)
+rows_one_kernel(int n, const int32_t *__restrict__ indptr, const int32_t *__restrict__ indices,
+                const double *__restrict__ data, const double *__restrict__ p_s, double *rec,
+                int rec_stride) {
+    rows_one_body<DEG>(n, indptr, indices, data, p_s, rec, rec_stride);
+}
+
+// many models (sp_pcd_epoch_multi): block row y computes the entry table[y] as rows_one_kernel does
+template <int DEG>
+__global__ void __launch_bounds__(ROWS_THREADS)
+rows_one_multi_kernel(int n, const int32_t *__restrict__ indptr, const int32_t *__restrict__ indices,
+                      const double *__restrict__ data, const SpRowsEntry *__restrict__ table, int rec_stride) {
+    const SpRowsEntry e = table[blockIdx.y];
+    rows_one_body<DEG>(n, indptr, indices, data, e.p, e.rec, rec_stride);
 }
 
 int grid_for(int n, int per_block) {
@@ -266,5 +282,31 @@ int sp_rows_precompute_one(const sp_dataset *ds, const double *p_s, int degree, 
 #undef SP_ONE
     sp_prof_end(st);
     SP_LAUNCH_CHECK("rows_one_kernel");
+    return SP_OK;
+}
+
+// pcd cache precompute of many (model, component) entries in one launch
+int sp_rows_precompute_multi(const sp_dataset *ds, const SpRowsEntry *table, int n_tab, int degree, int rec_stride,
+                             cudaStream_t st) {
+    const int n = ds->n_samples;
+    if (n == 0 || n_tab == 0) return SP_OK;
+    const dim3 grid((unsigned)grid_for(n, ROWS_THREADS / 8), (unsigned)n_tab);
+#define SP_MULTI(D)                                                                                  \
+    rows_one_multi_kernel<D><<<grid, ROWS_THREADS, 0, st>>>(n, ds->csr_indptr, ds->csr_indices,      \
+                                                            ds->csr_data, table, rec_stride)
+    sp_prof_begin(SP_PROF_ROWS, st);
+    switch (degree) {
+    case -1: SP_MULTI(-1); break;
+    case 2: SP_MULTI(2); break;
+    case 3: SP_MULTI(3); break;
+    case 4: SP_MULTI(4); break;
+    case 5: SP_MULTI(5); break;
+    default:
+        sp_set_error("pcd degree %d is not supported (2..%d or -1)", degree, SP_MAXDEG);
+        return SP_ERR_UNSUPPORTED;
+    }
+#undef SP_MULTI
+    sp_prof_end(st);
+    SP_LAUNCH_CHECK("rows_one_multi_kernel");
     return SP_OK;
 }

@@ -250,6 +250,17 @@ class _BaseSparseFactorizationMachine(_SparsePolyBase, metaclass=ABCMeta):
             first = False
         return out
 
+    def _init_coefs(self, n_features, rng):
+        """w_, P_ and lams_ at the start of fit (kept under warm_start); draws P_ then the lambdas from rng."""
+        if not (self.warm_start and hasattr(self, "w_")):
+            self.w_ = np.zeros(n_features, dtype=np.double)
+        n_orders = self.degree - 1 if self.fit_lower == "explicit" else 1
+        if not (self.warm_start and hasattr(self, "P_")):
+            self.P_ = 0.01 * rng.randn(n_orders, self.n_components, n_features)
+        self._init_lambdas(rng)
+        if np.unique(np.abs(self.lams_)) != np.array([1.0]):
+            raise ValueError("Lambdas must be +1 or -1.")
+
     # ---------------------------------------------------------------- pcd
     def _pcd_setup(self, X, y, rng, dev):
         """Move everything to the device and return (epoch, sync): epoch() runs one iteration of
@@ -582,14 +593,7 @@ class _BaseSparseFactorizationMachine(_SparsePolyBase, metaclass=ABCMeta):
         _lib.check(_lib.load().sp_set_device(dev.index if dev.index is not None else 0))
         upload = self._start_upload(X, dev) if self.solver == "psgd" else None
 
-        if not (self.warm_start and hasattr(self, "w_")):
-            self.w_ = np.zeros(n_features, dtype=np.double)
-        n_orders = self.degree - 1 if self.fit_lower == "explicit" else 1
-        if not (self.warm_start and hasattr(self, "P_")):
-            self.P_ = 0.01 * rng.randn(n_orders, self.n_components, n_features)
-        self._init_lambdas(rng)
-        if np.unique(np.abs(self.lams_)) != np.array([1.0]):
-            raise ValueError("Lambdas must be +1 or -1.")
+        self._init_coefs(n_features, rng)
 
         y = np.ascontiguousarray(y, dtype=np.float64)
         if self.solver == "pcd":
@@ -712,9 +716,7 @@ class _BaseSparseAllSubsets(_SparsePolyBase, metaclass=ABCMeta):
         self._check_combination(self.solver, self.regularizer, -1)
         dev = _device()
         _lib.check(_lib.load().sp_set_device(dev.index if dev.index is not None else 0))
-        if not (self.warm_start and hasattr(self, "P_")):
-            self.P_ = 0.01 * rng.randn(k, d)
-        self._init_lambdas(rng)
+        self._init_coefs(d, rng)
         y = np.ascontiguousarray(y, dtype=np.float64)
         epoch, sync = self._setup(X, y, rng, dev)
         converged, it = False, 0
@@ -732,6 +734,12 @@ class _BaseSparseAllSubsets(_SparsePolyBase, metaclass=ABCMeta):
         if not converged:
             warnings.warn("Objective did not converge. Increase max_iter.")
         return self
+
+    def _init_coefs(self, n_features, rng):
+        """P_ and lams_ at the start of fit (kept under warm_start); draws P_ then the lambdas from rng."""
+        if not (self.warm_start and hasattr(self, "P_")):
+            self.P_ = 0.01 * rng.randn(self.n_components, n_features)
+        self._init_lambdas(rng)
 
     def _setup(self, X, y, rng, dev):
         """Move everything to the device and return (epoch, sync): epoch() runs one iteration of

@@ -58,6 +58,19 @@ def pcd_epoch(ds, plan, P_kd, lams, degree, beta, gamma, eta, reg, loss, rec, st
                                  idx.ctypes.data_as(C.POINTER(C.c_int32)), _stream()))
 
 
+def cd_linear_epoch_multi(ds, n_cta, threads, col_norm_sq, models, loss, stride):
+    """cd_linear_epoch of every model of a ctypes SpPcdModel array in one launch (fit_many)."""
+    _lib.check(_L().sp_cd_linear_epoch_multi(ds.ref(), int(n_cta), int(threads), _ptr(col_norm_sq), models,
+                                             len(models), _lib.LOSS_IDS[loss], int(stride), _stream()))
+
+
+def pcd_epoch_multi(ds, n_cta, threads, models, k, degree, loss, stride):
+    """pcd_epoch of one order of every model of a ctypes SpPcdModel array; each launch covers all models
+    (fit_many)."""
+    _lib.check(_L().sp_pcd_epoch_multi(ds.ref(), int(n_cta), int(threads), models, len(models), int(k),
+                                       int(degree), _lib.LOSS_IDS[loss], int(stride), _stream()))
+
+
 def pbcd_epoch(ds, plan, P_dk, lams, degree, beta, gamma, eta, reg, loss, yrec, A, reg_norms, regstate,
                viol):
     """pbcd.pbcd_epoch (pbcd.py:82-148) / pbcd_all.pbcd_epoch (pbcd_all.py:68-132, degree=-1)."""
