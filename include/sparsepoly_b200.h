@@ -228,6 +228,31 @@ int sp_pbcd_epoch(const sp_dataset *ds, const sp_plan *plan, double *P_dk, int k
                   int degree, double beta, double gamma, double eta, int reg, int loss, double *yrec,
                   double *A, double *reg_norms, double *regstate, double *viol, sp_stream stream);
 
+/* Many pbcd models on one design matrix (fit_many; DESIGN.md 3.3).  One descriptor per model, passed as a host
+ * array.  One call runs one order of every model in at most four launches, each covering all models: the row DP,
+ * the row norms and the regularizer caches (only if a model has squaredl21 or omegacs) and the block sweep, one
+ * cluster of n_cta CTAs per model.  Each model's result is bit-identical to sp_pbcd_epoch with a cluster plan of
+ * the same n_cta / threads.  Models may share a plan (the same feature order), never P, yrec, A, reg_norms,
+ * regstate or viol.  At most 65535 models per call. */
+typedef struct sp_pbcd_model {
+    const int32_t *pos_ptr, *flag_idx, *idx_feat;  /* the model's cluster plan (sp_plan fields, built for the
+                                                      call's n_cta) */
+    double *P;                /* P_dk [d,k] of the order, feature-major */
+    const double *lams;       /* [k] */
+    double beta, gamma, eta;
+    int32_t reg;              /* reg id: l1, l21, squaredl21 (degree 2 only) or omegacs */
+    double *yrec;             /* [n,2] {y_pred, y} */
+    double *A;                /* [n,(m-1),k] (ANOVA) or [n,k] (all-subsets) scratch */
+    double *reg_norms;        /* [d] regularizer scratch */
+    double *regstate;         /* >= 16 doubles of regularizer scratch */
+    double *viol;             /* the model's running sum of |updates| */
+} sp_pbcd_model;
+
+/* pbcd.pbcd_epoch (pbcd.py:82-148; degree=-1: pbcd_all.pbcd_epoch, pbcd_all.py:68-132) of one order of every
+ * model.  n_cta: power of two <= 16; threads: multiple of 32 <= 256; k <= 128. */
+int sp_pbcd_epoch_multi(const sp_dataset *ds, int n_cta, int threads, const sp_pbcd_model *models, int n_models,
+                        int k, int degree, int loss, sp_stream stream);
+
 /* ----------------------------------------------------------------------------------- psgd */
 /* (eta_P, eta_w) of psgd._get_eta (psgd.py:9-22); host-side scalar helper. */
 int sp_get_eta(int learning_rate, double eta0, double alpha, double beta, double power_t,

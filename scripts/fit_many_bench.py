@@ -1,10 +1,14 @@
-"""fit_many against the sequential fit loop on three workloads; writes fit_many_bench.json into OUTDIR.
+"""fit_many against the sequential fit loop; writes fit_many_bench.json (fit_many_pbcd_bench.json with
+--solver pbcd) into OUTDIR.
 
-    python scripts/fit_many_bench.py OUTDIR [--epochs-a 20] [--epochs-bc 5]
+    python scripts/fit_many_bench.py OUTDIR [--solver pcd|pbcd] [--epochs-a 20] [--epochs-bc 5]
 
-(a) the reference notebook's grid: n=200, d=100, k=30, degree 2, dense, {l1, squaredl12, omegati} x 8 gamma
+pcd: (a) the reference notebook's grid: n=200, d=100, k=30, degree 2, dense, {l1, squaredl12, omegati} x 8 gamma
     x 4 beta = 96 models;  (b) the C1 shape: synth.uniform_sparse(10000, 1000, 50, 0), k=10, squaredl12,
     16 gamma values;  (c) one-vs-rest, 10 classes on (b)'s X.
+pbcd: (a) the notebook grid with {l21, squaredl21, omegacs};  (b) the C1 shape with l21, 16 gamma values;
+    (c) (b) at k=64, where the cluster sweep is the only pbcd sweep;  (d) one-vs-rest, 10 classes on (b)'s X,
+    omegacs.
 Every workload runs a fixed number of epochs (tol=-1).  Per workload: wall time of fit_many and of the loop of
 single fits (after a warm-up of each), the loop both with the cluster sweep (the bit-identical reference) and
 with the default "auto" sweep; model-epochs per second; launches per epoch by kernel class (sp_profile_*, in a
@@ -52,6 +56,28 @@ def workloads(epochs_a, epochs_bc):
             ("c_one_vs_rest_10", ovr, Xb, [(labels == c).astype(float) for c in range(10)])]
 
 
+def workloads_pbcd(epochs_a, epochs_bc):
+    rng = np.random.RandomState(0)
+    Xa = rng.randn(200, 100)
+    ya = Xa[:, :5].sum(1) + 0.1 * rng.randn(200)
+    grid = [S.SparseFactorizationMachineRegressor(degree=2, n_components=30, solver="pbcd", regularizer=reg, beta=b,
+                                                   gamma=g, max_iter=epochs_a, tol=-1, random_state=0)
+            for reg in ("l21", "squaredl21", "omegacs") for g in np.logspace(-4, -0.5, 8) for b in (1e-3, 1e-2, 0.1, 1.0)]
+    Xb = synth.uniform_sparse(10_000, 1_000, 50, 0)
+    yb = np.where(np.asarray(Xb[:, :20].sum(1)).ravel() > np.median(np.asarray(Xb[:, :20].sum(1))), 1.0, -1.0)
+
+    def c1(k, reg, gamma):
+        return S.SparseFactorizationMachineClassifier(degree=2, n_components=k, solver="pbcd", regularizer=reg,
+                                                      loss="logistic", beta=1e-3, gamma=gamma, max_iter=epochs_bc,
+                                                      tol=-1, random_state=0)
+    labels = np.random.RandomState(1).randint(0, 10, Xb.shape[0])
+    return [("a_notebook_grid", grid, Xa, ya),
+            ("b_c1_shape_l21_gamma16", [c1(10, "l21", g) for g in np.logspace(-5, -1, 16)], Xb, yb),
+            ("c_c1_shape_k64_gamma16", [c1(64, "l21", g) for g in np.logspace(-5, -1, 16)], Xb, yb),
+            ("d_one_vs_rest_10", [c1(10, "omegacs", 1e-3) for _ in range(10)], Xb,
+             [(labels == c).astype(float) for c in range(10)])]
+
+
 def _quiet(fn):
     with warnings.catch_warnings():
         warnings.simplefilter("ignore")
@@ -92,6 +118,7 @@ def gpu_info():
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("outdir")
+    ap.add_argument("--solver", choices=("pcd", "pbcd"), default="pcd")
     ap.add_argument("--epochs-a", type=int, default=20)
     ap.add_argument("--epochs-bc", type=int, default=5)
     args = ap.parse_args()
@@ -99,7 +126,8 @@ def main():
         raise SystemExit("fit_many_bench needs a CUDA device")
     torch.cuda.set_device(0)
     result = {"gpu": gpu_info(), "torch": torch.__version__, "workloads": {}}
-    for name, ests, X, y in workloads(args.epochs_a, args.epochs_bc):
+    make = workloads_pbcd if args.solver == "pbcd" else workloads
+    for name, ests, X, y in make(args.epochs_a, args.epochs_bc):
         ys = y if isinstance(y, list) else [y] * len(ests)
         epochs = ests[0].max_iter
         rec = {"models": len(ests), "epochs": epochs, "shape": list(X.shape)}
@@ -125,7 +153,8 @@ def main():
         result["workloads"][name] = rec
         print(name, json.dumps(rec), flush=True)
     os.makedirs(args.outdir, exist_ok=True)
-    with open(os.path.join(args.outdir, "fit_many_bench.json"), "w") as f:
+    out = "fit_many_pbcd_bench.json" if args.solver == "pbcd" else "fit_many_bench.json"
+    with open(os.path.join(args.outdir, out), "w") as f:
         json.dump(result, f, indent=1)
 
 

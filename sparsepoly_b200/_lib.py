@@ -83,6 +83,13 @@ class SpPcdModel(C.Structure):
                 ("rec", _vp), ("regstate", _vp), ("viol", _vp), ("idx_comp_host", C.POINTER(C.c_int32))]
 
 
+class SpPbcdModel(C.Structure):
+    """struct sp_pbcd_model (include/sparsepoly_b200.h): one model of sp_pbcd_epoch_multi."""
+    _fields_ = [("pos_ptr", _vp), ("flag_idx", _vp), ("idx_feat", _vp), ("P", _vp), ("lams", _vp),
+                ("beta", C.c_double), ("gamma", C.c_double), ("eta", C.c_double), ("reg", C.c_int32),
+                ("yrec", _vp), ("A", _vp), ("reg_norms", _vp), ("regstate", _vp), ("viol", _vp)]
+
+
 _DSP = C.POINTER(SpDataset)
 _PPP = C.POINTER(SpPsgdPlan)
 _PCP = C.POINTER(SpPsgdCtx)
@@ -118,6 +125,7 @@ SIGNATURES = {
     "sp_pcd_epoch_multi": (_i, [_DSP, _i, _i, C.POINTER(SpPcdModel), _i, _i, _i, _i, _i, _vp]),
     "sp_pbcd_epoch": (_i, [_DSP, _PLP, _vp, _i, _vp, _i, _d, _d, _d, _i, _i, _vp, _vp, _vp, _vp, _vp,
                            _vp]),
+    "sp_pbcd_epoch_multi": (_i, [_DSP, _i, _i, C.POINTER(SpPbcdModel), _i, _i, _i, _i, _vp]),
     "sp_get_eta": (_i, [_i, _d, _d, _d, _d, C.c_int64, C.POINTER(_d), C.POINTER(_d)]),
     "sp_psgd_grad": (_i, [_DSP, _vp, _vp, _i, _i, _vp, _vp, _i, _i, _i, _vp, _i, _i, _vp, _vp, _vp, _vp]),
     "sp_psgd_step": (_i, [_vp, _vp, _vp, _vp, _i, _i, _i, _d, _d, _d, _d, _i, _i, _vp]),

@@ -28,6 +28,14 @@ void sp_prof_end(cudaStream_t st);
 // sample records (rows.cu) or regularizer scratch and cache mode (regcache.cu)
 struct SpRowsEntry { const double *p; double *rec; };
 struct SpRegEntry { const double *p; double *regstate; int mode; };
+// sp_pbcd_epoch_multi: one model's feature-major P_dk [d,k] and what is computed from it (the row-DP cache A in
+// rows.cu, the row norms in pbcd.cu)
+struct SpBlockEntry { const double *P; double *out; };
+
+// pinned host staging of the many-model argument tables (pcd.cu): acquire waits until the copy that last read
+// the buffer has completed; upload copies its first `bytes` to the device and records that copy
+int sp_stage_acquire(size_t bytes, unsigned char **out);
+int sp_stage_upload(void *dst, size_t bytes, cudaStream_t st);
 
 void sp_set_error(const char *fmt, ...);
 int sp_check_cuda(cudaError_t e, const char *what);

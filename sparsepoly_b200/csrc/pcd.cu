@@ -354,8 +354,8 @@ extern "C" int sp_pcd_epoch(const sp_dataset *ds, const sp_plan *plan, double *P
 // the code a single sp_pcd_epoch / sp_cd_linear_epoch runs on that model's own records, P and scratch.
 namespace {
 
-// Pinned host staging of the argument tables.  It is rewritten only after the copy that last read it has
-// completed: `copied` is recorded behind every copy out of it.
+// Pinned host staging of the argument tables (also used by sp_pbcd_epoch_multi).  It is rewritten only after
+// the copy that last read it has completed: `copied` is recorded behind every copy out of it.
 struct Staging {
     unsigned char *host = nullptr;
     size_t cap = 0;
@@ -364,7 +364,9 @@ struct Staging {
 };
 thread_local Staging g_stage;
 
-int stage_acquire(size_t bytes, unsigned char **out) {
+}  // namespace
+
+int sp_stage_acquire(size_t bytes, unsigned char **out) {
     Staging &s = g_stage;
     int dev = 0;
     SP_CUDA(cudaGetDevice(&dev));
@@ -392,11 +394,13 @@ int stage_acquire(size_t bytes, unsigned char **out) {
     return SP_OK;
 }
 
-int stage_upload(void *dst, size_t bytes, cudaStream_t st) {
+int sp_stage_upload(void *dst, size_t bytes, cudaStream_t st) {
     SP_CUDA(cudaMemcpyAsync(dst, g_stage.host, bytes, cudaMemcpyHostToDevice, st));
     SP_CUDA(cudaEventRecord(g_stage.copied, st));
     return SP_OK;
 }
+
+namespace {
 
 constexpr int MULTI_MAX_MODELS = 65535;   // gridDim.y of the row-DP and dead-scan launches
 
@@ -445,7 +449,7 @@ extern "C" int sp_cd_linear_epoch_multi(const sp_dataset *ds, int n_cta, int thr
     cudaStream_t st = (cudaStream_t)stream;
     const size_t bytes = sizeof(SweepArgs) * n_models;
     unsigned char *h = nullptr;
-    rc = stage_acquire(bytes, &h);
+    rc = sp_stage_acquire(bytes, &h);
     if (rc) return rc;
     SweepArgs *tab = reinterpret_cast<SweepArgs *>(h);
     for (int b = 0; b < n_models; b++) {
@@ -457,7 +461,7 @@ extern "C" int sp_cd_linear_epoch_multi(const sp_dataset *ds, int n_cta, int thr
     const SweepArgs first = tab[0];
     SweepArgs *dtab = nullptr;
     SP_CUDA(cudaMallocAsync((void **)&dtab, bytes, st));
-    rc = stage_upload(dtab, bytes, st);
+    rc = sp_stage_upload(dtab, bytes, st);
     if (!rc) {
         sp_plan pl = {n_cta, threads, nullptr, nullptr, nullptr, nullptr, nullptr};
         rc = dispatch_loss<KIND_LINEAR, 1>(loss, first, dtab, n_models, threads, pick_nz(ds, &pl), st);
@@ -518,7 +522,7 @@ extern "C" int sp_pcd_epoch_multi(const sp_dataset *ds, int n_cta, int threads, 
     if (!scanned.empty()) {
         const int ns = (int)scanned.size();
         unsigned char *h = nullptr;
-        rc = stage_acquire(sizeof(double *) * ns, &h);
+        rc = sp_stage_acquire(sizeof(double *) * ns, &h);
         if (rc) return rc;
         const double **hp = reinterpret_cast<const double **>(h);
         for (int i = 0; i < ns; i++) hp[i] = models[scanned[i]].P;
@@ -527,7 +531,7 @@ extern "C" int sp_pcd_epoch_multi(const sp_dataset *ds, int n_cta, int threads, 
         const double **dP = reinterpret_cast<const double **>(buf);
         int *flags = reinterpret_cast<int *>(dP + ns);
         std::vector<int> f((size_t)ns * k);
-        rc = stage_upload(dP, sizeof(double *) * ns, st);
+        rc = sp_stage_upload(dP, sizeof(double *) * ns, st);
         cudaError_t e1 = cudaSuccess;
         if (!rc) {
             row_any_nonzero_multi_kernel<<<dim3((unsigned)k, (unsigned)ns), 256, 0, st>>>(dP, d, k, flags);
@@ -570,7 +574,7 @@ extern "C" int sp_pcd_epoch_multi(const sp_dataset *ds, int n_cta, int threads, 
     const size_t b_sw = sizeof(SweepArgs) * sw.size(), b_rw = sizeof(SpRowsEntry) * rw.size();
     const size_t bytes = b_sw + b_rw + sizeof(SpRegEntry) * rg.size();
     unsigned char *h = nullptr;
-    rc = stage_acquire(bytes, &h);
+    rc = sp_stage_acquire(bytes, &h);
     if (rc) return rc;
     memcpy(h, sw.data(), b_sw);
     memcpy(h + b_sw, rw.data(), b_rw);
@@ -580,7 +584,7 @@ extern "C" int sp_pcd_epoch_multi(const sp_dataset *ds, int n_cta, int threads, 
     const SweepArgs *dsw = reinterpret_cast<const SweepArgs *>(dbuf);
     const SpRowsEntry *drw = reinterpret_cast<const SpRowsEntry *>(dbuf + b_sw);
     const SpRegEntry *drg = reinterpret_cast<const SpRegEntry *>(dbuf + b_sw + b_rw);
-    rc = stage_upload(dbuf, bytes, st);
+    rc = sp_stage_upload(dbuf, bytes, st);
     for (int ss = 0; ss < k && !rc; ss++) {
         const int n = sw_off[ss + 1] - sw_off[ss], nr = rg_off[ss + 1] - rg_off[ss];
         if (n == 0) continue;

@@ -28,86 +28,25 @@ rows_all_kernel(int n, int k, const int32_t *__restrict__ indptr, const int32_t 
                 const double *__restrict__ data, const double *__restrict__ P_dk,
                 const double *__restrict__ lams, const double *__restrict__ w, double *out,
                 int out_stride, int accumulate, double *Aout) {
-    constexpr int ND = DEG > 0 ? DEG : 1;
-    const int lane = threadIdx.x & (G - 1);
-    const unsigned gmask = (G == 32) ? 0xffffffffu
-                                     : (((1u << G) - 1u) << ((threadIdx.x & 31) & ~(G - 1)));
-    const int groups_per_block = ROWS_THREADS / G;
-    const int group = blockIdx.x * groups_per_block + threadIdx.x / G;
-    const int n_groups = gridDim.x * groups_per_block;
-    for (int i = group; i < n; i += n_groups) {
-        const int st = indptr[i], en = indptr[i + 1];
-        double ypred = 0.0;
-        if (MODE == 0 && w != nullptr) {
-            // linear term <w, x_i>; tree order (reference: safe_sparse_dot)
-            double acc = 0.0;
-            for (int e = st + lane; e < en; e += G) acc += data[e] * w[indices[e]];
-#pragma unroll
-            for (int m = G / 2; m > 0; m >>= 1) acc += __shfl_xor_sync(gmask, acc, m, G);
-            ypred = acc;
-        }
-        for (int s0 = 0; s0 < k; s0 += G) {
-            const int s = s0 + lane;
-            const bool act = s < k;
-            double A[ND + 1];
-            A[0] = 1.0;
-#pragma unroll
-            for (int t = 1; t <= ND; t++) A[t] = (DEG > 0) ? 0.0 : 1.0;
-            for (int base = st; base < en; base += G) {
-                const int e = base + lane;
-                int jl = 0;
-                double xl = 0.0;
-                if (e < en) { jl = indices[e]; xl = data[e]; }
-                const int cnt = min(G, en - base);
-                for (int q0 = 0; q0 < cnt; q0 += 8) {
-                    double pv[8], xv[8];
-#pragma unroll
-                    for (int u = 0; u < 8; u++) {      // 8 independent row gathers in flight
-                        const int q = q0 + u;
-                        const int j = __shfl_sync(gmask, jl, q & (G - 1), G);
-                        xv[u] = __shfl_sync(gmask, xl, q & (G - 1), G);
-                        pv[u] = (q < cnt && act) ? P_dk[(size_t)j * k + s] : 0.0;
-                    }
-#pragma unroll
-                    for (int u = 0; u < 8; u++) {
-                        if (q0 + u < cnt) {
-                            if (DEG > 0) {
-#pragma unroll
-                                for (int t = 0; t < ND; t++) {
-                                    const double a = A[ND - t - 1];
-                                    const double inc = PX ? (a * pv[u]) * xv[u] : (a * xv[u]) * pv[u];
-                                    A[ND - t] += inc;
-                                }
-                            } else {
-                                // kernels.py:129 (1 + x*p); pcd_all.py:18 / pbcd_all.py:20 (1.0 + p*x)
-                                A[1] *= 1.0 + (PX ? pv[u] * xv[u] : xv[u] * pv[u]);
-                            }
-                        }
-                    }
-                }
-            }
-            if (MODE == 0) {
-                double v = act ? lams[s] * A[ND] : 0.0;
-#pragma unroll
-                for (int m = G / 2; m > 0; m >>= 1) v += __shfl_xor_sync(gmask, v, m, G);
-                ypred += v;
-            } else if (MODE == 2) {
-                if (act) Aout[(size_t)i * k + s] = A[ND];
-            } else if (act) {
-                if (DEG > 0) {
-#pragma unroll
-                    for (int t = 1; t < ND; t++)
-                        Aout[((size_t)i * (ND - 1) + (t - 1)) * k + s] = A[t];
-                } else {
-                    Aout[(size_t)i * k + s] = A[1];
-                }
-            }
-        }
-        if (MODE == 0 && lane == 0) {
-            double *o = out + (size_t)i * out_stride;
-            *o = accumulate ? (*o + ypred) : ypred;
-        }
-    }
+#include "rows_all_body.inc"
+}
+
+// many models (sp_pbcd_epoch_multi): block row y computes the pbcd cache (MODE 1, PX) of the entry table[y]
+// {P_dk, A} as rows_all_kernel does.  With the single kernel's register budget ptxas spills in 5 of the 15
+// instantiations; at three CTAs per SM none spills (72..80 registers).
+template <int DEG, int G>
+__global__ void __launch_bounds__(ROWS_THREADS, 3)
+rows_all_multi_kernel(int n, int k, const int32_t *__restrict__ indptr, const int32_t *__restrict__ indices,
+                      const double *__restrict__ data, const SpBlockEntry *__restrict__ table) {
+    constexpr int MODE = 1;
+    constexpr bool PX = true;
+    const SpBlockEntry e = table[blockIdx.y];
+    const double *__restrict__ P_dk = e.P;
+    const double *__restrict__ lams = nullptr;
+    const double *__restrict__ w = nullptr;
+    double *out = nullptr, *Aout = e.out;
+    const int out_stride = 1, accumulate = 0;
+#include "rows_all_body.inc"
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -257,6 +196,44 @@ int sp_rows_precompute_all(const sp_dataset *ds, const double *P_dk, int k, int 
     if (ds->n_samples == 0) return SP_OK;
     return dispatch_all<1, true>(degree, ds->n_samples, k, ds->csr_indptr, ds->csr_indices,
                                  ds->csr_data, P_dk, nullptr, nullptr, nullptr, 1, 0, A, st);
+}
+
+// pbcd cache precompute of many models in one launch: entry y is {P_dk, A} of one model; the group width is
+// the one launch_all picks for k
+namespace {
+template <int DEG>
+void launch_all_multi(int n, int k, const sp_dataset *ds, const SpBlockEntry *table, int n_tab, cudaStream_t st) {
+    if (k <= 8) {
+        rows_all_multi_kernel<DEG, 8><<<dim3(grid_for(n, ROWS_THREADS / 8), n_tab), ROWS_THREADS, 0, st>>>(
+            n, k, ds->csr_indptr, ds->csr_indices, ds->csr_data, table);
+    } else if (k <= 16) {
+        rows_all_multi_kernel<DEG, 16><<<dim3(grid_for(n, ROWS_THREADS / 16), n_tab), ROWS_THREADS, 0, st>>>(
+            n, k, ds->csr_indptr, ds->csr_indices, ds->csr_data, table);
+    } else {
+        rows_all_multi_kernel<DEG, 32><<<dim3(grid_for(n, ROWS_THREADS / 32), n_tab), ROWS_THREADS, 0, st>>>(
+            n, k, ds->csr_indptr, ds->csr_indices, ds->csr_data, table);
+    }
+}
+}  // namespace
+
+int sp_rows_precompute_all_multi(const sp_dataset *ds, const SpBlockEntry *table, int n_tab, int k, int degree,
+                                 cudaStream_t st) {
+    const int n = ds->n_samples;
+    if (n == 0 || n_tab == 0) return SP_OK;
+    sp_prof_begin(SP_PROF_ROWS, st);
+    switch (degree) {
+    case -1: launch_all_multi<-1>(n, k, ds, table, n_tab, st); break;
+    case 2: launch_all_multi<2>(n, k, ds, table, n_tab, st); break;
+    case 3: launch_all_multi<3>(n, k, ds, table, n_tab, st); break;
+    case 4: launch_all_multi<4>(n, k, ds, table, n_tab, st); break;
+    case 5: launch_all_multi<5>(n, k, ds, table, n_tab, st); break;
+    default:
+        sp_set_error("pbcd degree %d is not supported (2..%d or -1)", degree, SP_MAXDEG);
+        return SP_ERR_UNSUPPORTED;
+    }
+    sp_prof_end(st);
+    SP_LAUNCH_CHECK("rows_all_multi_kernel");
+    return SP_OK;
 }
 
 // pcd cache precompute (one component) into the record array

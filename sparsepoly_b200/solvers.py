@@ -80,6 +80,13 @@ def pbcd_epoch(ds, plan, P_dk, lams, degree, beta, gamma, eta, reg, loss, yrec, 
                                   _ptr(reg_norms), _ptr(regstate), _ptr(viol), _stream()))
 
 
+def pbcd_epoch_multi(ds, n_cta, threads, models, k, degree, loss):
+    """pbcd_epoch of one order of every model of a ctypes SpPbcdModel array; each launch covers all models
+    (fit_many)."""
+    _lib.check(_L().sp_pbcd_epoch_multi(ds.ref(), int(n_cta), int(threads), models, len(models), int(k),
+                                        int(degree), _lib.LOSS_IDS[loss], _stream()))
+
+
 def get_eta(learning_rate, eta0, alpha, beta, power_t, it):
     """psgd._get_eta (psgd.py:9-22)."""
     a, b = C.c_double(), C.c_double()
