@@ -24,16 +24,17 @@ enum { SP_PROF_ROWS = 0, SP_PROF_REGCACHE = 1, SP_PROF_SWEEP_PCD = 2, SP_PROF_SW
 void sp_prof_begin(int cls, cudaStream_t st);
 void sp_prof_end(cudaStream_t st);
 
-// table entries of the many-model launches (sp_pcd_epoch_multi): one component row of one model with its
-// sample records (rows.cu) or regularizer scratch and cache mode (regcache.cu)
+// table entries of the pcd / pbcd launches (a single fit is a table of one model): one component row of one model
+// with its sample records (rows.cu), or a vector with the regularizer scratch and cache mode computed from it
+// (regcache.cu)
 struct SpRowsEntry { const double *p; double *rec; };
 struct SpRegEntry { const double *p; double *regstate; int mode; };
-// sp_pbcd_epoch_multi: one model's feature-major P_dk [d,k] and what is computed from it (the row-DP cache A in
-// rows.cu, the row norms in pbcd.cu)
+// pbcd: one model's feature-major P_dk [d,k] and what is computed from it (the row-DP cache A in rows.cu, the row
+// norms in pbcd.cu)
 struct SpBlockEntry { const double *P; double *out; };
 
-// pinned host staging of the many-model argument tables (pcd.cu): acquire waits until the copy that last read
-// the buffer has completed; upload copies its first `bytes` to the device and records that copy
+// pinned host staging of the argument tables (pcd.cu): acquire waits until the copy that last read the buffer has
+// completed; upload copies its first `bytes` to the device and records that copy
 int sp_stage_acquire(size_t bytes, unsigned char **out);
 int sp_stage_upload(void *dst, size_t bytes, cudaStream_t st);
 

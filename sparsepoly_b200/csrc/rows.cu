@@ -18,26 +18,25 @@ constexpr int ROWS_THREADS = 256;
 // ---------------------------------------------------------------------------------------------
 // all-components kernel: one group of G lanes per sample, lanes over components.
 //   MODE 0: out[i*out_stride] (+)= sum_j x w_j + sum_s lam_s * K_s(i)      (predict)
-//   MODE 1: Aout[i, t-1, s] = A^t_s(i), t=1..DEG-1  (ANOVA)  /  Aout[i, s] = A_s(i) (all-subsets)
 //   MODE 2: Aout[i, s] = K_s(i) (the Gram matrix of kernels.anova_kernel / all_subsets_kernel)
-// PX=true  : A += (A*p)*x   (pcd.py:30, pbcd.py:33)
-// PX=false : A += (A*x)*p   (psgd.py:44)
-template <int DEG, int G, int MODE, bool PX>
+template <int DEG, int G, int MODE>
 __global__ void __launch_bounds__(ROWS_THREADS)
 rows_all_kernel(int n, int k, const int32_t *__restrict__ indptr, const int32_t *__restrict__ indices,
                 const double *__restrict__ data, const double *__restrict__ P_dk,
                 const double *__restrict__ lams, const double *__restrict__ w, double *out,
                 int out_stride, int accumulate, double *Aout) {
+    constexpr bool PX = false;
 #include "rows_all_body.inc"
 }
 
-// many models (sp_pbcd_epoch_multi): block row y computes the pbcd cache (MODE 1, PX) of the entry table[y]
-// {P_dk, A} as rows_all_kernel does.  With the single kernel's register budget ptxas spills in 5 of the 15
-// instantiations; at three CTAs per SM none spills (72..80 registers).
+// pbcd cache precompute (pbcd._precompute_A_all_degree / pbcd_all._precompute_A_all): block row y writes the cache
+// of the entry table[y] {P_dk, A}: A[i, t-1, s] = A^t_s(i), t=1..DEG-1 (ANOVA) / A[i, s] = A_s(i) (all-subsets), with
+// A += (A*p)*x (pcd.py:30, pbcd.py:33).  At three CTAs per SM ptxas spills in none of the instantiations (72..80
+// registers); with the budget of rows_all_kernel it spills in 5 of the 15.
 template <int DEG, int G>
 __global__ void __launch_bounds__(ROWS_THREADS, 3)
-rows_all_multi_kernel(int n, int k, const int32_t *__restrict__ indptr, const int32_t *__restrict__ indices,
-                      const double *__restrict__ data, const SpBlockEntry *__restrict__ table) {
+rows_pbcd_cache_kernel(int n, int k, const int32_t *__restrict__ indptr, const int32_t *__restrict__ indices,
+                       const double *__restrict__ data, const SpBlockEntry *__restrict__ table) {
     constexpr int MODE = 1;
     constexpr bool PX = true;
     const SpBlockEntry e = table[blockIdx.y];
@@ -50,13 +49,16 @@ rows_all_multi_kernel(int n, int k, const int32_t *__restrict__ indptr, const in
 }
 
 // ---------------------------------------------------------------------------------------------
-// single-component kernel for pcd: 8 lanes per sample; lanes own nonzeros (coalesced idx/val
-// load + parallel gather of p_s[j]); the recurrence itself is run redundantly by all lanes.
-// Writes rec[i*stride + 2 + (t-1)] = A^t(i), t=1..DEG-1 (ANOVA) or rec[i*stride+2] = A(i).
+// pcd cache precompute (one component per entry): block row y computes the entry table[y] {p_s, rec}.  8 lanes per
+// sample; lanes own nonzeros (coalesced idx/val load + parallel gather of p_s[j]); the recurrence itself is run
+// redundantly by all lanes.  Writes rec[i*stride + 2 + (t-1)] = A^t(i), t=1..DEG-1 (ANOVA) or rec[i*stride+2] = A(i).
 template <int DEG>
-__device__ __forceinline__ void rows_one_body(int n, const int32_t *__restrict__ indptr,
-                                              const int32_t *__restrict__ indices, const double *__restrict__ data,
-                                              const double *__restrict__ p_s, double *rec, int rec_stride) {
+__global__ void __launch_bounds__(ROWS_THREADS)
+rows_one_kernel(int n, const int32_t *__restrict__ indptr, const int32_t *__restrict__ indices,
+                const double *__restrict__ data, const SpRowsEntry *__restrict__ table, int rec_stride) {
+    const SpRowsEntry ent = table[blockIdx.y];
+    const double *__restrict__ p_s = ent.p;
+    double *rec = ent.rec;
     constexpr int G = 8;
     constexpr int ND = DEG > 0 ? DEG : 1;
     const int lane = threadIdx.x & (G - 1);
@@ -101,23 +103,6 @@ __device__ __forceinline__ void rows_one_body(int n, const int32_t *__restrict__
     }
 }
 
-template <int DEG>
-__global__ void __launch_bounds__(ROWS_THREADS)
-rows_one_kernel(int n, const int32_t *__restrict__ indptr, const int32_t *__restrict__ indices,
-                const double *__restrict__ data, const double *__restrict__ p_s, double *rec,
-                int rec_stride) {
-    rows_one_body<DEG>(n, indptr, indices, data, p_s, rec, rec_stride);
-}
-
-// many models (sp_pcd_epoch_multi): block row y computes the entry table[y] as rows_one_kernel does
-template <int DEG>
-__global__ void __launch_bounds__(ROWS_THREADS)
-rows_one_multi_kernel(int n, const int32_t *__restrict__ indptr, const int32_t *__restrict__ indices,
-                      const double *__restrict__ data, const SpRowsEntry *__restrict__ table, int rec_stride) {
-    const SpRowsEntry e = table[blockIdx.y];
-    rows_one_body<DEG>(n, indptr, indices, data, e.p, e.rec, rec_stride);
-}
-
 int grid_for(int n, int per_block) {
     long long blocks = ((long long)n + per_block - 1) / per_block;
     const long long cap = 148LL * 8 * 4;   // a few waves of 8 resident CTAs per SM
@@ -126,19 +111,19 @@ int grid_for(int n, int per_block) {
     return (int)blocks;
 }
 
-template <int DEG, int MODE, bool PX>
+template <int DEG, int MODE>
 int launch_all(int n, int k, const int32_t *indptr, const int32_t *indices, const double *data,
                const double *P_dk, const double *lams, const double *w, double *out, int out_stride,
                int accumulate, double *Aout, cudaStream_t st) {
     sp_prof_begin(SP_PROF_ROWS, st);
     if (k <= 8) {
-        rows_all_kernel<DEG, 8, MODE, PX><<<grid_for(n, ROWS_THREADS / 8), ROWS_THREADS, 0, st>>>(
+        rows_all_kernel<DEG, 8, MODE><<<grid_for(n, ROWS_THREADS / 8), ROWS_THREADS, 0, st>>>(
             n, k, indptr, indices, data, P_dk, lams, w, out, out_stride, accumulate, Aout);
     } else if (k <= 16) {
-        rows_all_kernel<DEG, 16, MODE, PX><<<grid_for(n, ROWS_THREADS / 16), ROWS_THREADS, 0, st>>>(
+        rows_all_kernel<DEG, 16, MODE><<<grid_for(n, ROWS_THREADS / 16), ROWS_THREADS, 0, st>>>(
             n, k, indptr, indices, data, P_dk, lams, w, out, out_stride, accumulate, Aout);
     } else {
-        rows_all_kernel<DEG, 32, MODE, PX><<<grid_for(n, ROWS_THREADS / 32), ROWS_THREADS, 0, st>>>(
+        rows_all_kernel<DEG, 32, MODE><<<grid_for(n, ROWS_THREADS / 32), ROWS_THREADS, 0, st>>>(
             n, k, indptr, indices, data, P_dk, lams, w, out, out_stride, accumulate, Aout);
     }
     sp_prof_end(st);
@@ -146,20 +131,35 @@ int launch_all(int n, int k, const int32_t *indptr, const int32_t *indices, cons
     return SP_OK;
 }
 
-template <int MODE, bool PX>
+template <int MODE>
 int dispatch_all(int degree, int n, int k, const int32_t *indptr, const int32_t *indices,
                  const double *data, const double *P_dk, const double *lams, const double *w,
                  double *out, int out_stride, int accumulate, double *Aout, cudaStream_t st) {
     switch (degree) {
-    case -1: return launch_all<-1, MODE, PX>(n, k, indptr, indices, data, P_dk, lams, w, out, out_stride, accumulate, Aout, st);
-    case 1: return launch_all<1, MODE, PX>(n, k, indptr, indices, data, P_dk, lams, w, out, out_stride, accumulate, Aout, st);
-    case 2: return launch_all<2, MODE, PX>(n, k, indptr, indices, data, P_dk, lams, w, out, out_stride, accumulate, Aout, st);
-    case 3: return launch_all<3, MODE, PX>(n, k, indptr, indices, data, P_dk, lams, w, out, out_stride, accumulate, Aout, st);
-    case 4: return launch_all<4, MODE, PX>(n, k, indptr, indices, data, P_dk, lams, w, out, out_stride, accumulate, Aout, st);
-    case 5: return launch_all<5, MODE, PX>(n, k, indptr, indices, data, P_dk, lams, w, out, out_stride, accumulate, Aout, st);
+    case -1: return launch_all<-1, MODE>(n, k, indptr, indices, data, P_dk, lams, w, out, out_stride, accumulate, Aout, st);
+    case 1: return launch_all<1, MODE>(n, k, indptr, indices, data, P_dk, lams, w, out, out_stride, accumulate, Aout, st);
+    case 2: return launch_all<2, MODE>(n, k, indptr, indices, data, P_dk, lams, w, out, out_stride, accumulate, Aout, st);
+    case 3: return launch_all<3, MODE>(n, k, indptr, indices, data, P_dk, lams, w, out, out_stride, accumulate, Aout, st);
+    case 4: return launch_all<4, MODE>(n, k, indptr, indices, data, P_dk, lams, w, out, out_stride, accumulate, Aout, st);
+    case 5: return launch_all<5, MODE>(n, k, indptr, indices, data, P_dk, lams, w, out, out_stride, accumulate, Aout, st);
     default:
         sp_set_error("degree %d is not supported (1..%d or -1 for all-subsets)", degree, SP_MAXDEG);
         return SP_ERR_UNSUPPORTED;
+    }
+}
+
+// the pbcd cache of n_tab entries {P_dk, A} in one launch, with the group width launch_all picks for k
+template <int DEG>
+void launch_pbcd_cache(int n, int k, const sp_dataset *ds, const SpBlockEntry *table, int n_tab, cudaStream_t st) {
+    if (k <= 8) {
+        rows_pbcd_cache_kernel<DEG, 8><<<dim3(grid_for(n, ROWS_THREADS / 8), n_tab), ROWS_THREADS, 0, st>>>(
+            n, k, ds->csr_indptr, ds->csr_indices, ds->csr_data, table);
+    } else if (k <= 16) {
+        rows_pbcd_cache_kernel<DEG, 16><<<dim3(grid_for(n, ROWS_THREADS / 16), n_tab), ROWS_THREADS, 0, st>>>(
+            n, k, ds->csr_indptr, ds->csr_indices, ds->csr_data, table);
+    } else {
+        rows_pbcd_cache_kernel<DEG, 32><<<dim3(grid_for(n, ROWS_THREADS / 32), n_tab), ROWS_THREADS, 0, st>>>(
+            n, k, ds->csr_indptr, ds->csr_indices, ds->csr_data, table);
     }
 }
 
@@ -173,9 +173,9 @@ extern "C" int sp_predict(const sp_dataset *ds, const double *P_dk, int k, const
         return SP_ERR_INVALID;
     }
     if (ds->n_samples == 0) return SP_OK;
-    return dispatch_all<0, false>(degree, ds->n_samples, k, ds->csr_indptr, ds->csr_indices,
-                                  ds->csr_data, P_dk, lams, w, out, out_stride, accumulate, nullptr,
-                                  (cudaStream_t)stream);
+    return dispatch_all<0>(degree, ds->n_samples, k, ds->csr_indptr, ds->csr_indices,
+                           ds->csr_data, P_dk, lams, w, out, out_stride, accumulate, nullptr,
+                           (cudaStream_t)stream);
 }
 
 extern "C" int sp_kernel_matrix(const sp_dataset *ds, const double *P_dk, int k, int degree, double *K,
@@ -185,66 +185,42 @@ extern "C" int sp_kernel_matrix(const sp_dataset *ds, const double *P_dk, int k,
         return SP_ERR_INVALID;
     }
     if (ds->n_samples == 0) return SP_OK;
-    return dispatch_all<2, false>(degree, ds->n_samples, k, ds->csr_indptr, ds->csr_indices,
-                                  ds->csr_data, P_dk, nullptr, nullptr, nullptr, 1, 0, K,
-                                  (cudaStream_t)stream);
+    return dispatch_all<2>(degree, ds->n_samples, k, ds->csr_indptr, ds->csr_indices,
+                           ds->csr_data, P_dk, nullptr, nullptr, nullptr, 1, 0, K,
+                           (cudaStream_t)stream);
 }
 
-// pbcd cache precompute (all components): A[n, m-1, k] (ANOVA) or A[n, k] (all-subsets)
-int sp_rows_precompute_all(const sp_dataset *ds, const double *P_dk, int k, int degree, double *A,
-                           cudaStream_t st) {
-    if (ds->n_samples == 0) return SP_OK;
-    return dispatch_all<1, true>(degree, ds->n_samples, k, ds->csr_indptr, ds->csr_indices,
-                                 ds->csr_data, P_dk, nullptr, nullptr, nullptr, 1, 0, A, st);
-}
-
-// pbcd cache precompute of many models in one launch: entry y is {P_dk, A} of one model; the group width is
-// the one launch_all picks for k
-namespace {
-template <int DEG>
-void launch_all_multi(int n, int k, const sp_dataset *ds, const SpBlockEntry *table, int n_tab, cudaStream_t st) {
-    if (k <= 8) {
-        rows_all_multi_kernel<DEG, 8><<<dim3(grid_for(n, ROWS_THREADS / 8), n_tab), ROWS_THREADS, 0, st>>>(
-            n, k, ds->csr_indptr, ds->csr_indices, ds->csr_data, table);
-    } else if (k <= 16) {
-        rows_all_multi_kernel<DEG, 16><<<dim3(grid_for(n, ROWS_THREADS / 16), n_tab), ROWS_THREADS, 0, st>>>(
-            n, k, ds->csr_indptr, ds->csr_indices, ds->csr_data, table);
-    } else {
-        rows_all_multi_kernel<DEG, 32><<<dim3(grid_for(n, ROWS_THREADS / 32), n_tab), ROWS_THREADS, 0, st>>>(
-            n, k, ds->csr_indptr, ds->csr_indices, ds->csr_data, table);
-    }
-}
-}  // namespace
-
+// pbcd cache precompute of n_tab models in one launch: entry y is {P_dk, A} of one model, A [n, m-1, k] (ANOVA)
+// or [n, k] (all-subsets)
 int sp_rows_precompute_all_multi(const sp_dataset *ds, const SpBlockEntry *table, int n_tab, int k, int degree,
                                  cudaStream_t st) {
     const int n = ds->n_samples;
     if (n == 0 || n_tab == 0) return SP_OK;
     sp_prof_begin(SP_PROF_ROWS, st);
     switch (degree) {
-    case -1: launch_all_multi<-1>(n, k, ds, table, n_tab, st); break;
-    case 2: launch_all_multi<2>(n, k, ds, table, n_tab, st); break;
-    case 3: launch_all_multi<3>(n, k, ds, table, n_tab, st); break;
-    case 4: launch_all_multi<4>(n, k, ds, table, n_tab, st); break;
-    case 5: launch_all_multi<5>(n, k, ds, table, n_tab, st); break;
+    case -1: launch_pbcd_cache<-1>(n, k, ds, table, n_tab, st); break;
+    case 2: launch_pbcd_cache<2>(n, k, ds, table, n_tab, st); break;
+    case 3: launch_pbcd_cache<3>(n, k, ds, table, n_tab, st); break;
+    case 4: launch_pbcd_cache<4>(n, k, ds, table, n_tab, st); break;
+    case 5: launch_pbcd_cache<5>(n, k, ds, table, n_tab, st); break;
     default:
         sp_set_error("pbcd degree %d is not supported (2..%d or -1)", degree, SP_MAXDEG);
         return SP_ERR_UNSUPPORTED;
     }
     sp_prof_end(st);
-    SP_LAUNCH_CHECK("rows_all_multi_kernel");
+    SP_LAUNCH_CHECK("rows_pbcd_cache_kernel");
     return SP_OK;
 }
 
-// pcd cache precompute (one component) into the record array
-int sp_rows_precompute_one(const sp_dataset *ds, const double *p_s, int degree, double *rec,
-                           int rec_stride, cudaStream_t st) {
+// pcd cache precompute of n_tab (model, component) entries in one launch, into each entry's record array
+int sp_rows_precompute_multi(const sp_dataset *ds, const SpRowsEntry *table, int n_tab, int degree, int rec_stride,
+                             cudaStream_t st) {
     const int n = ds->n_samples;
-    if (n == 0) return SP_OK;
-    const int grid = grid_for(n, ROWS_THREADS / 8);
-#define SP_ONE(D)                                                                                \
-    rows_one_kernel<D><<<grid, ROWS_THREADS, 0, st>>>(n, ds->csr_indptr, ds->csr_indices,        \
-                                                      ds->csr_data, p_s, rec, rec_stride)
+    if (n == 0 || n_tab == 0) return SP_OK;
+    const dim3 grid((unsigned)grid_for(n, ROWS_THREADS / 8), (unsigned)n_tab);
+#define SP_ONE(D)                                                                                    \
+    rows_one_kernel<D><<<grid, ROWS_THREADS, 0, st>>>(n, ds->csr_indptr, ds->csr_indices,            \
+                                                      ds->csr_data, table, rec_stride)
     sp_prof_begin(SP_PROF_ROWS, st);
     switch (degree) {
     case -1: SP_ONE(-1); break;
@@ -259,31 +235,5 @@ int sp_rows_precompute_one(const sp_dataset *ds, const double *p_s, int degree, 
 #undef SP_ONE
     sp_prof_end(st);
     SP_LAUNCH_CHECK("rows_one_kernel");
-    return SP_OK;
-}
-
-// pcd cache precompute of many (model, component) entries in one launch
-int sp_rows_precompute_multi(const sp_dataset *ds, const SpRowsEntry *table, int n_tab, int degree, int rec_stride,
-                             cudaStream_t st) {
-    const int n = ds->n_samples;
-    if (n == 0 || n_tab == 0) return SP_OK;
-    const dim3 grid((unsigned)grid_for(n, ROWS_THREADS / 8), (unsigned)n_tab);
-#define SP_MULTI(D)                                                                                  \
-    rows_one_multi_kernel<D><<<grid, ROWS_THREADS, 0, st>>>(n, ds->csr_indptr, ds->csr_indices,      \
-                                                            ds->csr_data, table, rec_stride)
-    sp_prof_begin(SP_PROF_ROWS, st);
-    switch (degree) {
-    case -1: SP_MULTI(-1); break;
-    case 2: SP_MULTI(2); break;
-    case 3: SP_MULTI(3); break;
-    case 4: SP_MULTI(4); break;
-    case 5: SP_MULTI(5); break;
-    default:
-        sp_set_error("pcd degree %d is not supported (2..%d or -1)", degree, SP_MAXDEG);
-        return SP_ERR_UNSUPPORTED;
-    }
-#undef SP_MULTI
-    sp_prof_end(st);
-    SP_LAUNCH_CHECK("rows_one_multi_kernel");
     return SP_OK;
 }
