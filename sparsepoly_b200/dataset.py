@@ -236,6 +236,8 @@ def choose_geometry(ds, solver, n_cta=None, threads=None):
 
 
 WINDOW_SIZES = (256, 192, 128, 96, 64, 48, 32, 24, 16, 12, 8, 4, 2, 1)
+WINDOW_MAX = 256              # SP_WINDOW_MAX: per-position arrays of the pcd / cd_linear engine CTA
+PBCD_WINDOW_MAX = 64          # per-position arrays and cold-sum ring of the pbcd engine CTA (pbcd_window.cu)
 
 
 class WindowPlan:
@@ -255,6 +257,10 @@ class WindowPlan:
         env_b = os.environ.get("SPARSEPOLY_B200_WINDOW")
         env_h = os.environ.get("SPARSEPOLY_B200_HORIZON")
         self.window = int(env_b) if (window is None and env_b) else window
+        wmax = WINDOW_MAX if pbcd_shape is None else PBCD_WINDOW_MAX
+        if self.window is not None and not 1 <= self.window <= wmax:
+            raise ValueError(f"window plan: window={self.window} is outside 1..{wmax} for the "
+                             f"{'pcd' if pbcd_shape is None else 'pbcd'} window sweep")
         self.horizon = int(env_h) if (horizon is None and env_h) else (0 if horizon is None else horizon)
         env_n = os.environ.get("SPARSEPOLY_B200_NEAR")
         self.near = int(env_n) if env_n else 1
@@ -320,6 +326,11 @@ class WindowPlan:
                                      _ptr(self.h_x), _ptr(self.ht_cls), _ptr(self.n_slots),
                                      _ptr(self.slot_row), _ptr(self.overflow), _stream()))
         if int(self.overflow.item()):
+            # (what the failed window needed, for the error of a forced window)
+            starts = torch.arange(0, d, B, device=dev)
+            ends = torch.clamp(starts + B, max=d)
+            self._overflow_need = (int(self.n_slots.max().item()),
+                                   int((self.ht_ptr[ends] - self.ht_ptr[starts]).max().item()))
             return False
         s = _lib.SpWPlan()
         s.window, s.horizon, s.n_windows, s.slot_cap = B, self.horizon, n_windows, self.slot_cap
@@ -351,8 +362,11 @@ class WindowPlan:
                     return True
         self.near = near0
         if self.window is not None:
+            slots, hot = self._overflow_need
+            ent_cap = (2 if self.pbcd_shape is None else 3) * self.slot_cap
             raise ValueError(f"window plan: window={self.window} horizon={self.horizon} does not fit "
-                             f"{self.slot_cap} shared-memory slots")
+                             f"{self.slot_cap} shared-memory slots: a window needs {slots} slots and "
+                             f"{hot} hot nonzeros (at most {self.slot_cap} and {ent_cap})")
         return False
 
 

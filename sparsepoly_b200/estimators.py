@@ -358,7 +358,7 @@ class _BaseSparseFactorizationMachine(_SparsePolyBase, metaclass=ABCMeta):
         reg_norms = torch.zeros(max(d, 1), dtype=_f64, device=dev)
         regstate = torch.zeros(16, dtype=_f64, device=dev)
         viol_dev = torch.zeros(1, dtype=_f64, device=dev)
-        self._dev_state = dict(ds=ds, plan=plan, rec=yrec, stride=2, P=P, w=w)
+        self._dev_state = dict(ds=ds, plan=plan, plan_lin=plan_lin, rec=yrec, stride=2, P=P, w=w)
 
         def sync():
             for o in range(P.shape[0]):
