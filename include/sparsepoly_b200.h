@@ -382,6 +382,11 @@ int sp_psgd_plan_run(sp_psgd_ctx *ctx, const sp_dataset *ds, const sp_psgd_plan 
 /* end of an epoch: *loss_sum (device, may be NULL) += sum of the per-sample losses of positions
  * [0, n_local) in fixed order; materialize != 0 rewrites P / w as the model (thr = 0, C = Cw = 1). */
 int sp_psgd_plan_end(sp_psgd_ctx *ctx, int n_local, double *loss_sum, int materialize, sp_stream stream);
+/* the model the lazy frame represents, written to device buffers without changing ctx (training continues in the
+ * same frame): P_out[o, s, j] = soft_threshold(P[o, j, s], thr[o*k+s]) / C in the component-major [n_orders, k, d]
+ * layout of the estimators' P_, w_out = w / Cw (w when !fit_linear).  Bit-identical to the materialising
+ * sp_psgd_plan_end followed by a transpose.  Single rank only (SP_ERR_UNSUPPORTED when world > 1). */
+int sp_psgd_plan_read(const sp_psgd_ctx *ctx, double *P_out, double *w_out, sp_stream stream);
 /* destroys the library-owned stream / events of ctx (idempotent) */
 int sp_psgd_plan_release(sp_psgd_ctx *ctx);
 

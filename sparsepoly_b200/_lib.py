@@ -138,6 +138,7 @@ SIGNATURES = {
     "sp_psgd_plan_begin": (_i, [_PCP, _vp]),
     "sp_psgd_plan_run": (_i, [_PCP, _DSP, _PPP, _vp, _vp, _d, _d, _d, _d, _i, _d, _i, _i, C.POINTER(C.c_int64), _vp]),
     "sp_psgd_plan_end": (_i, [_PCP, _i, _vp, _i, _vp]),
+    "sp_psgd_plan_read": (_i, [_PCP, _vp, _vp, _vp]),
     "sp_psgd_plan_release": (_i, [_PCP]),
     "sp_psgd_plan_solver_stats": (_i, [_PCP, C.POINTER(_d), _vp]),
     "sp_shm_alloc": (_i, [C.c_size_t, C.POINTER(_vp)]),

@@ -1262,6 +1262,34 @@ __global__ void psgd_materialize_kernel(double *P, int n_orders, size_t d, int k
     if (fit_linear)
         for (size_t e = (size_t)blockIdx.x * blockDim.x + threadIdx.x; e < d; e += stride) w[e] = w[e] * invCw;
 }
+// the model the frame represents, written out in the component-major [n_orders, k, d] layout of P_: a 32 x 32 tile
+// of (feature, component) per block, read along k and written along d; the value expressions are those of
+// psgd_materialize_kernel, so the result equals materialise + transpose bit for bit
+constexpr int READ_TILE = 32, READ_ROWS = 8;
+__global__ void psgd_read_kernel(const double *P, int d, int k, const double *thr, double invC, double *P_out) {
+    __shared__ double tile[READ_TILE][READ_TILE + 1];
+    const int o = blockIdx.z, s = blockIdx.y * READ_TILE + threadIdx.x;
+    const long long j0 = (long long)blockIdx.x * READ_TILE;
+    const double *Po = P + (size_t)o * d * k;
+    if (s < k) {
+        const double T = thr[o * k + s];
+        for (int r = threadIdx.y; r < READ_TILE; r += READ_ROWS) {
+            const long long j = j0 + r;
+            if (j < d) tile[r][threadIdx.x] = st_true(Po[(size_t)j * k + s], T, invC);
+        }
+    }
+    __syncthreads();
+    const long long j = j0 + threadIdx.x;
+    if (j < d)
+        for (int r = threadIdx.y; r < READ_TILE; r += READ_ROWS) {
+            const int s2 = blockIdx.y * READ_TILE + r;
+            if (s2 < k) P_out[((size_t)o * k + s2) * d + j] = tile[threadIdx.x][r];
+        }
+}
+__global__ void psgd_read_w_kernel(const double *w, int d, double invCw, int fit_linear, double *w_out) {
+    for (int j = blockIdx.x * blockDim.x + threadIdx.x; j < d; j += gridDim.x * blockDim.x)
+        w_out[j] = fit_linear ? w[j] * invCw : w[j];
+}
 __global__ void psgd_zero_kernel(double *p, int n) {
     for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) p[i] = 0.0;
 }
@@ -1760,6 +1788,26 @@ extern "C" int sp_psgd_plan_end(sp_psgd_ctx *cx, int n_local, double *loss_sum, 
         SP_LAUNCH_CHECK("psgd_zero_kernel");
         cx->C = 1.0; cx->Cw = 1.0;
         if (cx->world > 1) { cx->seq += 1; rc = xbarrier(cx, 0, cx->seq, st); if (rc) return rc; }
+    }
+    return SP_OK;
+}
+
+// the model the lazy frame represents, for a caller that goes on training: the context is only read
+extern "C" int sp_psgd_plan_read(const sp_psgd_ctx *cx, double *P_out, double *w_out, sp_stream stream) {
+    int rc = ctx_check(cx);
+    if (rc) return rc;
+    if (cx->world > 1) { sp_set_error("sp_psgd_plan_read: single rank only (got world %d)", cx->world); return SP_ERR_UNSUPPORTED; }
+    if (!P_out || !w_out) { sp_set_error("sp_psgd_plan_read: null pointer"); return SP_ERR_INVALID; }
+    cudaStream_t st = (cudaStream_t)stream;
+    const int d = cx->d_rows, k = cx->k;
+    if (d > 0) {
+        const dim3 grid((unsigned)((d + READ_TILE - 1) / READ_TILE), (unsigned)((k + READ_TILE - 1) / READ_TILE), (unsigned)cx->n_orders);
+        psgd_read_kernel<<<grid, dim3(READ_TILE, READ_ROWS), 0, st>>>(cx->P, d, k, cx->thr, 1.0 / cx->C, P_out);
+        SP_LAUNCH_CHECK("psgd_read_kernel");
+        int b = (d + 255) / 256;
+        if (b > 148 * 16) b = 148 * 16;
+        psgd_read_w_kernel<<<b, 256, 0, st>>>(cx->w, d, 1.0 / cx->Cw, cx->fit_linear, w_out);
+        SP_LAUNCH_CHECK("psgd_read_w_kernel");
     }
     return SP_OK;
 }

@@ -24,7 +24,7 @@ from sklearn.exceptions import NotFittedError
 from sklearn.preprocessing import LabelBinarizer, add_dummy_feature
 from sklearn.utils import check_random_state
 from sklearn.utils.multiclass import type_of_target
-from sklearn.utils.validation import check_array, check_consistent_length, check_X_y
+from sklearn.utils.validation import check_array, check_consistent_length, check_X_y, column_or_1d
 
 from . import _lib, solvers
 from .dataset import DeviceDataset, SweepPlan, _device
@@ -95,7 +95,7 @@ class _SparsePolyBase(BaseEstimator, metaclass=ABCMeta):
         # device handles (ctypes structs with pointers, CUDA tensors) are per-fit scratch, not model state:
         # a fitted estimator pickles / deep-copies like the reference's (P_, w_, lams_, ... are numpy)
         state = dict(self.__dict__)
-        for key in ("_dev_state", "_y_pred_train"):
+        for key in ("_dev_state", "_y_pred_train", "_psgd_stream"):
             state.pop(key, None)
         return state
 
@@ -118,6 +118,11 @@ class SparsePolyRegressorMixin(RegressorMixin):
         X, y = check_X_y(X, y, accept_sparse=True, multi_output=False, dtype=np.double,
                          y_numeric=True)
         return X, y.astype(np.double).ravel()
+
+    def _partial_fit_X_y(self, X, y, classes):
+        """X, y of one partial_fit call (classes is the classifier's; ignored here) and no label binarizer."""
+        X, y = self._check_X_y(X, y)
+        return X, y, None
 
     def predict(self, X):
         """Predict regression output for the samples in X ([n_samples] array)."""
@@ -177,6 +182,32 @@ class SparsePolyClassifierMixin(ClassifierMixin):
         self.label_binarizer_ = LabelBinarizer(pos_label=1, neg_label=-1)
         y = self.label_binarizer_.fit_transform(Y).ravel().astype(np.double)
         return X, y
+
+    def _partial_fit_X_y(self, X, y, classes):
+        """X, y in {-1, +1} of one partial_fit call, and the label binarizer of `classes` when the estimator has
+        none yet (the first call of a stream: classes is required there and ignored later, as in scikit-learn).
+        A chunk may hold one class only; labels map to +-1 as LabelBinarizer(pos_label=1, neg_label=-1) maps
+        them in fit."""
+        lb = getattr(self, "label_binarizer_", None)
+        new = None
+        if lb is not None and classes is not None and not np.array_equal(np.unique(classes), lb.classes_):
+            raise ValueError(f"classes={list(classes)!r} differs from the classes the model was fitted with "
+                             f"({lb.classes_.tolist()}).")
+        if lb is None:
+            if classes is None:
+                raise ValueError("classes must be passed on the first call to partial_fit.")
+            classes = np.asarray(classes)
+            if classes.ndim != 1 or classes.size != 2 or np.unique(classes).size != 2:
+                raise ValueError(f"classes must hold exactly two distinct labels, got {classes!r}.")
+            lb = new = LabelBinarizer(pos_label=1, neg_label=-1).fit(classes)
+        X = check_array(X, dtype=np.double, accept_sparse=True)
+        y = column_or_1d(y)
+        check_consistent_length(X, y)
+        known = np.isin(y, lb.classes_)
+        if not np.all(known):
+            raise ValueError(f"y contains labels that are not in classes {lb.classes_.tolist()}: "
+                             f"{np.unique(y[~known])[:5].tolist()}")
+        return X, np.where(y == lb.classes_[1], 1.0, -1.0), new
 
 
 # =============================================================================================
@@ -420,22 +451,97 @@ class _BaseSparseFactorizationMachine(_SparsePolyBase, metaclass=ABCMeta):
         th.start()
         return th, box
 
-    def _psgd_setup(self, X, y, rng, dev, upload=None):
-        """Move everything to the device and return (epoch, sync, close): epoch() runs one psgd.psgd_epoch
-        (sparse_factorization_machines.py:123-150) and returns the epoch's mean loss (None with
-        read_back=False).  l1 / squaredl12 run the planned path (psgd_plan.cu: gather passes over a batch-CSC
-        plan, touched rows only, sharded over peer memory); l21 / squaredl21 the dense-gradient path (psgd.cu)."""
-        n, d = X.shape
-        k = self.n_components
-        group = _process_group()
+    def _psgd_settings(self):
+        """(learning-rate id, process group, world, rank) of a psgd fit."""
         if self.learning_rate not in LEARNING_RATE:
             raise ValueError(f"learning_rate {self.learning_rate} is not supported."
                              f" Choose from {LEARNING_RATE}.")
-        learning_rate = LEARNING_RATE[self.learning_rate]
+        group = _process_group()
         world, rank = 1, 0
         if group is not None:
             import torch.distributed as dist
             world, rank = dist.get_world_size(group), dist.get_rank(group)
+        return LEARNING_RATE[self.learning_rate], group, world, rank
+
+    def _psgd_model(self, dev, batch_size, learning_rate, group=None, world=1, rank=0):
+        """The model half of psgd, which outlives a pass over the rows: P_ / w_ / lams_ on the device, the loss
+        accumulator and the dense-gradient path's buffers.  The planned path's context joins it with the first
+        plan (_psgd_bind)."""
+        d, k = self.P_.shape[2], self.n_components
+        P_kd = torch.from_numpy(np.ascontiguousarray(self.P_)).to(dev)
+        P = torch.stack([solvers.transpose(P_kd[o]) for o in range(P_kd.shape[0])])   # [n_orders, d, k]
+        del P_kd
+        m = dict(planned=self.regularizer in solvers.PLANNED_REGS, learning_rate=learning_rate, group=group,
+                 world=world, rank=rank, batch_size=batch_size, b_loc=max(1, batch_size // world), P=P,
+                 w=torch.from_numpy(np.ascontiguousarray(self.w_)).to(dev),
+                 lams=torch.from_numpy(np.ascontiguousarray(self.lams_, dtype=np.float64)).to(dev),
+                 loss=torch.zeros(1, dtype=_f64, device=dev), model_current=True, ctx=None)
+        if not m["planned"]:
+            m.update(grad_P=torch.zeros_like(P), grad_w=torch.zeros(d, dtype=_f64, device=dev),
+                     work=solvers.prox_work(d, k, dev))
+        return m
+
+    @staticmethod
+    def _psgd_data(ds, y, order, dev):
+        """The data half of a psgd pass: the rows, their targets and the order they are visited in (the planned
+        path adds the batch-CSC plan of that order, _psgd_plan)."""
+        return dict(ds=ds, n=ds.n_samples, order=order, y=torch.from_numpy(y).to(dev),
+                    idx=torch.from_numpy(order).to(dev), plan=None)
+
+    @staticmethod
+    def _psgd_plan(m, data):
+        from .psgd_plan import PsgdPlan
+        return PsgdPlan(data["ds"].csr, data["idx"], data["ds"].n_features, m["b_loc"], world=m["world"],
+                        rank=m["rank"], group=m["group"])
+
+    def _psgd_bind(self, m, plan, inbox_cap=None):
+        """Planned path: the context runs on `plan`.  The first plan creates it (model loaded, frame and selection
+        state reset); later plans (reshuffles, further partial_fit chunks) only grow its plan-sized scratch."""
+        if m["ctx"] is not None:
+            m["ctx"].rebind(plan)
+            return
+        from .psgd_plan import PsgdContext
+        ctx = PsgdContext(plan, m["P"].shape[0], self.n_components, self.degree, self.regularizer, self.loss,
+                          self.fit_linear, m["lams"], group=m["group"], inbox_cap=inbox_cap)
+        ctx.load_model(m["P"], m["w"])
+        solvers.psgd_planned_begin(ctx)
+        m["ctx"] = ctx
+
+    def _psgd_pass(self, m, data, n_glob, read_back=True):
+        """One psgd.psgd_epoch (sparse_factorization_machines.py:123-150) over the rows of `data` in its order:
+        advances it_ and returns the mean loss (None with read_back=False).  l1 / squaredl12 run the planned path
+        (psgd_plan.cu: gather passes over a batch-CSC plan, touched rows only, sharded over peer memory); l21 /
+        squaredl21 the dense-gradient path (psgd.cu)."""
+        ctx, loss = m["ctx"], m["loss"]
+        loss.zero_()
+        if m["planned"]:
+            self.it_ = solvers.psgd_planned_run(ctx, data["ds"], data["plan"], data["y"], data["idx"], self.alpha,
+                                                self.beta, self.gamma, self.eta0, m["learning_rate"], self.power_t,
+                                                self.it_)
+            # the lazy scales only grow: fold them back into the storage long before they overflow
+            big = not (1e-100 < ctx.struct.C < 1e100 and 1e-100 < ctx.struct.Cw < 1e100)
+            solvers.psgd_planned_end(ctx, data["n"], loss, big)
+            m["model_current"] = big
+        else:
+            self.it_ = solvers.psgd_epoch(data["ds"], data["y"], m["P"], m["w"], m["lams"], self.degree, self.alpha,
+                                          self.beta, self.gamma, self.regularizer, self.loss, m["grad_P"],
+                                          m["grad_w"], data["idx"], self.fit_linear, self.eta0, m["learning_rate"],
+                                          self.power_t, m["batch_size"], self.it_, loss, m["work"], m["group"])
+        if not read_back:
+            return None
+        sum_loss = loss.item()
+        if m["planned"]:
+            ctx.check_peers()
+        if m["group"] is not None:
+            sum_loss = global_sum([sum_loss], m["group"])[0]
+        return sum_loss / n_glob
+
+    def _psgd_setup(self, X, y, rng, dev, upload=None):
+        """Move everything to the device and return (epoch, sync, close): epoch() is one _psgd_pass over all of X,
+        reshuffled first with shuffle=True."""
+        n, d = X.shape
+        learning_rate, group, world, rank = self._psgd_settings()
+        if group is not None:
             # replicas must start identical whatever each rank's random_state drew, and shards must be equal
             it_arr = np.array([float(self.it_)])
             broadcast_arrays([self.P_, self.w_, self.lams_, it_arr], group)
@@ -468,82 +574,47 @@ class _BaseSparseFactorizationMachine(_SparsePolyBase, metaclass=ABCMeta):
         else:
             batch_size = self.batch_size
         batch_size = max(int(batch_size), 1)
-        indices_samples = np.arange(n, dtype=np.int32)
-        idx_dev = torch.from_numpy(indices_samples).to(dev)
-        y_dev = torch.from_numpy(y).to(dev)
-        P_kd = torch.from_numpy(np.ascontiguousarray(self.P_)).to(dev)
-        P = torch.stack([solvers.transpose(P_kd[o]) for o in range(P_kd.shape[0])])   # [n_orders, d, k]
-        del P_kd
-        w = torch.from_numpy(np.ascontiguousarray(self.w_)).to(dev)
-        lams = torch.from_numpy(np.ascontiguousarray(self.lams_, dtype=np.float64)).to(dev)
-        loss_dev = torch.zeros(1, dtype=_f64, device=dev)
-        st = {"model_current": True}
+        data = self._psgd_data(ds, y, np.arange(n, dtype=np.int32), dev)
+        m = self._psgd_model(dev, batch_size, learning_rate, group, world, rank)
         if planned:
-            from .psgd_plan import PsgdContext, PsgdPlan
-            b_loc = max(1, batch_size // world)
             t2 = _tick()
-            st["plan"] = PsgdPlan(ds.csr, idx_dev, d, b_loc, world=world, rank=rank, group=group)
+            data["plan"] = plan = self._psgd_plan(m, data)
             t3 = _tick()
-            ctx = PsgdContext(st["plan"], P.shape[0], k, self.degree, self.regularizer, self.loss, self.fit_linear, lams,
-                              group=group,
-                              inbox_cap=(min(st["plan"].d_rows, b_loc * int(ds.max_row_nnz())) if self.shuffle else None))
-            ctx.load_model(P, w)
-            solvers.psgd_planned_begin(ctx)
-            self._psgd_stats = {"plan_bytes": st["plan"].nbytes(), "minibatches": st["plan"].n_minibatches,
-                                "columns_per_minibatch": st["plan"].n_cols / max(st["plan"].n_minibatches, 1),
-                                "batch_size": batch_size, "batch_local": b_loc, "world": world,
+            self._psgd_bind(m, plan, inbox_cap=(min(plan.d_rows, m["b_loc"] * int(ds.max_row_nnz()))
+                                                if self.shuffle else None))     # (shuffle=True: bound for any order)
+            self._psgd_stats = {"plan_bytes": plan.nbytes(), "minibatches": plan.n_minibatches,
+                                "columns_per_minibatch": plan.n_cols / max(plan.n_minibatches, 1),
+                                "batch_size": batch_size, "batch_local": m["b_loc"], "world": world,
                                 "setup_seconds": {"upload_X": t1 - t0, "upload_model": t2 - t1, "plan": t3 - t2,
                                                   "context": _tick() - t3, "synchronised": timing}}
         else:
-            grad_P = torch.zeros_like(P)
-            grad_w = torch.zeros(d, dtype=_f64, device=dev)
-            work = solvers.prox_work(d, k, dev)
             self._psgd_stats = {"batch_size": batch_size, "world": world}
 
         def sync():
+            P, w = m["P"], m["w"]
             if planned:
-                if not st["model_current"]:
-                    solvers.psgd_planned_end(ctx, 0, None, True)
-                    st["model_current"] = True
-                ctx.store_model(P, w)
+                if not m["model_current"]:
+                    solvers.psgd_planned_end(m["ctx"], 0, None, True)
+                    m["model_current"] = True
+                m["ctx"].store_model(P, w)
             for o in range(P.shape[0]):
                 self.P_[o] = solvers.transpose(P[o]).cpu().numpy()
             self.w_[...] = w.cpu().numpy()
 
         def epoch(read_back=True):
             if self.shuffle:
-                rng.shuffle(indices_samples)
-                idx_dev.copy_(torch.from_numpy(indices_samples))
+                rng.shuffle(data["order"])
+                data["idx"].copy_(torch.from_numpy(data["order"]))
                 if planned:
-                    st["plan"] = PsgdPlan(ds.csr, idx_dev, d, b_loc, world=world, rank=rank, group=group)
-                    ctx.rebind(st["plan"])
-            loss_dev.zero_()
-            if planned:
-                self.it_ = solvers.psgd_planned_run(ctx, ds, st["plan"], y_dev, idx_dev, self.alpha, self.beta, self.gamma,
-                                                    self.eta0, learning_rate, self.power_t, self.it_)
-                # the lazy scales only grow: fold them back into the storage long before they overflow
-                big = not (1e-100 < ctx.struct.C < 1e100 and 1e-100 < ctx.struct.Cw < 1e100)
-                solvers.psgd_planned_end(ctx, n, loss_dev, big)
-                st["model_current"] = big
-            else:
-                self.it_ = solvers.psgd_epoch(ds, y_dev, P, w, lams, self.degree, self.alpha, self.beta,
-                                              self.gamma, self.regularizer, self.loss, grad_P, grad_w,
-                                              idx_dev, self.fit_linear, self.eta0, learning_rate,
-                                              self.power_t, batch_size, self.it_, loss_dev, work, group)
-            if not read_back:
-                return None
-            sum_loss = loss_dev.item()
-            if planned:
-                ctx.check_peers()
-            if group is not None:
-                sum_loss = global_sum([sum_loss], group)[0]
-            return sum_loss / n_glob
+                    data["plan"] = self._psgd_plan(m, data)
+                    self._psgd_bind(m, data["plan"])
+            return self._psgd_pass(m, data, n_glob, read_back)
 
         def close():
             if planned:
                 if self.regularizer == "squaredl12":
-                    self._psgd_stats["selection"] = solvers.psgd_planned_solver_stats(ctx)
-                ctx.close()
+                    self._psgd_stats["selection"] = solvers.psgd_planned_solver_stats(m["ctx"])
+                m["ctx"].close()
 
         return epoch, sync, close
 
@@ -589,6 +660,7 @@ class _BaseSparseFactorizationMachine(_SparsePolyBase, metaclass=ABCMeta):
         if self.solver not in ("pcd", "pbcd", "psgd"):
             raise ValueError(f"Solver {self.solver} is not supported.")
         self._check_combination(self.solver, self.regularizer, self.degree)
+        self._end_stream()
         dev = _device()
         _lib.check(_lib.load().sp_set_device(dev.index if dev.index is not None else 0))
         upload = self._start_upload(X, dev) if self.solver == "psgd" else None
@@ -607,6 +679,128 @@ class _BaseSparseFactorizationMachine(_SparsePolyBase, metaclass=ABCMeta):
         if not converged:
             warnings.warn("Objective did not converge. Increase max_iter.")
         return self
+
+    def partial_fit(self, X, y, classes=None):
+        """One pass of psgd over the rows of (X, y), continuing the model and the optimiser state of the earlier
+        calls: trains on data too large for the device, streamed from the host in chunks of rows.  Returns self.
+
+        The rows are cut into minibatches of batch_size from the call's first row (the last one may be short;
+        nothing is carried to the next call); it_ continues across calls and n_iter_ counts them.  Chunks of a
+        multiple of batch_size rows, passed in order E times with shuffle=False, give the model of
+        fit(max_iter=E) on their concatenation.  P_ / w_ are current after every call.  The first call starts from
+        the drawn initial model, or from the fitted one if there is one; the classifier's first call needs
+        `classes` (the two labels).  fit() afterwards starts over.  solver='psgd' on one GPU only."""
+        import time
+        t0 = time.perf_counter()
+        if self.solver != "psgd":
+            raise ValueError(f"partial_fit is implemented for solver='psgd' only (got solver={self.solver!r}).")
+        self._get_loss(self.loss)
+        self._get_regularizer(self.regularizer)
+        self._check_combination(self.solver, self.regularizer, self.degree)
+        learning_rate, group, _, _ = self._psgd_settings()
+        if group is not None:
+            raise ValueError("partial_fit runs psgd on one GPU; sharded psgd (distributed.enable_sharding) is not "
+                             "supported by it.")
+        X, y, label_binarizer = self._partial_fit_X_y(X, y, classes)
+        X = self._augment(X)
+        n, n_features = X.shape
+        if hasattr(self, "P_") and self.P_.shape[-1] != n_features:
+            raise ValueError(f"X has {n_features} features (after fit_lower), but the model has "
+                             f"{self.P_.shape[-1]}.")
+        n_orders = self.degree - 1 if self.fit_lower == "explicit" else 1
+        if hasattr(self, "P_") and self.P_.shape[:2] != (n_orders, self.n_components):
+            raise ValueError(f"degree / fit_lower / n_components ask for {n_orders} order(s) of {self.n_components} "
+                             f"components, but the model has P_ of shape {self.P_.shape}; fit() starts a new model.")
+        m = getattr(self, "_psgd_stream", None)
+        if m is not None and m["config"] != self._stream_config():
+            raise ValueError("degree / n_components / regularizer / loss / fit_lower / fit_linear changed since the "
+                             "stream started; fit() starts a new model.")
+        t1 = time.perf_counter()
+        dev = _device()
+        _lib.check(_lib.load().sp_set_device(dev.index if dev.index is not None else 0))
+        before = dict(self.__dict__) if m is None else None
+        try:
+            mean_loss = self._stream_call(X, y, label_binarizer, learning_rate, dev, m, t0, t1)
+        except BaseException:
+            if before is not None:                  # a failed first call leaves the estimator as it was
+                new = self.__dict__.get("_psgd_stream")
+                if new is not None and new["ctx"] is not None:
+                    new["ctx"].close()
+                self.__dict__.clear()
+                self.__dict__.update(before)
+            raise
+        if self.verbose:
+            print(f"Call {self.n_iter_} loss {mean_loss}")
+        return self
+
+    def _stream_config(self):
+        return (self.degree, self.n_components, self.regularizer, self.loss, self.fit_lower, self.fit_linear)
+
+    def _stream_call(self, X, y, label_binarizer, learning_rate, dev, m, t0, t1):
+        """The device part of partial_fit (m: the stream's model half, None on the first call of a process);
+        returns the call's mean loss and leaves the phase times in _partial_fit_stats."""
+        import time
+        n, n_features = X.shape
+        if label_binarizer is not None:
+            self.label_binarizer_ = label_binarizer
+        if m is None and not hasattr(self, "batch_size_"):     # a new stream (an unpickled one goes on as it was)
+            self._stream_rng = check_random_state(self.random_state)
+            self.n_iter_ = 0
+            if not hasattr(self, "P_"):
+                self._init_coefs(n_features, self._stream_rng)
+            self.it_ = getattr(self, "it_", 1)
+        t2 = time.perf_counter()
+        planned = self.regularizer in solvers.PLANNED_REGS
+        ev = [torch.cuda.Event(enable_timing=True) for _ in range(5)]
+        ev[0].record()
+        ds = DeviceDataset(X, need_csr=True, need_csc=False, device=dev, hot_features=not planned)
+        if not hasattr(self, "batch_size_"):
+            self.batch_size_ = max(int(n * n_features / ds.nnz) if self.batch_size == "auto"    # :101-102
+                                   else int(self.batch_size), 1)
+        order = np.arange(n, dtype=np.int32)
+        if self.shuffle:
+            self._stream_rng.shuffle(order)
+        data = self._psgd_data(ds, np.ascontiguousarray(y, dtype=np.float64), order, dev)
+        ev[1].record()
+        if m is None:
+            m = self._psgd_model(dev, self.batch_size_, learning_rate)
+            m["config"] = self._stream_config()
+        ev[2].record()
+        if planned:
+            data["plan"] = self._psgd_plan(m, data)
+            self._psgd_bind(m, data["plan"])
+        ev[3].record()
+        self._psgd_stream = m
+        mean_loss = self._psgd_pass(m, data, n)
+        ev[4].record()
+        t3 = time.perf_counter()
+        self._psgd_read(m)
+        self.n_iter_ += 1
+        sec = lambda i: ev[i].elapsed_time(ev[i + 1]) / 1e3          # noqa: E731
+        self._partial_fit_stats = {"rows": n, "validate_s": t1 - t0, "h2d_s": sec(0), "model_s": t2 - t1 + sec(1),
+                                   "plan_s": sec(2), "minibatches_s": sec(3), "readout_s": time.perf_counter() - t3}
+        return mean_loss
+
+    def _psgd_read(self, m):
+        """P_ / w_ of the stream's model, the device state left as it is: the planned path reads the lazy frame
+        (sp_psgd_plan_read) instead of materialising it, which would change the rounding of the calls to come."""
+        P = m["P"]
+        n_orders, d, k = P.shape
+        if m["planned"]:
+            P_out = torch.empty((n_orders, k, d), dtype=_f64, device=P.device)
+            w_out = torch.empty(d, dtype=_f64, device=P.device)
+            solvers.psgd_planned_read(m["ctx"], P_out, w_out)
+        else:
+            P_out, w_out = torch.stack([solvers.transpose(P[o]) for o in range(n_orders)]), m["w"]
+        self.P_, self.w_ = P_out.cpu().numpy(), w_out.cpu().numpy()
+
+    def _end_stream(self):
+        """fit starts over: the device state of a partial_fit stream is released and its attributes dropped."""
+        m = self.__dict__.pop("_psgd_stream", None)
+        if m is not None and m["ctx"] is not None:
+            m["ctx"].close()
+        for key in ("_stream_rng", "batch_size_", "_partial_fit_stats"):
+            self.__dict__.pop(key, None)
 
     def _get_output(self, X):
         dev = _device()

@@ -478,7 +478,11 @@ class PsgdContext:
             raise RuntimeError("sharded psgd: a cross-rank wait timed out (a peer rank failed or stalled)")
 
     def rebind(self, plan):
-        """The scratch sized by the plan must cover a rebuilt plan (shuffle=True rebuilds every epoch)."""
+        """The scratch sized by the plan must cover a rebuilt plan (shuffle=True rebuilds every epoch) and the plan of
+        another chunk of rows (partial_fit: any number of rows)."""
+        if plan.n_local > self.sample_loss.numel():
+            self.sample_loss = torch.zeros(plan.n_local, dtype=torch.float64, device=plan.device)
+            self.struct.sample_loss = self.sample_loss.data_ptr()
         if (plan.max_chunks, plan.max_cols, plan.batch_local) != self.plan_dims:
             dev, f64 = plan.device, torch.float64
             ncolk = self.n_orders * self.k

@@ -195,6 +195,11 @@ def psgd_planned_end(ctx, n_local, loss_sum, materialize):
     _lib.check(_L().sp_psgd_plan_end(ctx.ref(), int(n_local), _ptr(loss_sum), int(bool(materialize)), _stream()))
 
 
+def psgd_planned_read(ctx, P_okd, w):
+    """The model the lazy frame represents into P_okd [n_orders, k, d] / w [d] (device); ctx is left as it was."""
+    _lib.check(_L().sp_psgd_plan_read(ctx.ref(), _ptr(P_okd), _ptr(w), _stream()))
+
+
 # ------------------------------------------------------------------------------ objective
 def _sum_work(device):
     return torch.empty(int(_L().sp_sum_work_doubles()), dtype=_f64, device=device)
