@@ -159,6 +159,8 @@ int sp_wtrace_read(long long *out_host);
 int sp_wplan_slot_cap(int rec_stride);
 /* out[c*rows+r] = in[r*cols+c] */
 int sp_transpose_f64(const double *in, double *out, int rows, int cols, sp_stream stream);
+/* the same for `batch` (<= 65535) consecutive matrices in one launch: matrix b is in[b*rows*cols ...] -> out[b*rows*cols ...] */
+int sp_transpose_f64_batch(const double *in, double *out, int batch, int rows, int cols, sp_stream stream);
 /* doubles per sample record {y_pred, y, A^1..A^(m-1)} for a model of this top degree */
 int sp_rec_stride(int degree);
 
@@ -168,6 +170,21 @@ int sp_rec_stride(int degree);
  * P_dk is feature-major [d,k]; w may be NULL; accumulate != 0 adds to out. */
 int sp_predict(const sp_dataset *ds, const double *P_dk, int k, const double *lams, int degree,
                const double *w, double *out, int out_stride, int accumulate, sp_stream stream);
+
+/* Prediction of many models on one design matrix (decision_function_many; DESIGN.md 3.1).  One descriptor per model,
+ * passed as a host array of at most SP_PREDICT_MAX_MODELS entries; the call is one launch over all models (the table
+ * travels as a kernel parameter), and each model's rows are computed by the code sp_predict runs, so every model's
+ * output is bit-identical to sp_predict with the same arguments.  sp_predict is the one-model case of this call.
+ * k, degree, out_stride and accumulate hold for every model.  Models may share P_dk, lams and w, never out. */
+#define SP_PREDICT_MAX_MODELS 256
+typedef struct sp_predict_model {
+    const double *P_dk;       /* [d,k] feature-major */
+    const double *lams;       /* [k] */
+    const double *w;          /* [d] or NULL (no linear term) */
+    double *out;              /* out[i*out_stride] (+)= the model's output for sample i */
+} sp_predict_model;
+int sp_predict_multi(const sp_dataset *ds, const sp_predict_model *models, int n_models, int k, int degree,
+                     int out_stride, int accumulate, sp_stream stream);
 
 /* K[i*k+s] = K(P[:,s], x_i): the Gram matrix of kernels.anova_kernel (kernels.py:71-115) /
  * kernels.all_subsets_kernel (kernels.py:118-137, degree=-1). */
@@ -431,6 +448,36 @@ size_t sp_sum_work_doubles(void);
 int sp_reg_eval(const double *P_dk, int d, int k, int reg, int degree, double *work, double *out,
                 sp_stream stream);
 size_t sp_reg_eval_work_doubles(int d, int k);
+
+/* Many reductions of one length in one call (objective_many; DESIGN.md 3.5): host arrays of at most
+ * SP_OBJECTIVE_MAX_ENTRIES entries, each launch covers all entries (the table travels as a kernel parameter), and
+ * entry b's result is bit-identical to the single call on its arguments (the same blocks, partials and fixed tree),
+ * which is the one-entry case of these.  Work buffers are per entry: n_entries x sp_sum_work_doubles() doubles for the
+ * sums, n_entries x sp_reg_eval_work_doubles(d, k) for Omega; entry b uses the b-th slice.
+ *   sp_loss_sum_multi: entry b: out[0] = sum_i loss_b(y_pred[i*pred_stride], y[i*y_stride]), i < n;
+ *   sp_sqnorm_multi  : entry b: out[0] = sum_i v[i]^2, i < len;
+ *   sp_reg_eval_multi: entry b: out[0] = Omega_reg(P_dk) of a [d,k] matrix at this degree; at most two partial
+ *                      launches (column-fold and row-norm regularizers), one combine and one final launch. */
+#define SP_OBJECTIVE_MAX_ENTRIES 256
+typedef struct sp_loss_entry {
+    const double *y_pred, *y;
+    int32_t loss;             /* loss id */
+    double *out;
+} sp_loss_entry;
+typedef struct sp_sqnorm_entry {
+    const double *v;
+    double *out;
+} sp_sqnorm_entry;
+typedef struct sp_reg_entry {
+    const double *P_dk;       /* [d,k] feature-major */
+    int32_t reg;              /* reg id */
+    double *out;
+} sp_reg_entry;
+int sp_loss_sum_multi(const sp_loss_entry *entries, int n_entries, int pred_stride, int y_stride, int n,
+                      double *work, sp_stream stream);
+int sp_sqnorm_multi(const sp_sqnorm_entry *entries, int n_entries, int64_t len, double *work, sp_stream stream);
+int sp_reg_eval_multi(const sp_reg_entry *entries, int n_entries, int d, int k, int degree, double *work,
+                      sp_stream stream);
 
 #ifdef __cplusplus
 }

@@ -6,11 +6,15 @@ from .estimators import (
     SparseFactorizationMachineClassifier,
     SparseFactorizationMachineRegressor,
 )
-from .multi import fit_many
+from .multi import decision_function_many, fit_many, objective_many, predict_many, score_many
 from .objective import objective
 
 __all__ = [
+    "decision_function_many",
     "fit_many",
+    "objective_many",
+    "predict_many",
+    "score_many",
     "objective",
     "SparseAllSubsetsClassifier",
     "SparseAllSubsetsRegressor",

@@ -90,6 +90,30 @@ class SpPbcdModel(C.Structure):
                 ("yrec", _vp), ("A", _vp), ("reg_norms", _vp), ("regstate", _vp), ("viol", _vp)]
 
 
+PREDICT_MAX_MODELS = 256           # SP_PREDICT_MAX_MODELS
+OBJECTIVE_MAX_ENTRIES = 256        # SP_OBJECTIVE_MAX_ENTRIES
+
+
+class SpPredictModel(C.Structure):
+    """struct sp_predict_model (include/sparsepoly_b200.h): one model of sp_predict_multi."""
+    _fields_ = [("P_dk", _vp), ("lams", _vp), ("w", _vp), ("out", _vp)]
+
+
+class SpLossEntry(C.Structure):
+    """struct sp_loss_entry (include/sparsepoly_b200.h): one sum of sp_loss_sum_multi."""
+    _fields_ = [("y_pred", _vp), ("y", _vp), ("loss", C.c_int32), ("out", _vp)]
+
+
+class SpSqnormEntry(C.Structure):
+    """struct sp_sqnorm_entry (include/sparsepoly_b200.h): one sum of sp_sqnorm_multi."""
+    _fields_ = [("v", _vp), ("out", _vp)]
+
+
+class SpRegEntry(C.Structure):
+    """struct sp_reg_entry (include/sparsepoly_b200.h): one Omega of sp_reg_eval_multi."""
+    _fields_ = [("P_dk", _vp), ("reg", C.c_int32), ("out", _vp)]
+
+
 _DSP = C.POINTER(SpDataset)
 _PPP = C.POINTER(SpPsgdPlan)
 _PCP = C.POINTER(SpPsgdCtx)
@@ -115,8 +139,10 @@ SIGNATURES = {
     "sp_wtrace_read": (_i, [C.POINTER(C.c_longlong)]),
     "sp_wspec_read": (_i, [C.POINTER(C.c_ulonglong)]),
     "sp_transpose_f64": (_i, [_vp, _vp, _i, _i, _vp]),
+    "sp_transpose_f64_batch": (_i, [_vp, _vp, _i, _i, _i, _vp]),
     "sp_rec_stride": (_i, [_i]),
     "sp_predict": (_i, [_DSP, _vp, _i, _vp, _i, _vp, _vp, _i, _i, _vp]),
+    "sp_predict_multi": (_i, [_DSP, C.POINTER(SpPredictModel), _i, _i, _i, _i, _i, _vp]),
     "sp_kernel_matrix": (_i, [_DSP, _vp, _i, _i, _vp, _vp]),
     "sp_cd_linear_epoch": (_i, [_DSP, _PLP, _vp, _vp, _d, _i, _vp, _i, _vp, _vp]),
     "sp_pcd_epoch": (_i, [_DSP, _PLP, _vp, _i, _vp, _i, _d, _d, _d, _i, _i, _vp, _i, _vp, _vp,
@@ -152,6 +178,9 @@ SIGNATURES = {
     "sp_sum_work_doubles": (C.c_size_t, []),
     "sp_reg_eval": (_i, [_vp, _i, _i, _i, _i, _vp, _vp, _vp]),
     "sp_reg_eval_work_doubles": (C.c_size_t, [_i, _i]),
+    "sp_loss_sum_multi": (_i, [C.POINTER(SpLossEntry), _i, _i, _i, _i, _vp, _vp]),
+    "sp_sqnorm_multi": (_i, [C.POINTER(SpSqnormEntry), _i, C.c_int64, _vp, _vp]),
+    "sp_reg_eval_multi": (_i, [C.POINTER(SpRegEntry), _i, _i, _i, _i, _vp, _vp]),
 }
 
 _LIB = None

@@ -89,6 +89,9 @@ __global__ void order_flag_kernel(int d, const int32_t *__restrict__ idx_feat,
 __global__ void transpose_kernel(const double *__restrict__ in, double *__restrict__ out, int rows,
                                  int cols) {
     __shared__ double tile[32][33];
+    const size_t mat = (size_t)rows * cols;             // matrix blockIdx.y of a batch
+    in += blockIdx.y * mat;
+    out += blockIdx.y * mat;
     // tiles are numbered along ONE grid dimension (grid.y is limited to 65 535: a [d,k] matrix with d > 2 M rows
     // -- sparse CTR feature spaces -- would not fit there)
     const int tiles_x = (cols + 31) / 32;
@@ -158,13 +161,20 @@ extern "C" int sp_plan_order(const sp_dataset *ds, int n_cta, const int32_t *col
     return SP_OK;
 }
 
-extern "C" int sp_transpose_f64(const double *in, double *out, int rows, int cols, sp_stream stream) {
-    if (!in || !out || rows < 0 || cols < 0) { sp_set_error("sp_transpose_f64: invalid argument"); return SP_ERR_INVALID; }
-    if (rows == 0 || cols == 0) return SP_OK;
+extern "C" int sp_transpose_f64_batch(const double *in, double *out, int batch, int rows, int cols, sp_stream stream) {
+    if (!in || !out || batch < 0 || batch > 65535 || rows < 0 || cols < 0) {
+        sp_set_error("sp_transpose_f64: invalid argument");
+        return SP_ERR_INVALID;
+    }
+    if (batch == 0 || rows == 0 || cols == 0) return SP_OK;
     const long long tiles = (long long)((cols + 31) / 32) * ((rows + 31) / 32);
     if (tiles > 2147483647LL) { sp_set_error("sp_transpose_f64: matrix too large (%d x %d)", rows, cols); return SP_ERR_INVALID; }
-    dim3 grid((unsigned)tiles), block(32, 8);
+    dim3 grid((unsigned)tiles, (unsigned)batch), block(32, 8);
     transpose_kernel<<<grid, block, 0, (cudaStream_t)stream>>>(in, out, rows, cols);
     SP_LAUNCH_CHECK("transpose_kernel");
     return SP_OK;
+}
+
+extern "C" int sp_transpose_f64(const double *in, double *out, int rows, int cols, sp_stream stream) {
+    return sp_transpose_f64_batch(in, out, 1, rows, cols, stream);
 }

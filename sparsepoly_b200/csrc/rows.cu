@@ -16,16 +16,38 @@ namespace {
 constexpr int ROWS_THREADS = 256;
 
 // ---------------------------------------------------------------------------------------------
-// all-components kernel: one group of G lanes per sample, lanes over components.
-//   MODE 0: out[i*out_stride] (+)= sum_j x w_j + sum_s lam_s * K_s(i)      (predict)
-//   MODE 2: Aout[i, s] = K_s(i) (the Gram matrix of kernels.anova_kernel / all_subsets_kernel)
-template <int DEG, int G, int MODE>
+// all-components kernels: one group of G lanes per sample, lanes over components.
+//   MODE 0 (rows_predict_kernel): out[i*out_stride] (+)= sum_j x w_j + sum_s lam_s * K_s(i)      (predict)
+//   MODE 2 (rows_all_kernel): Aout[i, s] = K_s(i) (the Gram matrix of kernels.anova_kernel / all_subsets_kernel)
+template <int DEG, int G>
 __global__ void __launch_bounds__(ROWS_THREADS)
 rows_all_kernel(int n, int k, const int32_t *__restrict__ indptr, const int32_t *__restrict__ indices,
-                const double *__restrict__ data, const double *__restrict__ P_dk,
-                const double *__restrict__ lams, const double *__restrict__ w, double *out,
-                int out_stride, int accumulate, double *Aout) {
+                const double *__restrict__ data, const double *__restrict__ P_dk, double *Aout) {
+    constexpr int MODE = 2;
     constexpr bool PX = false;
+    const double *__restrict__ lams = nullptr;
+    const double *__restrict__ w = nullptr;
+    double *out = nullptr;
+    const int out_stride = 1, accumulate = 0;
+#include "rows_all_body.inc"
+}
+
+// prediction of a table of models: block row y computes the model tab.m[y] {P_dk, lams, w, out}.  The table is a
+// kernel parameter (no copy, no wait for one), so a single prediction is one launch as before.
+struct PredictTable { sp_predict_model m[SP_PREDICT_MAX_MODELS]; };
+
+template <int DEG, int G>
+__global__ void __launch_bounds__(ROWS_THREADS)
+rows_predict_kernel(int n, int k, const int32_t *__restrict__ indptr, const int32_t *__restrict__ indices,
+                    const double *__restrict__ data, const __grid_constant__ PredictTable tab, int out_stride,
+                    int accumulate) {
+    constexpr int MODE = 0;
+    constexpr bool PX = false;
+    const sp_predict_model &e = tab.m[blockIdx.y];
+    const double *__restrict__ P_dk = e.P_dk;
+    const double *__restrict__ lams = e.lams;
+    const double *__restrict__ w = e.w;
+    double *out = e.out, *Aout = nullptr;
 #include "rows_all_body.inc"
 }
 
@@ -111,41 +133,42 @@ int grid_for(int n, int per_block) {
     return (int)blocks;
 }
 
-template <int DEG, int MODE>
-int launch_all(int n, int k, const int32_t *indptr, const int32_t *indices, const double *data,
-               const double *P_dk, const double *lams, const double *w, double *out, int out_stride,
-               int accumulate, double *Aout, cudaStream_t st) {
+template <int DEG>
+int launch_kernel_matrix(int n, int k, const sp_dataset *ds, const double *P_dk, double *K, cudaStream_t st) {
     sp_prof_begin(SP_PROF_ROWS, st);
     if (k <= 8) {
-        rows_all_kernel<DEG, 8, MODE><<<grid_for(n, ROWS_THREADS / 8), ROWS_THREADS, 0, st>>>(
-            n, k, indptr, indices, data, P_dk, lams, w, out, out_stride, accumulate, Aout);
+        rows_all_kernel<DEG, 8><<<grid_for(n, ROWS_THREADS / 8), ROWS_THREADS, 0, st>>>(
+            n, k, ds->csr_indptr, ds->csr_indices, ds->csr_data, P_dk, K);
     } else if (k <= 16) {
-        rows_all_kernel<DEG, 16, MODE><<<grid_for(n, ROWS_THREADS / 16), ROWS_THREADS, 0, st>>>(
-            n, k, indptr, indices, data, P_dk, lams, w, out, out_stride, accumulate, Aout);
+        rows_all_kernel<DEG, 16><<<grid_for(n, ROWS_THREADS / 16), ROWS_THREADS, 0, st>>>(
+            n, k, ds->csr_indptr, ds->csr_indices, ds->csr_data, P_dk, K);
     } else {
-        rows_all_kernel<DEG, 32, MODE><<<grid_for(n, ROWS_THREADS / 32), ROWS_THREADS, 0, st>>>(
-            n, k, indptr, indices, data, P_dk, lams, w, out, out_stride, accumulate, Aout);
+        rows_all_kernel<DEG, 32><<<grid_for(n, ROWS_THREADS / 32), ROWS_THREADS, 0, st>>>(
+            n, k, ds->csr_indptr, ds->csr_indices, ds->csr_data, P_dk, K);
     }
     sp_prof_end(st);
     SP_LAUNCH_CHECK("rows_all_kernel");
     return SP_OK;
 }
 
-template <int MODE>
-int dispatch_all(int degree, int n, int k, const int32_t *indptr, const int32_t *indices,
-                 const double *data, const double *P_dk, const double *lams, const double *w,
-                 double *out, int out_stride, int accumulate, double *Aout, cudaStream_t st) {
-    switch (degree) {
-    case -1: return launch_all<-1, MODE>(n, k, indptr, indices, data, P_dk, lams, w, out, out_stride, accumulate, Aout, st);
-    case 1: return launch_all<1, MODE>(n, k, indptr, indices, data, P_dk, lams, w, out, out_stride, accumulate, Aout, st);
-    case 2: return launch_all<2, MODE>(n, k, indptr, indices, data, P_dk, lams, w, out, out_stride, accumulate, Aout, st);
-    case 3: return launch_all<3, MODE>(n, k, indptr, indices, data, P_dk, lams, w, out, out_stride, accumulate, Aout, st);
-    case 4: return launch_all<4, MODE>(n, k, indptr, indices, data, P_dk, lams, w, out, out_stride, accumulate, Aout, st);
-    case 5: return launch_all<5, MODE>(n, k, indptr, indices, data, P_dk, lams, w, out, out_stride, accumulate, Aout, st);
-    default:
-        sp_set_error("degree %d is not supported (1..%d or -1 for all-subsets)", degree, SP_MAXDEG);
-        return SP_ERR_UNSUPPORTED;
+// the predictions of n_tab models in one launch, with the group width launch_kernel_matrix picks for k
+template <int DEG>
+int launch_predict(int n, int k, const sp_dataset *ds, const PredictTable &tab, int n_tab, int out_stride,
+                   int accumulate, cudaStream_t st) {
+    sp_prof_begin(SP_PROF_ROWS, st);
+    if (k <= 8) {
+        rows_predict_kernel<DEG, 8><<<dim3(grid_for(n, ROWS_THREADS / 8), n_tab), ROWS_THREADS, 0, st>>>(
+            n, k, ds->csr_indptr, ds->csr_indices, ds->csr_data, tab, out_stride, accumulate);
+    } else if (k <= 16) {
+        rows_predict_kernel<DEG, 16><<<dim3(grid_for(n, ROWS_THREADS / 16), n_tab), ROWS_THREADS, 0, st>>>(
+            n, k, ds->csr_indptr, ds->csr_indices, ds->csr_data, tab, out_stride, accumulate);
+    } else {
+        rows_predict_kernel<DEG, 32><<<dim3(grid_for(n, ROWS_THREADS / 32), n_tab), ROWS_THREADS, 0, st>>>(
+            n, k, ds->csr_indptr, ds->csr_indices, ds->csr_data, tab, out_stride, accumulate);
     }
+    sp_prof_end(st);
+    SP_LAUNCH_CHECK("rows_predict_kernel");
+    return SP_OK;
 }
 
 // the pbcd cache of n_tab entries {P_dk, A} in one launch, with the group width launch_all picks for k
@@ -165,17 +188,42 @@ void launch_pbcd_cache(int n, int k, const sp_dataset *ds, const SpBlockEntry *t
 
 }  // namespace
 
-extern "C" int sp_predict(const sp_dataset *ds, const double *P_dk, int k, const double *lams,
-                          int degree, const double *w, double *out, int out_stride, int accumulate,
-                          sp_stream stream) {
-    if (!ds || !ds->csr_indptr || !P_dk || !lams || !out || k <= 0 || out_stride <= 0) {
+extern "C" int sp_predict_multi(const sp_dataset *ds, const sp_predict_model *models, int n_models, int k,
+                                int degree, int out_stride, int accumulate, sp_stream stream) {
+    if (!ds || !ds->csr_indptr || !models || n_models < 0 || n_models > SP_PREDICT_MAX_MODELS || k <= 0 ||
+        out_stride <= 0) {
         sp_set_error("sp_predict: invalid argument");
         return SP_ERR_INVALID;
     }
-    if (ds->n_samples == 0) return SP_OK;
-    return dispatch_all<0>(degree, ds->n_samples, k, ds->csr_indptr, ds->csr_indices,
-                           ds->csr_data, P_dk, lams, w, out, out_stride, accumulate, nullptr,
-                           (cudaStream_t)stream);
+    PredictTable tab;
+    for (int b = 0; b < n_models; b++) {
+        if (!models[b].P_dk || !models[b].lams || !models[b].out) {
+            sp_set_error("sp_predict: invalid argument (model %d)", b);
+            return SP_ERR_INVALID;
+        }
+        tab.m[b] = models[b];
+    }
+    const int n = ds->n_samples;
+    if (n == 0 || n_models == 0) return SP_OK;
+    cudaStream_t st = (cudaStream_t)stream;
+    switch (degree) {
+    case -1: return launch_predict<-1>(n, k, ds, tab, n_models, out_stride, accumulate, st);
+    case 1: return launch_predict<1>(n, k, ds, tab, n_models, out_stride, accumulate, st);
+    case 2: return launch_predict<2>(n, k, ds, tab, n_models, out_stride, accumulate, st);
+    case 3: return launch_predict<3>(n, k, ds, tab, n_models, out_stride, accumulate, st);
+    case 4: return launch_predict<4>(n, k, ds, tab, n_models, out_stride, accumulate, st);
+    case 5: return launch_predict<5>(n, k, ds, tab, n_models, out_stride, accumulate, st);
+    default:
+        sp_set_error("degree %d is not supported (1..%d or -1 for all-subsets)", degree, SP_MAXDEG);
+        return SP_ERR_UNSUPPORTED;
+    }
+}
+
+extern "C" int sp_predict(const sp_dataset *ds, const double *P_dk, int k, const double *lams,
+                          int degree, const double *w, double *out, int out_stride, int accumulate,
+                          sp_stream stream) {
+    const sp_predict_model m = {P_dk, lams, w, out};
+    return sp_predict_multi(ds, &m, 1, k, degree, out_stride, accumulate, stream);
 }
 
 extern "C" int sp_kernel_matrix(const sp_dataset *ds, const double *P_dk, int k, int degree, double *K,
@@ -184,10 +232,20 @@ extern "C" int sp_kernel_matrix(const sp_dataset *ds, const double *P_dk, int k,
         sp_set_error("sp_kernel_matrix: invalid argument");
         return SP_ERR_INVALID;
     }
-    if (ds->n_samples == 0) return SP_OK;
-    return dispatch_all<2>(degree, ds->n_samples, k, ds->csr_indptr, ds->csr_indices,
-                           ds->csr_data, P_dk, nullptr, nullptr, nullptr, 1, 0, K,
-                           (cudaStream_t)stream);
+    const int n = ds->n_samples;
+    if (n == 0) return SP_OK;
+    cudaStream_t st = (cudaStream_t)stream;
+    switch (degree) {
+    case -1: return launch_kernel_matrix<-1>(n, k, ds, P_dk, K, st);
+    case 1: return launch_kernel_matrix<1>(n, k, ds, P_dk, K, st);
+    case 2: return launch_kernel_matrix<2>(n, k, ds, P_dk, K, st);
+    case 3: return launch_kernel_matrix<3>(n, k, ds, P_dk, K, st);
+    case 4: return launch_kernel_matrix<4>(n, k, ds, P_dk, K, st);
+    case 5: return launch_kernel_matrix<5>(n, k, ds, P_dk, K, st);
+    default:
+        sp_set_error("degree %d is not supported (1..%d or -1 for all-subsets)", degree, SP_MAXDEG);
+        return SP_ERR_UNSUPPORTED;
+    }
 }
 
 // pbcd cache precompute of n_tab models in one launch: entry y is {P_dk, A} of one model, A [n, m-1, k] (ANOVA)

@@ -1,5 +1,6 @@
 """fit_many: fit many pcd or pbcd models on one design matrix at once (DESIGN.md 3.2 / 3.3, "Many models per
-launch").
+launch"); decision_function_many / predict_many / score_many / objective_many: evaluate many fitted models on one
+design matrix at once (DESIGN.md 3.1 / 3.5).
 
 A pcd or pbcd fit is one sequential coordinate chain and, at the sizes the reference is used at (hyper-parameter
 grids, one-vs-rest classes, gamma sweeps of the feature-selecting regularizers), one chain fills a single
@@ -17,9 +18,13 @@ import warnings
 import numpy as np
 import torch
 import scipy.sparse as sp
+from sklearn.base import ClassifierMixin
+from sklearn.exceptions import NotFittedError
+from sklearn.metrics import accuracy_score, r2_score
 from sklearn.utils import check_random_state
+from sklearn.utils.validation import check_array
 
-from . import _lib, solvers
+from . import _lib, objective as _objective, solvers
 from .dataset import DeviceDataset, SweepPlan, _device, choose_geometry
 from .estimators import _BaseSparseAllSubsets, _BaseSparseFactorizationMachine
 
@@ -30,11 +35,11 @@ _SHARED_FM = ("degree", "n_components", "loss", "fit_lower", "fit_linear")
 _SHARED_ALL = ("n_components", "loss")
 
 
-def _targets(y, n_models):
+def _targets(y, n_models, what="fit_many"):
     """One target per model: y itself, or the elements of a sequence of arrays."""
     if isinstance(y, (list, tuple)) and len(y) > 0 and all(np.ndim(t) >= 1 for t in y):
         if len(y) != n_models:
-            raise ValueError(f"fit_many: {len(y)} target arrays for {n_models} estimators")
+            raise ValueError(f"{what}: {len(y)} target arrays for {n_models} estimators")
         return list(y)
     return [y] * n_models
 
@@ -328,3 +333,261 @@ def fit_many(estimators, X, y):
         if not m.converged:
             warnings.warn("Objective did not converge. Increase max_iter.")
     return ests
+
+
+# ------------------------------------------------------------------------------ scoring many fitted models
+# parameters that fix the augmented X, the output orders and the kernel instantiation: equal across a scoring call
+_SCORE_SHARED_FM = ("degree", "n_components", "fit_lower", "fit_linear")
+_SCORE_SHARED_ALL = ("n_components",)
+SCORE_MAX_MODELS = min(_lib.PREDICT_MAX_MODELS, _lib.OBJECTIVE_MAX_ENTRIES)   # models per chunk: the kernel tables
+
+
+def _validate_fitted(ests, what):
+    """The checks of a scoring call that need no device: returns fm (factorization machine, not all-subsets)."""
+    first = ests[0]
+    if not isinstance(first, (_BaseSparseFactorizationMachine, _BaseSparseAllSubsets)):
+        raise ValueError(f"{what}: {type(first).__name__} is not a SparseFactorizationMachine or SparseAllSubsets "
+                         "estimator")
+    fm = isinstance(first, _BaseSparseFactorizationMachine)
+    for i, e in enumerate(ests):
+        if type(e) is not type(first):
+            raise ValueError(f"{what}: estimator {i} is a {type(e).__name__} and estimator 0 a "
+                             f"{type(first).__name__}; all estimators must be of one class")
+        if not hasattr(e, "P_"):
+            raise NotFittedError(f"{what}: estimator {i} is not fitted.")
+        for name in (_SCORE_SHARED_FM if fm else _SCORE_SHARED_ALL):
+            if getattr(e, name) != getattr(first, name):
+                raise ValueError(f"{what}: {name} must be equal across the estimators "
+                                 f"(estimator {i}: {getattr(e, name)!r}, estimator 0: {getattr(first, name)!r})")
+    return fm
+
+
+def _n_dummies(est):
+    """Dummy columns _augment adds (sparse_factorization_machines.py:86-92)."""
+    if est.fit_lower != "augment":
+        return 0
+    return max(0, est.degree - (2 if est.fit_linear else 1))
+
+
+def _check_X(ests, X, fm, what):
+    """X as the single-model _predict checks and augments it (0 rows allowed), after the checks that the models fit
+    it: every P_ of the call's shape, as wide as X after augmentation, and w_ / lams_ to match."""
+    first = ests[0]
+    X = check_array(X, accept_sparse=["csr", "csc"], dtype=np.double, ensure_min_samples=0)
+    if fm and X.shape[0] > 0:
+        X = first._augment(X)
+    d = X.shape[1] + (_n_dummies(first) if fm and X.shape[0] == 0 else 0)
+    k = first.n_components
+    shape = ((first.degree - 1 if first.fit_lower == "explicit" else 1), k, d) if fm else (k, d)
+    for i, e in enumerate(ests):
+        P_shape = np.shape(e.P_)
+        if P_shape[-1:] != (d,):
+            raise ValueError(f"{what}: X has {d} features" + (" after augmentation" if _n_dummies(first) else "") +
+                             f"; estimator {i} was fitted with {P_shape[-1] if P_shape else 0}")
+        if P_shape != shape or np.shape(e.lams_) != (k,) or (fm and np.shape(e.w_) != (d,)):
+            raise ValueError(f"{what}: estimator {i} has P_ {P_shape}, lams_ {np.shape(e.lams_)}"
+                             + (f", w_ {np.shape(e.w_)}" if fm else "") + f"; a model of this call has P_ {shape}")
+    return X, shape
+
+
+def _score_bytes(n, nnz, shape, objective):
+    """(shared, per model) device bytes of a scoring call: X's CSR, and per model P twice (as uploaded and
+    feature-major), w, lams and its scores; objective_many adds the targets and the reduction work."""
+    n_orders, k, d = shape if len(shape) == 3 else (1,) + shape
+    shared = 12 * nnz + 4 * (n + 1) + 8 * d
+    model = 8 * (2 * n_orders * k * d + d + k + max(n, 1))
+    if objective:
+        model += 8 * (max(n, 1) + solvers.reg_eval_work_doubles(d, k) + solvers.sum_work_doubles() + 8)
+    return shared, model
+
+
+def _chunk_size(ests, n, nnz, shape, objective, what):
+    shared, model = _score_bytes(n, nnz, shape, objective)
+    free = _free_device_bytes()
+    fit = int((free - shared) // model) if free > shared else 0
+    if fit < 1:
+        raise ValueError(f"{what}: one model of this shape needs {model / 2**20:.1f} MiB of device memory next to "
+                         f"X's {shared / 2**20:.1f} MiB and {free / 2**20:.1f} MiB are free")
+    return max(1, min(SCORE_MAX_MODELS, fit))
+
+
+class _Chunk:
+    """Device state of one chunk of a scoring call: the models' P (feature-major), w, lams and scores."""
+
+    def __init__(self, ests, fm, ds, n, shape, dev):
+        first = ests[0]
+        B = len(ests)
+        n_orders, k, d = shape if fm else (1,) + shape
+        P = torch.from_numpy(np.stack([np.asarray(e.P_, dtype=np.float64) for e in ests]).reshape(B * n_orders, k, d))
+        self.P_dk = solvers.transpose_batch(P.to(dev)).view(B, n_orders, d, k)   # one H2D, one transpose launch
+        self.lams = torch.from_numpy(np.stack([np.asarray(e.lams_, dtype=np.float64) for e in ests])).to(dev)
+        self.w = torch.from_numpy(np.stack([np.asarray(e.w_, dtype=np.float64) for e in ests])).to(dev) if fm else None
+        self.out = torch.zeros((B, max(n, 1)), dtype=_f64, device=dev)
+        if n == 0:
+            return
+        orders = first._output_orders() if fm else [(0, -1)]
+        for j, (o, deg) in enumerate(orders):          # the launches of _device_output, each over the whole chunk
+            tab = (_lib.SpPredictModel * B)()
+            for b in range(B):
+                w = self.w[b].data_ptr() if (fm and j == 0 and first.fit_linear) else None
+                tab[b] = _lib.SpPredictModel(P_dk=self.P_dk[b, o].data_ptr(), lams=self.lams[b].data_ptr(), w=w,
+                                             out=self.out[b].data_ptr())
+            solvers.predict_multi(ds, tab, k, deg, accumulate=j > 0)
+
+
+def _prepare(ests, X, what):
+    """Every check of a scoring call that needs no device: returns (fm, X checked and augmented, P_'s shape)."""
+    fm = _validate_fitted(ests, what)
+    Xc, shape = _check_X(ests, X, fm, what)
+    return fm, Xc, shape
+
+
+def _run_chunks(ests, Xc, fm, shape, what, objective=False):
+    """Upload X once and yield (b0, b1, chunk) over chunks of the models that fit the device."""
+    n = Xc.shape[0]
+    size = _chunk_size(ests, n, Xc.nnz if sp.issparse(Xc) else Xc.size, shape, objective, what)
+    dev = _device()
+    _lib.check(_lib.load().sp_set_device(dev.index if dev.index is not None else 0))
+    ds = DeviceDataset(Xc, need_csr=True, need_csc=False, device=dev) if n > 0 else None
+    for b0 in range(0, len(ests), size):
+        b1 = min(len(ests), b0 + size)
+        yield b0, b1, _Chunk(ests[b0:b1], fm, ds, n, shape, dev)
+
+
+def decision_function_many(estimators, X):
+    """Outputs of many fitted estimators on one design matrix: ndarray [n_models, n_samples] whose row b is
+    estimators[b].decision_function(X) (classifiers) or estimators[b].predict(X) (regressors), bit for bit.
+
+    estimators: fitted SparseFactorizationMachine{Regressor,Classifier} or SparseAllSubsets{Regressor,Classifier}
+    instances of one class; factorization machines with equal degree, n_components, fit_lower and fit_linear,
+    all-subsets models with equal n_components.  Solver, regularizer, loss, alpha / beta / gamma and mean may differ,
+    and so may how P_ was obtained (any solver, partial_fit, fit_many, warm start, set by hand).
+
+    X is checked, augmented and uploaded once; the models' P_ / w_ / lams_ go up stacked, in one copy each, and
+    every output order is one launch over all models of a chunk.  Chunks hold up to SCORE_MAX_MODELS models and as
+    many as the free device memory holds; results do not depend on the chunking."""
+    return _decision(list(estimators), X, "decision_function_many")
+
+
+def _decision(ests, X, what):
+    if not ests:
+        X = check_array(X, accept_sparse=["csr", "csc"], dtype=np.double, ensure_min_samples=0)
+        return np.zeros((0, X.shape[0]))
+    return _device_decision(ests, *_prepare(ests, X, what), what)
+
+
+def _device_decision(ests, fm, Xc, shape, what):
+    n = Xc.shape[0]
+    out = np.empty((len(ests), n))
+    for b0, b1, ch in _run_chunks(ests, Xc, fm, shape, what):
+        out[b0:b1] = ch.out[:, :n].cpu().numpy()          # one D2H per chunk
+        del ch                                            # before the next chunk is allocated
+    return out
+
+
+def _labels(ests, dec):
+    """Rows of predict(): the decision rows, or for classifiers their labels through each model's binarizer."""
+    if isinstance(ests[0], ClassifierMixin):
+        return [e.label_binarizer_.inverse_transform(dec[b] > 0) for b, e in enumerate(ests)]
+    return list(dec)
+
+
+def predict_many(estimators, X):
+    """Predictions of many fitted estimators on one design matrix: [n_models, n_samples], row b equal to
+    estimators[b].predict(X) (classifiers: labels through each model's own label_binarizer_; when the models' label
+    types differ, an object array).  The estimators are those decision_function_many accepts."""
+    ests = list(estimators)
+    if not ests:
+        return _decision(ests, X, "predict_many")
+    rows = _labels(ests, _decision(ests, X, "predict_many"))
+    if len({r.dtype for r in rows}) == 1:
+        return np.stack(rows)
+    out = np.empty((len(rows), len(rows[0])), dtype=object)
+    for b, r in enumerate(rows):
+        out[b] = r
+    return out
+
+
+def _check_targets(ests, y, n, what):
+    ys = _targets(y, len(ests), what)
+    for b, yb in enumerate(ys):
+        if len(yb) != n:
+            raise ValueError(f"{what}: target {b} has {len(yb)} samples and X has {n}")
+    return ys
+
+
+def score_many(estimators, X, y):
+    """Scores of many fitted estimators on one design matrix: ndarray [n_models], entry b equal to
+    estimators[b].score(X, y_b) -- R^2 for regressors, accuracy for classifiers -- computed on the host from
+    predict_many.  y: one target array for every model, or a sequence of one per estimator (one-vs-rest)."""
+    ests = list(estimators)
+    if not ests:
+        return np.zeros(0)
+    fm, Xc, shape = _prepare(ests, X, "score_many")
+    ys = _check_targets(ests, y, Xc.shape[0], "score_many")
+    rows = _labels(ests, _device_decision(ests, fm, Xc, shape, "score_many"))
+    metric = accuracy_score if isinstance(ests[0], ClassifierMixin) else r2_score
+    return np.array([float(metric(yb, r)) for yb, r in zip(ys, rows)])
+
+
+def objective_many(estimators, X, y):
+    """objective(est, X, y_b) of many fitted estimators on one design matrix: a list of dicts (loss, l2_w, l2_P,
+    omega, total), entry b equal to sparsepoly_b200.objective(estimators[b], X, y_b) key by key, bit for bit.  y: one
+    target array for every model, or a sequence of one per estimator.  Each reduction is one launch pair over all
+    models of a chunk (Omega: at most two partial launches, one per fold kind, per order); the estimators are those
+    decision_function_many accepts."""
+    ests = list(estimators)
+    if not ests:
+        return []
+    what = "objective_many"
+    fm, Xc, shape = _prepare(ests, X, what)
+    n = Xc.shape[0]
+    ys = _check_targets(ests, y, n, what)
+    n_orders, k, d = shape if fm else (1,) + shape
+    results = []
+    for b0, b1, ch in _run_chunks(ests, Xc, fm, shape, what, objective=True):
+        results += _chunk_objective(ests[b0:b1], ys[b0:b1], ch, fm, n, n_orders, k, d)
+        del ch                                            # before the next chunk is allocated
+    return results
+
+
+def _chunk_objective(chunk, ys, ch, fm, n, n_orders, k, d):
+    first = chunk[0]
+    B, dev = len(chunk), ch.out.device
+    y_dev = torch.zeros((B, max(n, 1)), dtype=_f64)
+    if n > 0:
+        y_dev[:, :n] = torch.from_numpy(np.stack([_objective._targets(e, yb) for e, yb in zip(chunk, ys)]))
+    y_dev = y_dev.to(dev)
+    parts = torch.zeros((4, B), dtype=_f64, device=dev)          # loss, l2_w, l2_P, omega
+    sum_work = torch.empty(B * solvers.sum_work_doubles(), dtype=_f64, device=dev)
+    loss_tab = (_lib.SpLossEntry * B)()
+    for b, e in enumerate(chunk):
+        loss_tab[b] = _lib.SpLossEntry(y_pred=ch.out[b].data_ptr(), y=y_dev[b].data_ptr(),
+                                       loss=_lib.LOSS_IDS[e.loss], out=parts[0, b].data_ptr())
+    solvers.loss_sum_multi(loss_tab, n, sum_work)
+    if fm and first.fit_linear:
+        w_tab = (_lib.SpSqnormEntry * B)()
+        for b in range(B):
+            w_tab[b] = _lib.SpSqnormEntry(v=ch.w[b].data_ptr(), out=parts[1, b].data_ptr())
+        solvers.sqnorm_multi(w_tab, d, sum_work)
+    reg_work = torch.empty(B * solvers.reg_eval_work_doubles(d, k), dtype=_f64, device=dev)
+    per_order = torch.empty((2, B), dtype=_f64, device=dev)
+    for o in range(n_orders):                       # l2_P and omega: 0 + order 0 + order 1 ..., as objective()
+        sq_tab, reg_tab = (_lib.SpSqnormEntry * B)(), (_lib.SpRegEntry * B)()
+        for b, e in enumerate(chunk):
+            P = ch.P_dk[b, o].data_ptr()
+            sq_tab[b] = _lib.SpSqnormEntry(v=P, out=per_order[0, b].data_ptr())
+            reg_tab[b] = _lib.SpRegEntry(P_dk=P, reg=_lib.REG_IDS[e.regularizer], out=per_order[1, b].data_ptr())
+        solvers.sqnorm_multi(sq_tab, d * k, sum_work)
+        solvers.reg_eval_multi(reg_tab, d, k, first.degree - o if fm else -1, reg_work)
+        parts[2:] += per_order
+    host = parts.cpu().numpy()                      # one D2H per chunk
+    results = []
+    for b, e in enumerate(chunk):
+        scale = n if e.mean else 1
+        alpha = e.alpha * scale if fm else 0.0
+        beta, gamma = e.beta * scale, e.gamma * scale
+        out = dict(loss=float(host[0, b]), l2_w=float(host[1, b]), l2_P=float(host[2, b]), omega=float(host[3, b]))
+        out["total"] = out["loss"] + 0.5 * alpha * out["l2_w"] + 0.5 * beta * out["l2_P"] + gamma * out["omega"]
+        results.append(out)
+    return results

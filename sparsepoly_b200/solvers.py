@@ -30,6 +30,14 @@ def transpose(t):
     return out
 
 
+def transpose_batch(t):
+    """Device transpose of every matrix of a 3-D fp64 tensor [batch, rows, cols] in one launch (sp_transpose_f64_batch)."""
+    batch, rows, cols = t.shape
+    out = torch.empty((batch, cols, rows), dtype=_f64, device=t.device)
+    _lib.check(_L().sp_transpose_f64_batch(_ptr(t), _ptr(out), batch, rows, cols, _stream()))
+    return out
+
+
 def poly_predict(ds, P_dk, lams, degree, w=None, out=None, out_stride=1, accumulate=False):
     """kernels.poly_predict on device (kernels.py:140-153): out[i*stride] (+)= <w,x_i> +
     sum_s lams[s] K(P[:,s], x_i); degree=-1 selects the all-subsets kernel."""
@@ -38,6 +46,12 @@ def poly_predict(ds, P_dk, lams, degree, w=None, out=None, out_stride=1, accumul
     _lib.check(_L().sp_predict(ds.ref(), _ptr(P_dk), int(P_dk.shape[1]), _ptr(lams), int(degree),
                                _ptr(w), _ptr(out), int(out_stride), int(bool(accumulate)), _stream()))
     return out
+
+
+def predict_multi(ds, models, k, degree, out_stride=1, accumulate=False):
+    """poly_predict of every model of a ctypes SpPredictModel array (<= _lib.PREDICT_MAX_MODELS) in one launch."""
+    _lib.check(_L().sp_predict_multi(ds.ref(), models, len(models), int(k), int(degree), int(out_stride),
+                                     int(bool(accumulate)), _stream()))
 
 
 def cd_linear_epoch(ds, plan, w, col_norm_sq, alpha, loss, rec, stride, viol):
@@ -231,3 +245,29 @@ def reg_eval(P_dk, reg, degree):
     _lib.check(_L().sp_reg_eval(_ptr(P_dk), int(d), int(k), _lib.REG_IDS[reg], int(degree), _ptr(work),
                                 _ptr(out), _stream()))
     return out
+
+
+def loss_sum_multi(entries, n, work, pred_stride=1, y_stride=1):
+    """loss_sum of every entry of a ctypes SpLossEntry array (<= _lib.OBJECTIVE_MAX_ENTRIES); work holds
+    len(entries) * sp_sum_work_doubles() doubles."""
+    _lib.check(_L().sp_loss_sum_multi(entries, len(entries), int(pred_stride), int(y_stride), int(n), _ptr(work),
+                                      _stream()))
+
+
+def sqnorm_multi(entries, length, work):
+    """sqnorm of every entry of a ctypes SpSqnormEntry array, all of `length` doubles."""
+    _lib.check(_L().sp_sqnorm_multi(entries, len(entries), int(length), _ptr(work), _stream()))
+
+
+def reg_eval_multi(entries, d, k, degree, work):
+    """reg_eval of every entry of a ctypes SpRegEntry array, all [d,k] at this degree; work holds
+    len(entries) * sp_reg_eval_work_doubles(d, k) doubles."""
+    _lib.check(_L().sp_reg_eval_multi(entries, len(entries), int(d), int(k), int(degree), _ptr(work), _stream()))
+
+
+def sum_work_doubles():
+    return int(_L().sp_sum_work_doubles())
+
+
+def reg_eval_work_doubles(d, k):
+    return int(_L().sp_reg_eval_work_doubles(int(d), int(k)))
