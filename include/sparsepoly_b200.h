@@ -391,7 +391,8 @@ int sp_psgd_plan_begin(sp_psgd_ctx *ctx, sp_stream stream);
 /* minibatches [m_begin, m_end) of psgd.psgd_epoch (psgd.py:150-198): per minibatch the rows pass
  * (_pred, psgd.py:47-57), the column pass (_update_grads + the SGD step of _update_params,
  * psgd.py:60-117, on the touched rows only) and the prox (psgd.py:119-122) as a lazily applied column
- * threshold; *it_io_host advances once per minibatch. */
+ * threshold; *it_io_host advances once per minibatch.  After a minibatch that takes C or Cw out of
+ * (1e-100, 1e100) the frame is folded into P / w (thr = 0, C = Cw = 1), so the scales never overflow. */
 int sp_psgd_plan_run(sp_psgd_ctx *ctx, const sp_dataset *ds, const sp_psgd_plan *plan, const double *y,
                      const int32_t *idx_samples, double alpha, double beta, double gamma, double eta0,
                      int learning_rate, double power_t, int m_begin, int m_end, int64_t *it_io_host,

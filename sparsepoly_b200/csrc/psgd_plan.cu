@@ -1567,6 +1567,32 @@ extern "C" int sp_psgd_plan_begin(sp_psgd_ctx *cx, sp_stream stream) {
     return SP_OK;
 }
 
+// The lazy scales only grow (by 1 + eta * beta per minibatch): the frame is folded back into the storage as soon
+// as C or Cw leaves (1e-100, 1e100), long before either can overflow.  The rule depends on the C trajectory alone,
+// so every way of cutting the same minibatches into calls (epochs, partial_fit chunks) folds after the same ones.
+constexpr double FRAME_MAX = 1e100;
+static inline bool frame_in_range(double C, double Cw) {
+    return 1.0 / FRAME_MAX < C && C < FRAME_MAX && 1.0 / FRAME_MAX < Cw && Cw < FRAME_MAX;
+}
+
+// P / w <- the model the frame represents, thresholds 0, scales 1; sharded: every rank's rows are folded before
+// any rank reads a peer's rows again
+static int fold_frame(sp_psgd_ctx *cx, cudaStream_t st) {
+    const size_t n = (size_t)cx->n_orders * cx->d_rows * cx->k;
+    if (n > 0) {
+        size_t b = (n + 255) / 256;
+        if (b > 148 * 16) b = 148 * 16;
+        psgd_materialize_kernel<<<(int)b, 256, 0, st>>>(cx->P, cx->n_orders, (size_t)cx->d_rows, cx->k, cx->thr, 1.0 / cx->C,
+                                                      cx->w, 1.0 / cx->Cw, cx->fit_linear);
+        SP_LAUNCH_CHECK("psgd_materialize_kernel");
+    }
+    psgd_zero_kernel<<<1, 256, 0, st>>>(cx->thr, cx->n_orders * cx->k);
+    SP_LAUNCH_CHECK("psgd_zero_kernel");
+    cx->C = 1.0; cx->Cw = 1.0;
+    if (cx->world > 1) { cx->seq += 1; return xbarrier(cx, 0, cx->seq, st); }
+    return SP_OK;
+}
+
 // Minibatches [m_begin, m_end) of one epoch = the body of psgd.psgd_epoch (psgd.py:150-198) for them.
 extern "C" int sp_psgd_plan_run(sp_psgd_ctx *cx, const sp_dataset *ds, const sp_psgd_plan *pl, const double *y,
                                 const int32_t *idx_samples, double alpha, double beta, double gamma, double eta0,
@@ -1642,6 +1668,7 @@ extern "C" int sp_psgd_plan_run(sp_psgd_ctx *cx, const sp_dataset *ds, const sp_
         sa.rP = 1.0 / sa.denP; sa.rw = 1.0 / sa.denw;
         sa.fit_linear = cx->fit_linear;
         const double strength = gamma * eta_P / (1.0 + eta_P * beta);                     // psgd.py:122
+        const bool fold = !frame_in_range(sa.CnP, sa.Cnw);                // the frame is folded after this minibatch
         if (sharded) SP_CUDA(cudaStreamWaitEvent(st, ev_pull, 0));          // this minibatch's rows are staged
 #define SP_MB(D, N, GG, KC) rc = launch_minibatch<D, N, GG, KC>(cx, ds, pl, y, idx_samples, mb, sa, st)
 #define SP_MB_K(D, N)                                                                      \
@@ -1684,7 +1711,8 @@ extern "C" int sp_psgd_plan_run(sp_psgd_ctx *cx, const sp_dataset *ds, const sp_
 #undef SP_OW
             sp_prof_end(st);
             if (rc) return rc;
-            if (m + 1 < m_end) {                                   // next minibatch's rows: see above
+            if (m + 1 < m_end && !fold) {                          // next minibatch's rows: see above (after a fold they
+                                                                   // are pulled once every rank's rows are folded)
                 SP_CUDA(cudaEventRecord(ev_own, st));
                 SP_CUDA(cudaStreamWaitEvent(s2, ev_own, 0));
                 cx->seq_pull += 1;
@@ -1755,6 +1783,16 @@ extern "C" int sp_psgd_plan_run(sp_psgd_ctx *cx, const sp_dataset *ds, const sp_
             sp_prof_end(st);
             if (e != cudaSuccess) return sp_check_cuda(e, "psgd_solve_kernel launch");
         }
+        if (fold) {
+            rc = fold_frame(cx, st);
+            if (rc) return rc;
+            if (sharded && m + 1 < m_end) {                        // (fold_frame ended with a cross-rank barrier)
+                SP_CUDA(cudaEventRecord(ev_own, st));
+                SP_CUDA(cudaStreamWaitEvent(s2, ev_own, 0));
+                rc = pull(m + 1);
+                if (rc) return rc;
+            }
+        }
         it++;
     }
     *it_io_host = it;
@@ -1775,20 +1813,7 @@ extern "C" int sp_psgd_plan_end(sp_psgd_ctx *cx, int n_local, double *loss_sum, 
         psgd_loss_sum_kernel<<<1, 256, 0, st>>>(part, loss_sum);
         SP_LAUNCH_CHECK("psgd_loss_sum_kernel");
     }
-    if (materialize) {
-        const size_t n = (size_t)cx->n_orders * cx->d_rows * cx->k;
-        if (n > 0) {
-            size_t b = (n + 255) / 256;
-            if (b > 148 * 16) b = 148 * 16;
-            psgd_materialize_kernel<<<(int)b, 256, 0, st>>>(cx->P, cx->n_orders, (size_t)cx->d_rows, cx->k, cx->thr, 1.0 / cx->C,
-                                                          cx->w, 1.0 / cx->Cw, cx->fit_linear);
-            SP_LAUNCH_CHECK("psgd_materialize_kernel");
-        }
-        psgd_zero_kernel<<<1, 256, 0, st>>>(cx->thr, cx->n_orders * cx->k);
-        SP_LAUNCH_CHECK("psgd_zero_kernel");
-        cx->C = 1.0; cx->Cw = 1.0;
-        if (cx->world > 1) { cx->seq += 1; rc = xbarrier(cx, 0, cx->seq, st); if (rc) return rc; }
-    }
+    if (materialize) return fold_frame(cx, st);
     return SP_OK;
 }
 

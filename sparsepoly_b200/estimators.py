@@ -518,10 +518,10 @@ class _BaseSparseFactorizationMachine(_SparsePolyBase, metaclass=ABCMeta):
             self.it_ = solvers.psgd_planned_run(ctx, data["ds"], data["plan"], data["y"], data["idx"], self.alpha,
                                                 self.beta, self.gamma, self.eta0, m["learning_rate"], self.power_t,
                                                 self.it_)
-            # the lazy scales only grow: fold them back into the storage long before they overflow
-            big = not (1e-100 < ctx.struct.C < 1e100 and 1e-100 < ctx.struct.Cw < 1e100)
-            solvers.psgd_planned_end(ctx, data["n"], loss, big)
-            m["model_current"] = big
+            # (the run folds the lazy scales back into the storage after any minibatch that takes them out of
+            # (1e-100, 1e100); sync() materialises the frame the pass leaves)
+            solvers.psgd_planned_end(ctx, data["n"], loss, False)
+            m["model_current"] = False
         else:
             self.it_ = solvers.psgd_epoch(data["ds"], data["y"], m["P"], m["w"], m["lams"], self.degree, self.alpha,
                                           self.beta, self.gamma, self.regularizer, self.loss, m["grad_P"],

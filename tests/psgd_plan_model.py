@@ -128,10 +128,20 @@ class RankState:
         self.sloss = np.zeros(plan.n_local)
 
 
+FRAME_MAX = 1e100
+
+
+def frame_in_range(C, Cw):
+    """sp_psgd_plan_run folds the frame into the storage after a minibatch that takes C or Cw out of this range."""
+    return 1.0 / FRAME_MAX < C < FRAME_MAX and 1.0 / FRAME_MAX < Cw < FRAME_MAX
+
+
 def run_model(ranks, d, n_orders, k, degree, reg, loss, fit_linear, lams, alpha, beta, gamma, eta0, lr, power_t, it,
-              P_odk, w, epochs=1):
+              P_odk, w, epochs=1, folds=None):
     """`epochs` epochs over the plans of `ranks` (list of RankState, one per simulated rank).  P_odk [o,d,k] / w [d]
-    are updated in place; returns (it, sum of losses of the last epoch)."""
+    are updated in place; returns (it, sum of losses of the last epoch).  `folds` (a list) receives the `it` of
+    every minibatch after which the frame was folded."""
+    folds = [] if folds is None else folds
     G = len(ranks)
     ncol = n_orders * k
     for r, R in enumerate(ranks):                       # load_model
@@ -315,9 +325,10 @@ def run_model(ranks, d, n_orders, k, degree, reg, loss, fit_linear, lams, alpha,
                         if fit_linear:
                             R.w[q] = ((R.w[q] * invCw - gw * cw) / denw) * Cnw
             C, Cw = CnP, Cnw
+            fold = not frame_in_range(C, Cw)
             # ---- early pull of the next minibatch's raw rows (every owner's rows are final; the prox below only
-            #      moves thr)
-            if m + 1 < M:
+            #      moves thr); after a fold the rows are read from the folded storage instead
+            if m + 1 < M and not fold:
                 for r, R in enumerate(ranks):
                     nf = R.u_feat[R.plan.mb_uptr[m + 1]:R.plan.mb_uptr[m + 2]]
                     early[r] = (np.stack([ranks[j % G].P[:, j // G, :].copy() for j in nf]) if len(nf) else np.zeros((0, n_orders, k)),
@@ -331,6 +342,14 @@ def run_model(ranks, d, n_orders, k, degree, reg, loss, fit_linear, lams, alpha,
                     for s in range(k):
                         vals = np.concatenate([np.maximum(np.abs(R.P[o, :, s]) - thr[o, s], 0.0) * invCn for R in ranks])
                         thr[o, s] = thr[o, s] + C * michelot(vals[vals > 0], strength)
+            if fold:                                    # psgd_materialize_kernel + threshold reset (fold_frame)
+                for R in ranks:
+                    R.P[:] = st_true(R.P, thr[:, None, :], 1.0 / C)
+                    if fit_linear:
+                        R.w[:] = R.w * (1.0 / Cw)
+                thr = np.zeros((n_orders, k))
+                C = Cw = 1.0
+                folds.append(it)
             it += 1
         sum_loss = sum(float(R.sloss.sum()) for R in ranks)
     for r, R in enumerate(ranks):                       # materialise + store_model

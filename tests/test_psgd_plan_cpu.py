@@ -190,3 +190,34 @@ def test_band_solve_reports_a_miss():
         above = vals[vals > b_hi]
         band = vals[(vals > b_lo) & ~(vals > b_hi)]
         assert M.band_solve(band, float(above.sum()), float(above.size), strength, b_lo, b_hi) is None
+
+
+# ---------------------------------------------------------------- long horizons of the lazy frame
+def test_plan_model_folds_the_frame_inside_an_epoch():
+    """batch_size=1 with eta * alpha = 0.5: Cw grows by 1.5 per minibatch and would overflow after ~1750 of them
+    (every w then reads back as 0; w itself stays O(1), held by the loss).  The model folds the frame after every
+    minibatch that takes Cw past 1e100 -- here three times inside one epoch -- and ends at the oracle's model."""
+    n, d, k = 2000, 40, 4
+    X = synth.uniform_sparse(n, d, 5, 11)
+    y = np.where(np.random.RandomState(5).rand(n) < 0.4, 1.0, -1.0)
+    kw = dict(degree=2, loss="logistic", n_components=k, solver="psgd", regularizer="squaredl12", alpha=1.0, beta=0.02,
+              gamma=1e-4, eta0=0.5, learning_rate="constant", fit_lower=None)
+    idx = np.arange(n, dtype=np.int32)
+    plan = _plans([X], [idx], d, 1)[0]
+    ranks = [RankState(plan, (X.indptr, X.indices, X.data), y, idx, 1, k, 2)]
+    P = np.ascontiguousarray((0.01 * np.random.RandomState(0).randn(1, k, d)).swapaxes(1, 2))
+    w = np.zeros(d)
+    folds = []
+    it, _ = run_model(ranks, d, 1, k, 2, "squaredl12", "logistic", True, np.ones(k), kw["alpha"], kw["beta"],
+                      kw["gamma"], kw["eta0"], "constant", 1.0, 1, P, w, folds=folds)
+    # Cw after the minibatch of `it` = 1.5 ** (minibatches since the last fold): folded after 568, 1136, 1704;
+    # C = 1.01 ** 2000 stays far below the bound
+    assert 1.5 ** 567 < 1e100 < 1.5 ** 568 and 1.01 ** n < 1e10
+    assert folds == [568, 1136, 1704]
+    out = _oracle_fit(X, y, dict(kw, batch_size=1), 1)
+    P_ref = out["P_"].swapaxes(1, 2)
+    assert 0.2 < np.mean(P_ref != 0) and np.all(np.isfinite(P)) and np.max(np.abs(out["w_"])) > 1e-3
+    assert np.max(np.abs(P - P_ref)) <= 1e-9 * np.max(np.abs(P_ref))
+    assert np.array_equal(P != 0, P_ref != 0)
+    assert np.max(np.abs(w - out["w_"])) <= 1e-9 * np.max(np.abs(out["w_"]))
+    assert it == out["it_"] == n + 1
