@@ -480,6 +480,40 @@ int sp_sqnorm_multi(const sp_sqnorm_entry *entries, int n_entries, int64_t len, 
 int sp_reg_eval_multi(const sp_reg_entry *entries, int n_entries, int d, int k, int degree, double *work,
                       sp_stream stream);
 
+/* Device input (DESIGN.md 2): a design matrix that is already on the GPU, checked and converted there.  These are
+ * the only entries whose input may be int32 OR int64 (indptr, indices) and fp32 OR fp64 (values).
+ *
+ * sp_csr_prepare: one pass over a CSR (indptr != NULL; `indptr_i64` / `indices_i64` / `values_f64` pick the types)
+ * or a dense strided matrix (indptr == NULL: X[i, j] = values[i*stride_row + j*stride_col], every entry stored).
+ * It fills report[SP_CSR_REPORT_LEN] (initialised by the call; "first" entries are the lowest offending row, or
+ * INT64_MAX when there is none):
+ *   [0] first row i with indptr[i+1] < indptr[i]     [1] indptr[0]       [2] indptr[n_rows] (dense: n_rows*n_cols)
+ *   [3] first row with a column outside [0, n_cols)   [4] first row holding a NaN   [5] first row holding +-inf
+ *   [6] number of rows whose columns are not strictly increasing      [7] the first of them
+ * With out_indptr / out_indices / out_data (all or none) it also writes the int32 / fp64 CSR with n_dummy (<= 32)
+ * columns of ones prepended to every row (columns 0..n_dummy-1; the others shift by n_dummy), in the input's order
+ * within a row.  nnz is the length of indices / values; a corrupt indptr is reported, never read past nnz.
+ *
+ * sp_csr_sum_runs: canonicalisation after a stable sort of the keys row*n_cols+col of a CSR: for every run of equal
+ * keys (head p: p == 0 or keys[p-1] != keys[p]), out_data[run_index[p]] = data[perm[p]] + data[perm[p+1]] + ...
+ * summed left to right and out_indices[run_index[p]] = key % n_cols. */
+#define SP_CSR_REPORT_LEN 8
+#define SP_CSR_REPORT_DECREASING 0
+#define SP_CSR_REPORT_INDPTR0 1
+#define SP_CSR_REPORT_INDPTRN 2
+#define SP_CSR_REPORT_RANGE 3
+#define SP_CSR_REPORT_NAN 4
+#define SP_CSR_REPORT_INF 5
+#define SP_CSR_REPORT_N_UNSORTED 6
+#define SP_CSR_REPORT_UNSORTED 7
+int sp_csr_prepare(int64_t n_rows, int64_t n_cols, int64_t nnz, const void *indptr, int indptr_i64,
+                   const void *indices, int indices_i64, const void *values, int values_f64, int64_t stride_row,
+                   int64_t stride_col, int n_dummy, int32_t *out_indptr, int32_t *out_indices, double *out_data,
+                   int64_t *report, sp_stream stream);
+int sp_csr_sum_runs(int64_t nnz, const int64_t *keys, const int64_t *perm, const double *data,
+                    const int64_t *run_index, int64_t n_cols, int32_t *out_indices, double *out_data,
+                    sp_stream stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -92,6 +92,7 @@ class SpPbcdModel(C.Structure):
 
 PREDICT_MAX_MODELS = 256           # SP_PREDICT_MAX_MODELS
 OBJECTIVE_MAX_ENTRIES = 256        # SP_OBJECTIVE_MAX_ENTRIES
+CSR_REPORT_LEN = 8                 # SP_CSR_REPORT_LEN: sp_csr_prepare's report (its entries: dataset.check_X)
 
 
 class SpPredictModel(C.Structure):
@@ -181,6 +182,9 @@ SIGNATURES = {
     "sp_loss_sum_multi": (_i, [C.POINTER(SpLossEntry), _i, _i, _i, _i, _vp, _vp]),
     "sp_sqnorm_multi": (_i, [C.POINTER(SpSqnormEntry), _i, C.c_int64, _vp, _vp]),
     "sp_reg_eval_multi": (_i, [C.POINTER(SpRegEntry), _i, _i, _i, _i, _vp, _vp]),
+    "sp_csr_prepare": (_i, [C.c_int64, C.c_int64, C.c_int64, _vp, _i, _vp, _i, _vp, _i, C.c_int64, C.c_int64, _i,
+                            _vp, _vp, _vp, _vp, _vp]),
+    "sp_csr_sum_runs": (_i, [C.c_int64, _vp, _vp, _vp, _vp, C.c_int64, _vp, _vp, _vp]),
 }
 
 _LIB = None

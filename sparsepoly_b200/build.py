@@ -18,7 +18,7 @@ CSRC = os.path.join(HERE, "csrc")
 INC = os.path.join(HERE, "..", "include")
 OUT = os.path.join(HERE, "libsparsepoly_b200.so")
 OBJ = os.path.join(HERE, "csrc", "_obj")
-SOURCES = ["errors.cu", "rows.cu", "plan.cu", "regcache.cu", "wplan.cu", "pcd.cu", "pcd_window.cu", "pbcd.cu", "pbcd_window.cu", "psgd.cu", "psgd_plan.cu", "objective.cu"]
+SOURCES = ["errors.cu", "rows.cu", "plan.cu", "regcache.cu", "wplan.cu", "pcd.cu", "pcd_window.cu", "pbcd.cu", "pbcd_window.cu", "psgd.cu", "psgd_plan.cu", "objective.cu", "input.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-std=c++17", "-O3", "-lineinfo",
               "-fmad=false", "-Xcompiler", "-fPIC", "-I", INC, "-I", CSRC]
 

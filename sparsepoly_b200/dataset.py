@@ -13,6 +13,8 @@ import os
 import numpy as np
 import scipy.sparse as sp
 import torch
+from sklearn.utils.validation import _check_y, check_array, check_consistent_length
+from sklearn.utils.validation import check_X_y as _sk_check_X_y
 
 from . import _lib
 
@@ -81,6 +83,186 @@ def host_csc(X):
     return indptr, indices, np.ascontiguousarray(X.T).reshape(-1)
 
 
+_NO_ROW = 2 ** 63 - 1          # a "first row" entry of sp_csr_prepare's report that found nothing
+_REPORT = dict(decreasing=0, indptr0=1, indptrn=2, range=3, nan=4, inf=5, n_unsorted=6, unsorted=7)
+
+
+def is_device_input(X):
+    """A CUDA tensor, or the DeviceCSR check_X made of one."""
+    return isinstance(X, DeviceCSR) or (isinstance(X, torch.Tensor) and X.is_cuda)
+
+
+def host_y(y):
+    """Targets on the host: a torch tensor (on any device) becomes a numpy array; anything else is returned as is."""
+    return y.detach().cpu().numpy() if isinstance(y, torch.Tensor) else y
+
+
+class DeviceCSR:
+    """A CUDA design matrix after check_X: the CSR host_csr gives for the same matrix (sorted, duplicate-free rows,
+    int32 indptr / indices, fp64 data), on the device.  Canonical int32 / fp64 input is the caller's own tensors."""
+
+    def __init__(self, shape, indptr, indices, data, dense):
+        self.shape = (int(shape[0]), int(shape[1]))
+        self.indptr, self.indices, self.data = indptr, indices, data
+        self.nnz = int(data.numel())
+        self.dense = dense              # from a strided tensor: every entry is stored
+
+    def augment(self, n_dummy):
+        """add_dummy_feature applied n_dummy times: columns 0..n_dummy-1 of ones, the others shifted by n_dummy."""
+        if n_dummy == 0:
+            return self
+        n, d = self.shape
+        _check_stored(self.nnz + n * n_dummy, self.dense)
+        out = _alloc_csr(n, self.nnz + n * n_dummy, self.data.device)
+        _run_prepare(n, d, self.indptr, self.indices, self.data, (0, 0), n_dummy, out)
+        return DeviceCSR((n, d + n_dummy), *out, self.dense)
+
+
+def _check_stored(stored, dense):
+    if stored < 2 ** 31:
+        return
+    if dense:
+        raise ValueError("dense input with n_samples * n_features >= 2^31 is not supported (int32 indptr, reference "
+                         "dataset.py:60-66); pass a scipy sparse matrix")
+    raise ValueError("nnz >= 2^31 is not supported (int32 indptr, reference dataset.py:60-66)")
+
+
+def _alloc_csr(n, nnz, dev):
+    return (torch.empty(n + 1, dtype=torch.int32, device=dev), torch.empty(nnz, dtype=torch.int32, device=dev),
+            torch.empty(nnz, dtype=torch.float64, device=dev))
+
+
+def _run_prepare(n, d, indptr, indices, values, strides, n_dummy, out=None):
+    """sp_csr_prepare (indptr None: dense strided values); returns the report tensor (still on the device)."""
+    report = torch.empty(_lib.CSR_REPORT_LEN, dtype=torch.int64, device=values.device)
+    o = out if out is not None else (None, None, None)
+    _lib.check(_lib.load().sp_csr_prepare(
+        n, d, int(values.numel()), _ptr(indptr), int(indptr is not None and indptr.dtype == torch.int64),
+        _ptr(indices), int(indices is not None and indices.dtype == torch.int64), _ptr(values),
+        int(values.dtype == torch.float64), int(strides[0]), int(strides[1]), int(n_dummy), _ptr(o[0]), _ptr(o[1]),
+        _ptr(o[2]), _ptr(report), _stream()))
+    return report
+
+
+def _raise_on_report(r, n_cols, dense, nnz, input_name):
+    name = f" {input_name}" if input_name else ""
+    if not dense:
+        if r[_REPORT["decreasing"]] != _NO_ROW:
+            raise ValueError(f"X: indptr decreases at row {r[_REPORT['decreasing']]} "
+                             "(indptr[row + 1] < indptr[row])")
+        if r[_REPORT["indptr0"]] != 0:
+            raise ValueError(f"X: indptr[0] is {r[_REPORT['indptr0']]}, not 0")
+        if r[_REPORT["indptrn"]] != nnz:
+            raise ValueError(f"X: indptr[-1] is {r[_REPORT['indptrn']]} but X stores {nnz} entries")
+        if r[_REPORT["range"]] != _NO_ROW:
+            raise ValueError(f"X: a column index outside [0, {n_cols}) in row {r[_REPORT['range']]}")
+    # sklearn's wording (_assert_all_finite): NaN wins over infinity
+    if r[_REPORT["nan"]] != _NO_ROW:
+        raise ValueError(f"Input{name} contains NaN. First in row {r[_REPORT['nan']]}.")
+    if r[_REPORT["inf"]] != _NO_ROW:
+        raise ValueError(f"Input{name} contains infinity or a value too large for dtype('float64'). "
+                         f"First in row {r[_REPORT['inf']]}.")
+
+
+def _canonical(n, d, indptr, indices, data):
+    """Sorted, duplicate-free rows of a CSR: stable sort of the (row, column) keys, then every run of equal keys summed
+    left to right (sp_csr_sum_runs), as scipy's sum_duplicates; sums that come to zero stay stored."""
+    nnz, dev = int(data.numel()), data.device
+    counts = (indptr[1:] - indptr[:-1]).to(torch.int64)
+    rows = torch.repeat_interleave(torch.arange(n, dtype=torch.int64, device=dev), counts, output_size=nnz)
+    keys, perm = torch.sort(rows * d + indices.to(torch.int64), stable=True)
+    del rows
+    head = torch.ones(nnz, dtype=torch.bool, device=dev)
+    head[1:] = keys[1:] != keys[:-1]
+    runs_before = torch.zeros(nnz + 1, dtype=torch.int64, device=dev)       # runs_before[p]: heads in [0, p)
+    torch.cumsum(head, 0, out=runs_before[1:])
+    del head
+    n_runs = int(runs_before[-1].item())
+    out_indices = torch.empty(n_runs, dtype=torch.int32, device=dev)
+    out_data = torch.empty(n_runs, dtype=torch.float64, device=dev)
+    _lib.check(_lib.load().sp_csr_sum_runs(nnz, _ptr(keys), _ptr(perm), _ptr(data), _ptr(runs_before), d,
+                                           _ptr(out_indices), _ptr(out_data), _stream()))
+    return runs_before[indptr.to(torch.int64)].to(torch.int32), out_indices, out_data
+
+
+def device_csr(X, ensure_min_samples=1, ensure_min_features=1, input_name=""):
+    """Check a CUDA X (torch.sparse_csr or strided, 2-D, float32 / float64 values, int32 / int64 indices) on the
+    device and return it as a DeviceCSR: one sp_csr_prepare pass, one small report read back; rows with unsorted or
+    repeated columns are canonicalised on the device.  A DeviceCSR is already checked and is returned as it is."""
+    if isinstance(X, DeviceCSR):
+        return X
+    dev = torch.device("cuda", torch.cuda.current_device())
+    if X.device != dev:
+        raise ValueError(f"X is on {X.device} but the current CUDA device is {dev}; move X there or make its device "
+                         "current (torch.cuda.set_device)")
+    floats = (torch.float32, torch.float64)
+    if X.layout == torch.sparse_csr:
+        if X.dim() != 2 or X.dense_dim() != 0:
+            raise ValueError(f"a CUDA sparse CSR X must be 2-D, not batched and without dense dimensions; got shape "
+                             f"{tuple(X.shape)} with {X.dense_dim()} dense dimension(s)")
+        indptr, indices, values = X.crow_indices(), X.col_indices(), X.values()
+        if indptr.dtype not in (torch.int32, torch.int64) or indices.dtype not in (torch.int32, torch.int64):
+            raise ValueError(f"a CUDA sparse CSR X needs int32 or int64 indices, got {indices.dtype}")
+        if values.dtype not in floats:
+            raise ValueError(f"a CUDA X needs float32 or float64 values, got {values.dtype}")
+        indptr, indices, values = indptr.contiguous(), indices.contiguous(), values.contiguous()
+        if indices.numel() != values.numel() or indptr.numel() != X.shape[0] + 1:
+            raise ValueError(f"X: {indptr.numel()} indptr entries, {indices.numel()} indices and {values.numel()} "
+                             f"values do not form a CSR matrix of shape {tuple(X.shape)}")
+        dense, strides = False, (0, 0)
+    elif X.layout == torch.strided:
+        if X.dim() != 2:
+            raise ValueError(f"a CUDA X must be 2-D; got shape {tuple(X.shape)}")
+        if X.dtype not in floats:
+            raise ValueError(f"a CUDA X needs float32 or float64 values, got {X.dtype}")
+        indptr = indices = None
+        values, dense, strides = X, True, X.stride()
+    else:
+        raise ValueError(f"a CUDA X must be a torch.sparse_csr or a strided (dense) tensor, got layout {X.layout}; "
+                         "convert it with .to_sparse_csr()")
+    n, d = int(X.shape[0]), int(X.shape[1])
+    if n < ensure_min_samples:
+        raise ValueError(f"Found array with {n} sample(s) (shape={(n, d)}) while a minimum of {ensure_min_samples} "
+                         "is required.")
+    if d < ensure_min_features:
+        raise ValueError(f"Found array with {d} feature(s) (shape={(n, d)}) while a minimum of {ensure_min_features} "
+                         "is required.")
+    nnz = n * d if dense else int(values.numel())
+    _check_stored(nnz, dense)
+    wrap = not dense and indptr.dtype == indices.dtype == torch.int32 and values.dtype == torch.float64
+    out = None if wrap else _alloc_csr(n, nnz, dev)
+    r = _run_prepare(n, d, indptr, indices, values, strides, 0, out).tolist()      # the one D2H of the check
+    _raise_on_report(r, d, dense, nnz, input_name)
+    if r[_REPORT["n_unsorted"]]:
+        if out is None:
+            out = _alloc_csr(n, nnz, dev)
+            _run_prepare(n, d, indptr, indices, values, strides, 0, out)
+        out = _canonical(n, d, *out)
+    return DeviceCSR((n, d), *(out if out is not None else (indptr, indices, values)), dense)
+
+
+def check_X(X, **check_array_kwargs):
+    """The one place that decides between the host and the device path: a CUDA tensor is checked and converted on the
+    device (device_csr; ensure_min_samples / ensure_min_features / input_name are honoured, the result is always
+    fp64), anything else goes through sklearn's check_array with the same arguments."""
+    if not is_device_input(X):
+        return check_array(X, **check_array_kwargs)
+    keys = ("ensure_min_samples", "ensure_min_features", "input_name")
+    return device_csr(X, **{k: v for k, v in check_array_kwargs.items() if k in keys})
+
+
+def check_X_y(X, y, **check_X_y_kwargs):
+    """sklearn's check_X_y for host X; for a CUDA X, check_X then sklearn's checks of y (y_numeric as given)."""
+    y = host_y(y)
+    if not is_device_input(X):
+        return _sk_check_X_y(X, y, **check_X_y_kwargs)
+    X = device_csr(X, input_name="X")
+    y = _check_y(y, multi_output=check_X_y_kwargs.get("multi_output", False),
+                 y_numeric=check_X_y_kwargs.get("y_numeric", False))
+    check_consistent_length(X, y)
+    return X, y
+
+
 def csr_to_csc_device(n, d, indptr, indices, data):
     """CSC (indptr, indices, data) of a canonical device CSR matrix: stable sort of the nonzeros by
     column keeps the rows ascending inside every column, i.e. scipy's canonical CSC, bit for bit."""
@@ -109,10 +291,15 @@ class DeviceDataset:
         self.n_samples, self.n_features = int(X.shape[0]), int(X.shape[1])
         self.h2d_bytes = 0
         self.csr = self.csc = None
-        if need_csr:
+        if isinstance(X, DeviceCSR):          # (check_X of a CUDA X: already on the device, nothing to copy)
+            csr = (X.indptr, X.indices, X.data)
+            if need_csc:
+                self.csc = csr_to_csc_device(self.n_samples, self.n_features, *csr)
+            self.csr = csr if need_csr else None
+        elif need_csr:
             self.csr = tuple(_h2d(a, self.device, pin) for a in host_csr(X))
             self.h2d_bytes += sum(t.numel() * t.element_size() for t in self.csr)
-        if need_csc:
+        if need_csc and self.csc is None:
             if need_csr and sp.issparse(X):
                 # transpose on the device (the reference's get_dataset does a host tocsc(),
                 # dataset.py:119-134; at C2 that is ~1 s of scipy against a few ms here)

@@ -24,10 +24,10 @@ from sklearn.exceptions import NotFittedError
 from sklearn.preprocessing import LabelBinarizer, add_dummy_feature
 from sklearn.utils import check_random_state
 from sklearn.utils.multiclass import type_of_target
-from sklearn.utils.validation import check_array, check_consistent_length, check_X_y, column_or_1d
+from sklearn.utils.validation import check_consistent_length, column_or_1d
 
 from . import _lib, solvers
-from .dataset import DeviceDataset, SweepPlan, _device
+from .dataset import DeviceCSR, DeviceDataset, SweepPlan, _device, check_X, check_X_y, host_y
 from .distributed import active_group, broadcast_arrays, global_sum
 
 REGRESSION_LOSSES = ("squared",)
@@ -165,9 +165,10 @@ class SparsePolyClassifierMixin(ClassifierMixin):
         return np.array([lo, hi], dtype=y.dtype), np.where(is_hi, 1.0, -1.0)
 
     def _check_X_y(self, X, y):
+        y = host_y(y)
         fast = self._binary_labels(y)
         if fast is not None:
-            X = check_array(X, dtype=np.double, accept_sparse=True)
+            X = check_X(X, dtype=np.double, accept_sparse=True)
             check_consistent_length(X, y)
             lb = LabelBinarizer(pos_label=1, neg_label=-1)
             lb.classes_, lb.y_type_, lb.sparse_input_ = fast[0], "binary", False
@@ -200,8 +201,8 @@ class SparsePolyClassifierMixin(ClassifierMixin):
             if classes.ndim != 1 or classes.size != 2 or np.unique(classes).size != 2:
                 raise ValueError(f"classes must hold exactly two distinct labels, got {classes!r}.")
             lb = new = LabelBinarizer(pos_label=1, neg_label=-1).fit(classes)
-        X = check_array(X, dtype=np.double, accept_sparse=True)
-        y = column_or_1d(y)
+        X = check_X(X, dtype=np.double, accept_sparse=True)
+        y = column_or_1d(host_y(y))
         check_consistent_length(X, y)
         known = np.isin(y, lb.classes_)
         if not np.all(known):
@@ -254,6 +255,8 @@ class _BaseSparseFactorizationMachine(_SparsePolyBase, metaclass=ABCMeta):
         # one dummy all-ones column per missing lower order (sparse_factorization_machines.py:86-92)
         if self.fit_lower == "augment":
             k = 2 if self.fit_linear else 1
+            if isinstance(X, DeviceCSR):
+                return X.augment(max(0, self.degree - k))
             for _ in range(self.degree - k):
                 X = add_dummy_feature(X, value=1)
         return X
@@ -663,7 +666,7 @@ class _BaseSparseFactorizationMachine(_SparsePolyBase, metaclass=ABCMeta):
         self._end_stream()
         dev = _device()
         _lib.check(_lib.load().sp_set_device(dev.index if dev.index is not None else 0))
-        upload = self._start_upload(X, dev) if self.solver == "psgd" else None
+        upload = self._start_upload(X, dev) if self.solver == "psgd" and not isinstance(X, DeviceCSR) else None
 
         self._init_coefs(n_features, rng)
 
@@ -816,7 +819,7 @@ class _BaseSparseFactorizationMachine(_SparsePolyBase, metaclass=ABCMeta):
     def _predict(self, X):
         if not hasattr(self, "P_"):
             raise NotFittedError("Estimator not fitted.")
-        X = check_array(X, accept_sparse=["csr", "csc"], dtype=np.double)
+        X = check_X(X, accept_sparse=["csr", "csc"], dtype=np.double)
         X = self._augment(X)
         return self._get_output(X)
 
@@ -999,7 +1002,7 @@ class _BaseSparseAllSubsets(_SparsePolyBase, metaclass=ABCMeta):
     def _predict(self, X):
         if not hasattr(self, "P_"):
             raise NotFittedError("Estimator not fitted.")
-        X = check_array(X, accept_sparse=["csr", "csc"], dtype=np.double)
+        X = check_X(X, accept_sparse=["csr", "csc"], dtype=np.double)
         return self._get_output(X)
 
 

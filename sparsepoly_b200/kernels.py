@@ -7,11 +7,13 @@ import numpy as np
 import torch
 
 from . import _lib
-from .dataset import DeviceDataset, _device, _ptr, _stream
+from .dataset import DeviceDataset, _device, _ptr, _stream, check_X, is_device_input
 
 
 def _gram(X, P, degree):
     dev = _device()
+    if is_device_input(X):              # (host X goes to DeviceDataset as it is, as before)
+        X = check_X(X)
     ds = DeviceDataset(X, need_csr=True, need_csc=False, device=dev)
     P = np.ascontiguousarray(np.asarray(P, dtype=np.float64))
     P_dk = torch.from_numpy(np.ascontiguousarray(P.T)).to(dev)

@@ -17,15 +17,13 @@ import warnings
 
 import numpy as np
 import torch
-import scipy.sparse as sp
 from sklearn.base import ClassifierMixin
 from sklearn.exceptions import NotFittedError
 from sklearn.metrics import accuracy_score, r2_score
 from sklearn.utils import check_random_state
-from sklearn.utils.validation import check_array
 
 from . import _lib, objective as _objective, solvers
-from .dataset import DeviceDataset, SweepPlan, _device, choose_geometry
+from .dataset import DeviceDataset, SweepPlan, _device, check_X, choose_geometry, host_y, is_device_input
 from .estimators import _BaseSparseAllSubsets, _BaseSparseFactorizationMachine
 
 _f64 = torch.float64
@@ -37,11 +35,11 @@ _SHARED_ALL = ("n_components", "loss")
 
 def _targets(y, n_models, what="fit_many"):
     """One target per model: y itself, or the elements of a sequence of arrays."""
-    if isinstance(y, (list, tuple)) and len(y) > 0 and all(np.ndim(t) >= 1 for t in y):
+    if isinstance(y, (list, tuple)) and len(y) > 0 and all(np.ndim(host_y(t)) >= 1 for t in y):
         if len(y) != n_models:
             raise ValueError(f"{what}: {len(y)} target arrays for {n_models} estimators")
-        return list(y)
-    return [y] * n_models
+        return [host_y(t) for t in y]
+    return [host_y(y)] * n_models
 
 
 def _check_generators(ests):
@@ -249,7 +247,11 @@ def fit_many(estimators, X, y):
     fm, solver = _validate(ests)
     pbcd = solver == "pbcd"
     first = ests[0]
-    checked = [e._check_X_y(X, yi) for e, yi in zip(ests, _targets(y, len(ests)))]
+    ys = _targets(y, len(ests))
+    checked = [first._check_X_y(X, ys[0])]
+    # a CUDA X is checked and converted once; the other models take that device matrix
+    X_rest = checked[0][0] if is_device_input(X) else X
+    checked += [e._check_X_y(X_rest, yi) for e, yi in zip(ests[1:], ys[1:])]
     Xc = checked[0][0]
     if fm:
         Xc = first._augment(Xc)
@@ -257,7 +259,7 @@ def fit_many(estimators, X, y):
     degree = first.degree if fm else -1
     k, loss = first.n_components, first.loss
     if pbcd:
-        _check_memory(ests, n, d, Xc.nnz if sp.issparse(Xc) else n * d, fm)
+        _check_memory(ests, n, d, Xc.nnz if hasattr(Xc, "nnz") else n * d, fm)
 
     dev = _device()
     _lib.check(_lib.load().sp_set_device(dev.index if dev.index is not None else 0))
@@ -373,7 +375,7 @@ def _check_X(ests, X, fm, what):
     """X as the single-model _predict checks and augments it (0 rows allowed), after the checks that the models fit
     it: every P_ of the call's shape, as wide as X after augmentation, and w_ / lams_ to match."""
     first = ests[0]
-    X = check_array(X, accept_sparse=["csr", "csc"], dtype=np.double, ensure_min_samples=0)
+    X = check_X(X, accept_sparse=["csr", "csc"], dtype=np.double, ensure_min_samples=0)
     if fm and X.shape[0] > 0:
         X = first._augment(X)
     d = X.shape[1] + (_n_dummies(first) if fm and X.shape[0] == 0 else 0)
@@ -445,7 +447,7 @@ def _prepare(ests, X, what):
 def _run_chunks(ests, Xc, fm, shape, what, objective=False):
     """Upload X once and yield (b0, b1, chunk) over chunks of the models that fit the device."""
     n = Xc.shape[0]
-    size = _chunk_size(ests, n, Xc.nnz if sp.issparse(Xc) else Xc.size, shape, objective, what)
+    size = _chunk_size(ests, n, Xc.nnz if hasattr(Xc, "nnz") else Xc.size, shape, objective, what)
     dev = _device()
     _lib.check(_lib.load().sp_set_device(dev.index if dev.index is not None else 0))
     ds = DeviceDataset(Xc, need_csr=True, need_csc=False, device=dev) if n > 0 else None
@@ -471,7 +473,7 @@ def decision_function_many(estimators, X):
 
 def _decision(ests, X, what):
     if not ests:
-        X = check_array(X, accept_sparse=["csr", "csc"], dtype=np.double, ensure_min_samples=0)
+        X = check_X(X, accept_sparse=["csr", "csc"], dtype=np.double, ensure_min_samples=0)
         return np.zeros((0, X.shape[0]))
     return _device_decision(ests, *_prepare(ests, X, what), what)
 

@@ -14,13 +14,13 @@ import numpy as np
 import torch
 
 from . import _lib, solvers
-from .dataset import DeviceDataset, _device
+from .dataset import DeviceDataset, _device, check_X, host_y
 
 _f64 = torch.float64
 
 
 def _targets(est, y):
-    y = np.asarray(y)
+    y = np.asarray(host_y(y))
     if hasattr(est, "label_binarizer_"):
         return est.label_binarizer_.transform(y).ravel().astype(np.float64)
     return np.ascontiguousarray(y, dtype=np.float64).ravel()
@@ -31,12 +31,11 @@ def objective(est, X, y):
     {Regressor,Classifier} on (X, y): dict(loss, l2_w, l2_P, omega, total).  Order o of an FM's P_
     enters with degree `degree - o` (explicit lower orders, sparse_factorization_machines.py:207-225)."""
     from sklearn.exceptions import NotFittedError
-    from sklearn.utils.validation import check_array
     if not hasattr(est, "P_"):
         raise NotFittedError("Estimator not fitted.")
     dev = _device()
     _lib.check(_lib.load().sp_set_device(dev.index if dev.index is not None else 0))
-    X = check_array(X, accept_sparse=["csr", "csc"], dtype=np.double)
+    X = check_X(X, accept_sparse=["csr", "csc"], dtype=np.double)
     is_fm = hasattr(est, "degree")
     if is_fm:
         X = est._augment(X)
