@@ -27,6 +27,13 @@ def _device(device=None):
     return torch.device(device)
 
 
+def _use_device(device=None):
+    """_device(device), made the device of the library's calls from this thread (sp_set_device)."""
+    dev = _device(device)
+    _lib.check(_lib.load().sp_set_device(dev.index if dev.index is not None else 0))
+    return dev
+
+
 def _stream():
     return C.c_void_p(torch.cuda.current_stream().cuda_stream)
 

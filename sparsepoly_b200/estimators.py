@@ -26,8 +26,8 @@ from sklearn.utils import check_random_state
 from sklearn.utils.multiclass import type_of_target
 from sklearn.utils.validation import check_consistent_length, column_or_1d
 
-from . import _lib, solvers
-from .dataset import DeviceCSR, DeviceDataset, SweepPlan, _device, check_X, check_X_y, host_y
+from . import _lib, cd, solvers
+from .dataset import DeviceCSR, DeviceDataset, _use_device, check_X, check_X_y, host_y
 from .distributed import active_group, broadcast_arrays, global_sum
 
 REGRESSION_LOSSES = ("squared",)
@@ -95,9 +95,13 @@ class _SparsePolyBase(BaseEstimator, metaclass=ABCMeta):
         # device handles (ctypes structs with pointers, CUDA tensors) are per-fit scratch, not model state:
         # a fitted estimator pickles / deep-copies like the reference's (P_, w_, lams_, ... are numpy)
         state = dict(self.__dict__)
-        for key in ("_dev_state", "_y_pred_train", "_psgd_stream"):
+        for key in ("_dev_state", "_psgd_stream"):
             state.pop(key, None)
         return state
+
+    def _cd_setup(self, X, y, rng, dev):
+        """pcd / pbcd: move everything to the device and return (epoch, sync), see cd.setup."""
+        return cd.setup(self, X, y, rng, dev)
 
     def _after_epoch(self, it, value, what, sync):
         """callback / verbose handling shared by the epoch loops; True = stop."""
@@ -295,145 +299,7 @@ class _BaseSparseFactorizationMachine(_SparsePolyBase, metaclass=ABCMeta):
         if np.unique(np.abs(self.lams_)) != np.array([1.0]):
             raise ValueError("Lambdas must be +1 or -1.")
 
-    # ---------------------------------------------------------------- pcd
-    def _pcd_setup(self, X, y, rng, dev):
-        """Move everything to the device and return (epoch, sync): epoch() runs one iteration of
-        the reference driver loop (linear CD -> lower orders ascending -> top order,
-        sparse_factorization_machines.py:196-243) and returns the violation sum."""
-        n, d = X.shape
-        k, m = self.n_components, self.degree
-        alpha, beta, gamma = self._scaled(n)
-        ds = DeviceDataset(X, need_csr=True, need_csc=True, device=dev)
-        plan = SweepPlan(ds, "pcd", rec_stride=solvers.rec_stride(m))
-        self._h2d_bytes = ds.h2d_bytes + y.nbytes + self.P_.nbytes + self.w_.nbytes
-        indices_feature = np.arange(d, dtype=np.int32)
-        indices_component = np.arange(k, dtype=np.int32)
-        plan.set_order(indices_feature)
-        stride = solvers.rec_stride(m)
-        rec = torch.zeros(n * stride, dtype=_f64, device=dev)
-        rec[1::stride] = torch.from_numpy(y).to(dev)
-        P = torch.from_numpy(np.ascontiguousarray(self.P_)).to(dev)         # [n_orders, k, d]
-        w = torch.from_numpy(np.ascontiguousarray(self.w_)).to(dev)
-        lams = torch.from_numpy(np.ascontiguousarray(self.lams_, dtype=np.float64)).to(dev)
-        self._device_output(ds, P, w, lams, rec, stride)                     # y_pred -> rec[0::stride]
-        col_norm_sq = ds.col_norm_sq()
-        regstate = torch.zeros(16, dtype=_f64, device=dev)
-        viol_dev = torch.zeros(1, dtype=_f64, device=dev)
-        self._dev_state = dict(ds=ds, plan=plan, rec=rec, stride=stride, P=P, w=w)
-
-        def sync():
-            self.P_[...] = P.cpu().numpy()
-            self.w_[...] = w.cpu().numpy()
-
-        def epoch(read_back=True):
-            viol_dev.zero_()
-            if self.shuffle:
-                rng.shuffle(indices_component)
-                rng.shuffle(indices_feature)
-                plan.set_order(indices_feature)
-            if self.fit_linear:
-                solvers.cd_linear_epoch(ds, plan, w, col_norm_sq, alpha, self.loss, rec, stride, viol_dev)
-            if self.fit_lower == "explicit":
-                for deg in range(2, m):
-                    solvers.pcd_epoch(ds, plan, P[m - deg], lams, deg, beta, gamma, self.eta0,
-                                      self.regularizer, self.loss, rec, stride, regstate, viol_dev,
-                                      indices_component)
-            solvers.pcd_epoch(ds, plan, P[0], lams, m, beta, gamma, self.eta0, self.regularizer,
-                              self.loss, rec, stride, regstate, viol_dev, indices_component)
-            return viol_dev.item() if read_back else None
-
-        return epoch, sync
-
-    def _fit_pcd(self, X, y, rng, dev):
-        epoch, sync = self._pcd_setup(X, y, rng, dev)
-        converged, it = False, 0
-        for it in range(self.max_iter):
-            viol = epoch()
-            if self._after_epoch(it, viol, "Iteration {} violation sum {}", sync):
-                break
-            if viol < self.tol:
-                if self.verbose:
-                    print(f"Converged at iteration {it+1}")
-                converged = True
-                break
-        sync()
-        return converged, it
-
-    # ---------------------------------------------------------------- pbcd
-    def _pbcd_setup(self, X, y, rng, dev):
-        """As _pcd_setup for the block solver (sparse_factorization_machines.py:260-337)."""
-        n, d = X.shape
-        k, m = self.n_components, self.degree
-        alpha, beta, gamma = self._scaled(n)
-        ds = DeviceDataset(X, need_csr=True, need_csc=True, device=dev)
-        plan = SweepPlan(ds, "pbcd", pbcd_shape=(m, k))
-        plans_lower = {}                                   # explicit lower orders: own record shape
-        if self.fit_lower == "explicit":
-            for deg in range(2, m):
-                plans_lower[deg] = SweepPlan(ds, "pbcd", pbcd_shape=(deg, k))
-        plan_lin = SweepPlan(ds, "pcd", rec_stride=2) if self.fit_linear else None
-        self._h2d_bytes = ds.h2d_bytes + y.nbytes + self.P_.nbytes + self.w_.nbytes
-        indices_feature = np.arange(d, dtype=np.int32)
-        plan.set_order(indices_feature)
-        for pl in plans_lower.values():
-            pl.set_order(indices_feature)
-        if plan_lin is not None:
-            plan_lin.set_order(indices_feature)
-        yrec = torch.zeros(n * 2, dtype=_f64, device=dev)
-        yrec[1::2] = torch.from_numpy(y).to(dev)
-        P_kd = torch.from_numpy(np.ascontiguousarray(self.P_)).to(dev)
-        w = torch.from_numpy(np.ascontiguousarray(self.w_)).to(dev)
-        lams = torch.from_numpy(np.ascontiguousarray(self.lams_, dtype=np.float64)).to(dev)
-        self._device_output(ds, P_kd, w, lams, yrec, 2)
-        # feature-major copy for training (sparse_factorization_machines.py:285)
-        P = torch.stack([solvers.transpose(P_kd[o]) for o in range(P_kd.shape[0])])   # [n_orders, d, k]
-        col_norm_sq = ds.col_norm_sq()
-        A = torch.empty(max(n * (m - 1) * k, 1), dtype=_f64, device=dev)
-        reg_norms = torch.zeros(max(d, 1), dtype=_f64, device=dev)
-        regstate = torch.zeros(16, dtype=_f64, device=dev)
-        viol_dev = torch.zeros(1, dtype=_f64, device=dev)
-        self._dev_state = dict(ds=ds, plan=plan, plan_lin=plan_lin, rec=yrec, stride=2, P=P, w=w)
-
-        def sync():
-            for o in range(P.shape[0]):
-                self.P_[o] = solvers.transpose(P[o]).cpu().numpy()
-            self.w_[...] = w.cpu().numpy()
-
-        def epoch(read_back=True):
-            viol_dev.zero_()
-            if self.shuffle:
-                rng.shuffle(indices_feature)
-                plan.set_order(indices_feature)
-                for pl in plans_lower.values():
-                    pl.set_order(indices_feature)
-                if plan_lin is not None:
-                    plan_lin.set_order(indices_feature)
-            if self.fit_linear:
-                solvers.cd_linear_epoch(ds, plan_lin, w, col_norm_sq, alpha, self.loss, yrec, 2, viol_dev)
-            if self.fit_lower == "explicit":
-                for deg in range(2, m):
-                    solvers.pbcd_epoch(ds, plans_lower[deg], P[m - deg], lams, deg, beta, gamma, self.eta0,
-                                       self.regularizer, self.loss, yrec, A, reg_norms, regstate, viol_dev)
-            solvers.pbcd_epoch(ds, plan, P[0], lams, m, beta, gamma, self.eta0, self.regularizer,
-                               self.loss, yrec, A, reg_norms, regstate, viol_dev)
-            return viol_dev.item() if read_back else None
-
-        return epoch, sync
-
-    def _fit_pbcd(self, X, y, rng, dev):
-        epoch, sync = self._pbcd_setup(X, y, rng, dev)
-        converged, it = False, 0
-        for it in range(self.max_iter):
-            viol = epoch()
-            if self._after_epoch(it, viol, "Iteration {} violation sum {}", sync):
-                break
-            if viol < self.tol:
-                if self.verbose:
-                    print(f"Converged at iteration {it+1}")
-                converged = True
-                break
-        sync()
-        return converged, it
+    _pcd_setup = _pbcd_setup = _SparsePolyBase._cd_setup
 
     # ---------------------------------------------------------------- psgd
     def _start_upload(self, X, dev):
@@ -446,7 +312,7 @@ class _BaseSparseFactorizationMachine(_SparsePolyBase, metaclass=ABCMeta):
         def work():
             try:
                 torch.cuda.set_device(dev)
-                _lib.check(_lib.load().sp_set_device(dev.index if dev.index is not None else 0))
+                _use_device(dev)
                 box["ds"] = DeviceDataset(X, need_csr=True, need_csc=False, device=dev, hot_features=not planned)
             except BaseException as e:          # re-raised by the joining thread
                 box["error"] = e
@@ -471,9 +337,7 @@ class _BaseSparseFactorizationMachine(_SparsePolyBase, metaclass=ABCMeta):
         accumulator and the dense-gradient path's buffers.  The planned path's context joins it with the first
         plan (_psgd_bind)."""
         d, k = self.P_.shape[2], self.n_components
-        P_kd = torch.from_numpy(np.ascontiguousarray(self.P_)).to(dev)
-        P = torch.stack([solvers.transpose(P_kd[o]) for o in range(P_kd.shape[0])])   # [n_orders, d, k]
-        del P_kd
+        P = solvers.transpose_batch(torch.from_numpy(np.ascontiguousarray(self.P_)).to(dev))   # [n_orders, d, k]
         m = dict(planned=self.regularizer in solvers.PLANNED_REGS, learning_rate=learning_rate, group=group,
                  world=world, rank=rank, batch_size=batch_size, b_loc=max(1, batch_size // world), P=P,
                  w=torch.from_numpy(np.ascontiguousarray(self.w_)).to(dev),
@@ -600,8 +464,7 @@ class _BaseSparseFactorizationMachine(_SparsePolyBase, metaclass=ABCMeta):
                     solvers.psgd_planned_end(m["ctx"], 0, None, True)
                     m["model_current"] = True
                 m["ctx"].store_model(P, w)
-            for o in range(P.shape[0]):
-                self.P_[o] = solvers.transpose(P[o]).cpu().numpy()
+            self.P_[...] = solvers.transpose_batch(P).cpu().numpy()
             self.w_[...] = w.cpu().numpy()
 
         def epoch(read_back=True):
@@ -629,12 +492,8 @@ class _BaseSparseFactorizationMachine(_SparsePolyBase, metaclass=ABCMeta):
         try:
             for epoch in range(self.max_iter):
                 sum_loss = epoch_fn()
-                if (self.callback is not None) and epoch % self.n_calls == 0:
-                    sync()
-                    if self.callback(self) is not None:
-                        break
-                if self.verbose:
-                    print(f"Epoch {epoch+1} loss {sum_loss}")
+                if self._after_epoch(epoch, sum_loss, "Epoch {} loss {}", sync):
+                    break
                 if sum_loss > (best_loss - self.tol):
                     no_improvement_count += 1
                 else:
@@ -664,23 +523,21 @@ class _BaseSparseFactorizationMachine(_SparsePolyBase, metaclass=ABCMeta):
             raise ValueError(f"Solver {self.solver} is not supported.")
         self._check_combination(self.solver, self.regularizer, self.degree)
         self._end_stream()
-        dev = _device()
-        _lib.check(_lib.load().sp_set_device(dev.index if dev.index is not None else 0))
+        dev = _use_device()
         upload = self._start_upload(X, dev) if self.solver == "psgd" and not isinstance(X, DeviceCSR) else None
 
         self._init_coefs(n_features, rng)
 
         y = np.ascontiguousarray(y, dtype=np.float64)
-        if self.solver == "pcd":
-            converged, self.n_iter_ = self._fit_pcd(X, y, rng, dev)
-        elif self.solver == "pbcd":
-            converged, self.n_iter_ = self._fit_pbcd(X, y, rng, dev)
-        else:
+        if self.solver == "psgd":
             if not (self.warm_start and hasattr(self, "it_")):
                 self.it_ = 1
             converged, self.n_iter_ = self._fit_psgd(X, y, rng, dev, upload)
-        if not converged:
-            warnings.warn("Objective did not converge. Increase max_iter.")
+            if not converged:
+                warnings.warn("Objective did not converge. Increase max_iter.")
+        else:
+            epoch, sync = self._cd_setup(X, y, rng, dev)
+            cd.stopping_loop([self], [sync], lambda active: [epoch()])
         return self
 
     def partial_fit(self, X, y, classes=None):
@@ -719,8 +576,7 @@ class _BaseSparseFactorizationMachine(_SparsePolyBase, metaclass=ABCMeta):
             raise ValueError("degree / n_components / regularizer / loss / fit_lower / fit_linear changed since the "
                              "stream started; fit() starts a new model.")
         t1 = time.perf_counter()
-        dev = _device()
-        _lib.check(_lib.load().sp_set_device(dev.index if dev.index is not None else 0))
+        dev = _use_device()
         before = dict(self.__dict__) if m is None else None
         try:
             mean_loss = self._stream_call(X, y, label_binarizer, learning_rate, dev, m, t0, t1)
@@ -794,7 +650,7 @@ class _BaseSparseFactorizationMachine(_SparsePolyBase, metaclass=ABCMeta):
             w_out = torch.empty(d, dtype=_f64, device=P.device)
             solvers.psgd_planned_read(m["ctx"], P_out, w_out)
         else:
-            P_out, w_out = torch.stack([solvers.transpose(P[o]) for o in range(n_orders)]), m["w"]
+            P_out, w_out = solvers.transpose_batch(P), m["w"]
         self.P_, self.w_ = P_out.cpu().numpy(), w_out.cpu().numpy()
 
     def _end_stream(self):
@@ -806,8 +662,7 @@ class _BaseSparseFactorizationMachine(_SparsePolyBase, metaclass=ABCMeta):
             self.__dict__.pop(key, None)
 
     def _get_output(self, X):
-        dev = _device()
-        _lib.check(_lib.load().sp_set_device(dev.index if dev.index is not None else 0))
+        dev = _use_device()
         ds = DeviceDataset(X, need_csr=True, need_csc=False, device=dev)
         P = torch.from_numpy(np.ascontiguousarray(self.P_)).to(dev)
         w = torch.from_numpy(np.ascontiguousarray(self.w_)).to(dev)
@@ -903,33 +758,18 @@ class _BaseSparseAllSubsets(_SparsePolyBase, metaclass=ABCMeta):
     def fit(self, X, y):
         """Fit the all-subsets model to (X, y) on the current CUDA device; returns self."""
         X, y = self._check_X_y(X, y)
-        n, d = X.shape
-        k = self.n_components
+        d = X.shape[1]
         rng = check_random_state(self.random_state)
         self._get_loss(self.loss)
         self._get_regularizer(self.regularizer)
         if self.solver not in ("pcd", "pbcd"):
             raise ValueError(f"Solver {self.solver} is not supported.")
         self._check_combination(self.solver, self.regularizer, -1)
-        dev = _device()
-        _lib.check(_lib.load().sp_set_device(dev.index if dev.index is not None else 0))
+        dev = _use_device()
         self._init_coefs(d, rng)
         y = np.ascontiguousarray(y, dtype=np.float64)
         epoch, sync = self._setup(X, y, rng, dev)
-        converged, it = False, 0
-        for it in range(self.max_iter):
-            viol = epoch()
-            if self._after_epoch(it, viol, "Iteration {} violation sum {}", sync):
-                break
-            if viol < self.tol:
-                if self.verbose:
-                    print(f"Converged at iteration {it+1}")
-                converged = True
-                break
-        sync()
-        self.n_iter_ = it
-        if not converged:
-            warnings.warn("Objective did not converge. Increase max_iter.")
+        cd.stopping_loop([self], [sync], lambda active: [epoch()])
         return self
 
     def _init_coefs(self, n_features, rng):
@@ -938,62 +778,10 @@ class _BaseSparseAllSubsets(_SparsePolyBase, metaclass=ABCMeta):
             self.P_ = 0.01 * rng.randn(self.n_components, n_features)
         self._init_lambdas(rng)
 
-    def _setup(self, X, y, rng, dev):
-        """Move everything to the device and return (epoch, sync): epoch() runs one iteration of
-        the reference driver loop (sparse_all_subsets.py:104-133 / :160-199)."""
-        n, d = X.shape
-        k = self.n_components
-        beta, gamma = (n * self.beta, n * self.gamma) if self.mean else (self.beta, self.gamma)
-        ds = DeviceDataset(X, need_csr=True, need_csc=True, device=dev)
-        self._h2d_bytes = ds.h2d_bytes + y.nbytes + self.P_.nbytes
-        plan = SweepPlan(ds, self.solver,
-                         rec_stride=solvers.rec_stride(-1) if self.solver == "pcd" else None,
-                         pbcd_shape=(-1, k) if self.solver == "pbcd" else None)
-        indices_feature = np.arange(d, dtype=np.int32)
-        indices_component = np.arange(k, dtype=np.int32)
-        plan.set_order(indices_feature)
-        P_kd = torch.from_numpy(np.ascontiguousarray(self.P_)).to(dev)
-        lams = torch.from_numpy(np.ascontiguousarray(self.lams_, dtype=np.float64)).to(dev)
-        regstate = torch.zeros(16, dtype=_f64, device=dev)
-        viol_dev = torch.zeros(1, dtype=_f64, device=dev)
-        pcd = self.solver == "pcd"
-        stride = solvers.rec_stride(-1) if pcd else 2
-        rec = torch.zeros(n * stride, dtype=_f64, device=dev)
-        rec[1::stride] = torch.from_numpy(y).to(dev)
-        P_dk = solvers.transpose(P_kd)
-        solvers.poly_predict(ds, P_dk, lams, -1, out=rec, out_stride=stride)     # _get_output
-        self._dev_state = dict(ds=ds, plan=plan, rec=rec, stride=stride, P=P_kd if pcd else P_dk)
-        self._y_pred_train = rec[0::stride]
-        if not pcd:
-            A = torch.empty(max(n * k, 1), dtype=_f64, device=dev)
-            reg_norms = torch.zeros(max(d, 1), dtype=_f64, device=dev)
-
-        def sync():
-            if pcd:
-                self.P_[...] = P_kd.cpu().numpy()
-            else:
-                self.P_[...] = solvers.transpose(P_dk).cpu().numpy()
-
-        def epoch(read_back=True):
-            viol_dev.zero_()
-            if self.shuffle:
-                if pcd:
-                    rng.shuffle(indices_component)
-                rng.shuffle(indices_feature)
-                plan.set_order(indices_feature)
-            if pcd:
-                solvers.pcd_epoch(ds, plan, P_kd, lams, -1, beta, gamma, self.eta0, self.regularizer,
-                                  self.loss, rec, stride, regstate, viol_dev, indices_component)
-            else:
-                solvers.pbcd_epoch(ds, plan, P_dk, lams, -1, beta, gamma, self.eta0, self.regularizer,
-                                   self.loss, rec, A, reg_norms, regstate, viol_dev)
-            return viol_dev.item() if read_back else None
-
-        return epoch, sync
+    _setup = _SparsePolyBase._cd_setup
 
     def _get_output(self, X):
-        dev = _device()
-        _lib.check(_lib.load().sp_set_device(dev.index if dev.index is not None else 0))
+        dev = _use_device()
         ds = DeviceDataset(X, need_csr=True, need_csc=False, device=dev)
         P_dk = solvers.transpose(torch.from_numpy(np.ascontiguousarray(self.P_)).to(dev))
         lams = torch.from_numpy(np.ascontiguousarray(self.lams_, dtype=np.float64)).to(dev)

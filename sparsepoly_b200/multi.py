@@ -8,12 +8,10 @@ thread-block cluster of the GPU.  fit_many runs the chains of many models side b
 covers all models still running, one cluster (one row-DP block row, one regularizer-cache block) per model.  Each
 cluster runs the code a single fit runs on that model's own records, so every model ends bit-identical to
 ``est.fit(X, y_i)`` run alone with the cluster sweep (SPARSEPOLY_B200_SWEEP=cluster) and the same geometry.
+The model state, the epoch's sub-epochs and the stopping rule are those of a single fit: both run through cd.py,
+fit_many with one table launch per sub-epoch over its models.
 """
-import contextlib
-import ctypes as C
-import io
 import numbers
-import warnings
 
 import numpy as np
 import torch
@@ -22,8 +20,8 @@ from sklearn.exceptions import NotFittedError
 from sklearn.metrics import accuracy_score, r2_score
 from sklearn.utils import check_random_state
 
-from . import _lib, objective as _objective, solvers
-from .dataset import DeviceDataset, SweepPlan, _device, check_X, choose_geometry, host_y, is_device_input
+from . import _lib, cd, objective as _objective, solvers
+from .dataset import DeviceDataset, SweepPlan, _device, _use_device, check_X, choose_geometry, host_y, is_device_input
 from .estimators import _BaseSparseAllSubsets, _BaseSparseFactorizationMachine
 
 _f64 = torch.float64
@@ -135,92 +133,6 @@ def _check_memory(ests, n, d, nnz, fm):
                          "doubles): split the call")
 
 
-class _Model:
-    """Device state and stopping state of one model of a fit_many call."""
-
-    def __init__(self, b, est, rng, y, ds, plan, stride, fm, pbcd, dev):
-        self.b, self.est, self.rng, self.plan = b, est, rng, plan
-        self.fm, self.pbcd = fm, pbcd
-        n, d = ds.n_samples, ds.n_features
-        self.rec = torch.zeros(n * stride, dtype=_f64, device=dev)
-        self.rec[1::stride] = torch.from_numpy(y).to(dev)
-        self.P = torch.from_numpy(np.ascontiguousarray(est.P_)).to(dev)
-        self.lams = torch.from_numpy(np.ascontiguousarray(est.lams_, dtype=np.float64)).to(dev)
-        if fm:
-            self.w = torch.from_numpy(np.ascontiguousarray(est.w_)).to(dev)
-            est._device_output(ds, self.P, self.w, self.lams, self.rec, stride)          # y_pred -> rec[0::stride]
-            self.alpha, self.beta, self.gamma = est._scaled(n)
-        else:
-            self.w = None
-            solvers.poly_predict(ds, solvers.transpose(self.P), self.lams, -1, out=self.rec, out_stride=stride)
-            self.alpha = 0.0
-            self.beta, self.gamma = (n * est.beta, n * est.gamma) if est.mean else (est.beta, est.gamma)
-        self.regstate = torch.zeros(16, dtype=_f64, device=dev)
-        self.idx_feat = np.arange(d, dtype=np.int32)
-        self.idx_comp = None
-        if pbcd:                    # the feature-major copy and scratch of _pbcd_setup / _setup
-            k = est.n_components
-            if fm:
-                self.P = torch.stack([solvers.transpose(self.P[o]) for o in range(self.P.shape[0])])
-                self.A = torch.empty(max(n * (est.degree - 1) * k, 1), dtype=_f64, device=dev)
-            else:
-                self.P = solvers.transpose(self.P)
-                self.A = torch.empty(max(n * k, 1), dtype=_f64, device=dev)
-            self.reg_norms = torch.zeros(max(d, 1), dtype=_f64, device=dev)
-        else:
-            self.idx_comp = np.arange(est.n_components, dtype=np.int32)
-        self.it, self.converged, self.out = 0, False, io.StringIO()
-
-    def shuffle(self):
-        """The draws of one epoch: pcd shuffles the components then the features, pbcd the features only."""
-        if self.idx_comp is not None:
-            self.rng.shuffle(self.idx_comp)
-        self.rng.shuffle(self.idx_feat)
-        self.plan.set_order(self.idx_feat)
-
-    def sync(self):
-        if not self.pbcd:
-            self.est.P_[...] = self.P.cpu().numpy()
-        elif self.fm:
-            for o in range(self.P.shape[0]):
-                self.est.P_[o] = solvers.transpose(self.P[o]).cpu().numpy()
-        else:
-            self.est.P_[...] = solvers.transpose(self.P).cpu().numpy()
-        if self.w is not None:
-            self.est.w_[...] = self.w.cpu().numpy()
-
-    def descriptor(self, P, ab, viol):
-        s = self.plan.struct
-        idx_comp = None if self.idx_comp is None else self.idx_comp.ctypes.data_as(C.POINTER(C.c_int32))
-        return _lib.SpPcdModel(pos_ptr=s.pos_ptr, flag_idx=s.flag_idx, idx_feat=s.idx_feat, pos_conf=s.pos_conf,
-                               P=P.data_ptr(), lams=self.lams.data_ptr(), ab=float(ab), gamma=float(self.gamma),
-                               eta=float(self.est.eta0), reg=_lib.REG_IDS[self.est.regularizer],
-                               rec=self.rec.data_ptr(), regstate=self.regstate.data_ptr(),
-                               viol=viol.data_ptr() + 8 * self.b, idx_comp_host=idx_comp)
-
-    def pbcd_descriptor(self, P, viol):
-        s = self.plan.struct
-        return _lib.SpPbcdModel(pos_ptr=s.pos_ptr, flag_idx=s.flag_idx, idx_feat=s.idx_feat, P=P.data_ptr(),
-                                lams=self.lams.data_ptr(), beta=float(self.beta), gamma=float(self.gamma),
-                                eta=float(self.est.eta0), reg=_lib.REG_IDS[self.est.regularizer],
-                                yrec=self.rec.data_ptr(), A=self.A.data_ptr(), reg_norms=self.reg_norms.data_ptr(),
-                                regstate=self.regstate.data_ptr(), viol=viol.data_ptr() + 8 * self.b)
-
-
-def _descriptors(models, P_of, ab_of, viol):
-    arr = (_lib.SpPcdModel * len(models))()
-    for i, m in enumerate(models):
-        arr[i] = m.descriptor(P_of(m), ab_of(m), viol)
-    return arr
-
-
-def _pbcd_descriptors(models, P_of, viol):
-    arr = (_lib.SpPbcdModel * len(models))()
-    for i, m in enumerate(models):
-        arr[i] = m.pbcd_descriptor(P_of(m), viol)
-    return arr
-
-
 def fit_many(estimators, X, y):
     """Fit many pcd or pbcd estimators on one design matrix X at once; returns them (fitted in place) as a list.
 
@@ -261,8 +173,7 @@ def fit_many(estimators, X, y):
     if pbcd:
         _check_memory(ests, n, d, Xc.nnz if hasattr(Xc, "nnz") else n * d, fm)
 
-    dev = _device()
-    _lib.check(_lib.load().sp_set_device(dev.index if dev.index is not None else 0))
+    dev = _use_device()
     rngs = [check_random_state(e.random_state) for e in ests]
     for e, rng in zip(ests, rngs):                # the draws of sequential fits, in list order
         e._init_coefs(d, rng)
@@ -271,9 +182,7 @@ def fit_many(estimators, X, y):
     ds = DeviceDataset(Xc, need_csr=True, need_csc=True, device=dev)
 
     def new_plan():
-        plan = SweepPlan(ds, solver, rec_stride=None if pbcd else stride, sweep="cluster")
-        plan.set_order(np.arange(d, dtype=np.int32))
-        return plan
+        return SweepPlan(ds, solver, rec_stride=None if pbcd else stride, sweep="cluster")
 
     plan0 = new_plan()                            # the unshuffled models' order
     n_cta, threads = plan0.n_cta, plan0.threads
@@ -282,58 +191,30 @@ def fit_many(estimators, X, y):
     threads_lin = choose_geometry(ds, "pcd")[1] if pbcd else threads
     col_norm_sq = ds.col_norm_sq()
     viol = torch.zeros(len(ests), dtype=_f64, device=dev)
-    models = []
-    for b, (e, rng, (_, yb)) in enumerate(zip(ests, rngs, checked)):
-        plan = new_plan() if e.shuffle else plan0
-        models.append(_Model(b, e, rng, np.ascontiguousarray(yb, dtype=np.float64), ds, plan, stride, fm, pbcd,
-                             dev))
+    models = [cd.CdModel(e, ds, np.ascontiguousarray(yb, dtype=np.float64), stride,
+                         [new_plan() if e.shuffle else plan0], viol[b:b + 1], rng)
+              for b, (e, rng, (_, yb)) in enumerate(zip(ests, rngs, checked))]
 
-    def epoch_orders(active):
-        """The per-epoch order of _pcd_setup / _pbcd_setup / _setup: linear CD -> explicit lower orders
-        ascending -> top order."""
-        if fm and first.fit_linear:
-            solvers.cd_linear_epoch_multi(ds, n_cta, threads_lin, col_norm_sq,
-                                          _descriptors(active, lambda m: m.w, lambda m: m.alpha, viol), loss, stride)
-        top = (lambda m: m.P[0]) if fm else (lambda m: m.P)
-        orders = [(deg, lambda m, deg=deg: m.P[degree - deg])
-                  for deg in (range(2, degree) if fm and first.fit_lower == "explicit" else ())]
-        for deg, P_of in orders + [(degree, top)]:
-            if pbcd:
-                solvers.pbcd_epoch_multi(ds, n_cta, threads, _pbcd_descriptors(active, P_of, viol), k, deg, loss)
-            else:
-                solvers.pcd_epoch_multi(ds, n_cta, threads, _descriptors(active, P_of, lambda m: m.beta, viol),
-                                        k, deg, loss, stride)
+    def table(ms, kind, order):
+        arr = ((_lib.SpPbcdModel if kind == "pbcd" else _lib.SpPcdModel) * len(ms))()
+        for i, m in enumerate(ms):
+            arr[i] = m.entry(kind, order)
+        return arr
 
-    active = [m for m in models if m.est.max_iter > 0]
-    it = 0
-    while active:
-        viol.zero_()
-        for m in active:
-            if m.est.shuffle:
-                m.shuffle()
-        epoch_orders(active)
+    launch = {
+        "linear": lambda ms, deg, o: solvers.cd_linear_epoch_multi(ds, n_cta, threads_lin, col_norm_sq,
+                                                                   table(ms, "linear", o), loss, stride),
+        "pcd": lambda ms, deg, o: solvers.pcd_epoch_multi(ds, n_cta, threads, table(ms, "pcd", o), k, deg, loss,
+                                                          stride),
+        "pbcd": lambda ms, deg, o: solvers.pbcd_epoch_multi(ds, n_cta, threads, table(ms, "pbcd", o), k, deg, loss),
+    }
+
+    def epoch(active):
+        cd.run_epoch([models[i] for i in active], viol, launch)
         v = viol.cpu().numpy()
-        running = []
-        for m in active:
-            e = m.est
-            m.it = it
-            with contextlib.redirect_stdout(m.out):
-                stop = e._after_epoch(it, float(v[m.b]), "Iteration {} violation sum {}", m.sync)
-                if not stop and float(v[m.b]) < e.tol:
-                    if e.verbose:
-                        print(f"Converged at iteration {it+1}")
-                    m.converged = stop = True
-            if not stop and it + 1 < e.max_iter:
-                running.append(m)
-        active = running
-        it += 1
+        return [float(v[i]) for i in active]
 
-    for m in models:
-        m.sync()
-        m.est.n_iter_ = m.it
-        print(m.out.getvalue(), end="")
-        if not m.converged:
-            warnings.warn("Objective did not converge. Increase max_iter.")
+    cd.stopping_loop(ests, [m.sync for m in models], epoch, buffered=True)
     return ests
 
 
@@ -448,8 +329,7 @@ def _run_chunks(ests, Xc, fm, shape, what, objective=False):
     """Upload X once and yield (b0, b1, chunk) over chunks of the models that fit the device."""
     n = Xc.shape[0]
     size = _chunk_size(ests, n, Xc.nnz if hasattr(Xc, "nnz") else Xc.size, shape, objective, what)
-    dev = _device()
-    _lib.check(_lib.load().sp_set_device(dev.index if dev.index is not None else 0))
+    dev = _use_device()
     ds = DeviceDataset(Xc, need_csr=True, need_csc=False, device=dev) if n > 0 else None
     for b0 in range(0, len(ests), size):
         b1 = min(len(ests), b0 + size)

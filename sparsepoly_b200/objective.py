@@ -13,8 +13,8 @@ DP kernel and three deterministic device reductions (csrc/objective.cu) and retu
 import numpy as np
 import torch
 
-from . import _lib, solvers
-from .dataset import DeviceDataset, _device, check_X, host_y
+from . import solvers
+from .dataset import DeviceDataset, _use_device, check_X, host_y
 
 _f64 = torch.float64
 
@@ -33,8 +33,7 @@ def objective(est, X, y):
     from sklearn.exceptions import NotFittedError
     if not hasattr(est, "P_"):
         raise NotFittedError("Estimator not fitted.")
-    dev = _device()
-    _lib.check(_lib.load().sp_set_device(dev.index if dev.index is not None else 0))
+    dev = _use_device()
     X = check_X(X, accept_sparse=["csr", "csc"], dtype=np.double)
     is_fm = hasattr(est, "degree")
     if is_fm:

@@ -146,7 +146,6 @@ def test_fitted_estimators_pickle_without_device_state():
     est = S.SparseFactorizationMachineRegressor(degree=2, n_components=3)
     est.P_ = np.zeros((1, 3, 5)); est.w_ = np.zeros(5); est.lams_ = np.ones(3); est.n_iter_ = 4
     est._dev_state = {"ds": _lib.SpDataset(), "plan": C.pointer(_lib.SpPlan())}      # what fit leaves behind
-    est._y_pred_train = object()
     est2 = pickle.loads(pickle.dumps(est))
     assert np.array_equal(est2.P_, est.P_) and est2.n_iter_ == 4 and not hasattr(est2, "_dev_state")
     est3 = copy.deepcopy(est)
